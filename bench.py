@@ -2,8 +2,10 @@
 """bench.py -- the reference's load -> convert -> repeat-multiply loop (src/main.cpp:58-102) on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c1..c5] [--format FMT] [--impl reference]
+                    [--dump-outputs DIR]
 
-One "step" = one SpMV (y := A x) over the whole synthetic matrix of the workload.
+One "step" = one SpMV (y := A x) over the whole synthetic matrix of the workload.  Inputs are seeded, so two builds
+run with the same arguments can be compared on the y that --dump-outputs writes.
 Metric: SpMV GFLOP/s = 2 nnz / t (src/main.cpp:196), with effective HBM GB/s (compulsory bytes / t)
 in `roofline`.  Workloads are BASELINE.json's configs (SURVEY.md 8d):
 
@@ -36,8 +38,10 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree it runs from as it found it
 
 L2_BYTES = 126 * 1024 * 1024
+DUMP_ROWS = 1 << 21                     # --dump-outputs: rows of y kept from a larger result (<= 32 MiB with their indices)
 
 WORKLOADS = {
     "c1": dict(kind="lap2d5", p0=1024, p1=0, seed=1, fmt="crs", formats=["crs", "dia", "ell"], f32=["crs"],
@@ -308,6 +312,28 @@ def run_reference_arm(args, wl, wl_key):
             "e2e": {"value": gflops, "unit": "GFLOP/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ref.y)
+
+
+def dump_outputs(out_dir, y):
+    """--dump-outputs: the y of the timed path's last step as out_dir/y.npy, every row, or for more than DUMP_ROWS rows a
+    fixed seeded sample of rows whose indices go to out_dir/y_rows.npy.  y is a numpy array or a CUDA tensor."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    rows_path = os.path.join(out_dir, "y_rows.npy")
+    rows = None
+    if len(y) > DUMP_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(len(y), size=DUMP_ROWS, replace=False))
+        np.save(rows_path, rows.astype(np.float64))
+    elif os.path.exists(rows_path):
+        os.remove(rows_path)
+    if not isinstance(y, np.ndarray):                        # gather the sample on the device, copy only that
+        import torch
+        y = (y if rows is None else y[torch.from_numpy(rows).to(y.device)]).cpu().numpy()
+    elif rows is not None:
+        y = y[rows]
+    np.save(os.path.join(out_dir, "y.npy"), y)
 
 
 # ------------------------------------------------------------------------------------------ GPU arm, N = 1
@@ -408,8 +434,10 @@ def cpu_sample(sp, wl, x_h):
     return ref, rows, y_ref, mag
 
 
-def run_case(sp, torch, timer, wl_key, wl, fmt, options, coo, x_d, y_d, sptr, steps, warmup, peak, mini, sample):
-    """Convert + time one format on one config.  Returns (entry dict, handle)."""
+def run_case(sp, torch, timer, wl_key, wl, fmt, options, coo, x_d, y_d, sptr, steps, warmup, peak, mini, sample,
+             after_timed=None):
+    """Convert + time one format on one config.  Returns (entry dict, handle).  after_timed(y) is called with the result
+    of the last timed step, before anything else writes y."""
     t0 = time.perf_counter()
     A = sp.SpMatOpt(fmt, **options).convert_device(coo)
     torch.cuda.synchronize()
@@ -428,6 +456,8 @@ def run_case(sp, torch, timer, wl_key, wl, fmt, options, coo, x_d, y_d, sptr, st
             A.multiply(x_d.data_ptr(), y_d.data_ptr(), sptr if s is None else s)
     y_d.fill_(float("nan"))
     ms = timer.run(step, steps, warmup, cold)
+    if after_timed is not None:
+        after_timed(y_d)
     nnz = A.nNnz
     e = {"format": fmt, "options": {k: v for k, v in options.items() if v}, "gflops": 2.0 * nnz / (ms * 1e-3) / 1e9,
          "ms_per_step": ms, "alg_bytes": alg_bytes, "alg_gbs": alg_bytes / (ms * 1e-3) / 1e9,
@@ -575,8 +605,9 @@ def run_single(args, wl_key, only_format):
 
     sampler = ClockSampler(0)
     sampler.start()
+    dump = (lambda y: dump_outputs(args.dump_outputs, y)) if args.dump_outputs else None
     head, A = run_case(sp, torch, timer, wl_key, wl, fmt, options, coo, x_d, y_d, sptr, args.steps, args.warmup, peak,
-                       args.mini, sample)
+                       args.mini, sample, dump)
     nnz, ms, alg_bytes = A.nNnz, head["ms_per_step"], head["alg_bytes"]
 
     # e2e: the reference-facing call SpMV(A_opt, x_opt, y) with HOST vectors, exactly as the C++ plugin issues it
@@ -741,7 +772,14 @@ def main():
     ap.add_argument("--sigma", type=int, default=0)
     ap.add_argument("--value-f32", action="store_true", help="CRS: fp32 storage of the matrix values, fp64 arithmetic")
     ap.add_argument("--precision", type=int, default=0, help="CRS / ELL: 1 = fp32 values, vectors and sums, 2 = fp32 with fp64 sums")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write y of the last timed step of the headline case to DIR/y.npy (a seeded sample of rows, "
+                         "listed in DIR/y_rows.npy, when y is large); one process only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "b200" and (args.gpus != 1 or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs needs a single-GPU run (--gpus 1) or --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     args.options = dict(segment_width=args.segment_width, n_block=args.n_block, csr5_sigma=args.sigma,
                         value_f32=1 if args.value_f32 else 0, precision=args.precision)

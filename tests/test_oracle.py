@@ -1,12 +1,10 @@
 """CPU tests of the test infrastructure itself: the C restatement (oracle/spmv_oracle.c) must
-reproduce, bit for bit, what the reference's own plugins produced -- on the committed golden
-vectors (tests/golden/, made by make_golden.py from the unmodified reference) and, where the
-compiled reference (oracle/_ref) is present, live on larger randomized inputs."""
+reproduce, bit for bit, what the reference's own plugins produced on the committed golden
+vectors (tests/golden/, made by make_golden.py from the unmodified reference)."""
 import numpy as np
 import pytest
 
-from conftest import golden_names, load_golden, skewed_matrix
-from oracle_lib import RefPlugin, ref_available, ref_csr5_convert
+from conftest import golden_names, load_golden
 
 GOLD = golden_names()
 
@@ -154,48 +152,3 @@ def test_csr5(oracle, name, sigma):
 def test_csr5_auto_sigma(oracle):
     # CSR5_cuda/anonymouslib_cuda.h:293-317
     assert [oracle.csr5_auto_sigma(10, n) for n in (0, 40, 50, 320, 330, 2560, 2570)] == [4, 4, 5, 32, 32, 32, 6]
-
-
-# ---------------------------------------------------------------- live against oracle/_ref
-needs_ref = pytest.mark.skipif(not ref_available("crs"), reason="oracle/_ref not built (no /root/reference)")
-
-
-@needs_ref
-@pytest.mark.parametrize("seed", [0, 1])
-def test_live_against_reference(oracle, seed):
-    rng = np.random.default_rng(seed)
-    nRow, nCol = 257, 301
-    row, col, val = skewed_matrix(rng, nRow, nCol, 12)
-    x = rng.random(nCol)
-    r = RefPlugin("crs"); r.convert(nRow, nCol, row, col, val, x)
-    assert np.array_equal(oracle.crs_result(nRow, row, col, val, x), r.spmv())
-    e = RefPlugin("ell"); ge = e.convert(nRow, nCol, row, col, val, x)
-    me = oracle.ell_convert(nRow, row, col, val)
-    assert np.array_equal(me["col_idx"].ravel(), ge["col_idx"]) and np.array_equal(oracle.ell_spmv(me, x), e.spmv())
-    j = RefPlugin("jds"); gj = j.convert(nRow, nCol, row, col, val, x)
-    mj = oracle.jds_convert(nRow, row, col, val, perm_in=gj["perm"])
-    assert np.array_equal(mj["col_idx"], gj["col_idx"]) and np.array_equal(oracle.jds_spmv(mj, x), j.spmv())
-    d = RefPlugin("dia"); gd = d.convert(nRow, nCol, row, col, val, x)
-    md = oracle.dia_convert(nRow, nCol, row, col, val)
-    assert np.array_equal(md["diag"].ravel(), gd["diag"]) and np.array_equal(oracle.dia_spmv(md, x), d.spmv())
-    s = RefPlugin("ss_opt_w32"); gs = s.convert(nRow, nCol, row, col, val, x)
-    ms = oracle.ss_convert(nRow, row, col, val, 32)
-    assert ms["nStep"] == gs["nStep"] and np.array_equal(ms["sum_segs"], gs["sum_segs"])
-    assert np.array_equal(oracle.ss_spmv(ms, x), s.spmv())
-    c = RefPlugin("css_opt_w32_n4"); gc = c.convert(nRow, nCol, row, col, val, x)
-    mc = oracle.css_convert(nRow, nCol, row, col, val, 32, 4)
-    assert np.array_equal(mc["row_ptr"], gc["row_ptr"]) and np.array_equal(mc["sum_segs"], gc["sum_segs"])
-    assert np.array_equal(oracle.css_spmv(mc, x), c.spmv())
-
-
-needs_ref5 = pytest.mark.skipif(not ref_available("csr5"), reason="oracle/_ref/libref_csr5.so not built")
-
-
-@needs_ref5
-@pytest.mark.parametrize("seed", [0, 1, 2])
-def test_csr5_live_against_reference(oracle, seed):
-    rng = np.random.default_rng(seed)
-    nRow, nCol = int(rng.integers(50, 3000)), int(rng.integers(50, 3000))
-    row, col, val = skewed_matrix(rng, nRow, nCol, int(rng.integers(2, 40)))
-    for sigma in (4, 7, 12, 32, oracle.csr5_auto_sigma(nRow, len(row))):
-        _csr5_same(oracle.csr5_convert(nRow, row, col, val, sigma), ref_csr5_convert(nRow, row, col, val, sigma))
