@@ -29,6 +29,8 @@ struct ColBlockEngine {
     virtual ~ColBlockEngine() {}
     virtual int run(const double *x, double *y, int rb, int re, cudaStream_t s) = 0;
     virtual int run_block(int, const double *, double *, int, int, cudaStream_t) { return B200SPMV_ERR_UNSUPPORTED; }   // one block only
+    // host-side bookkeeping of rows [rb, re) (may synchronise): afterwards run() on them never does (graph capture)
+    virtual int prepare(int, int) { return B200SPMV_OK; }
     virtual int n_blocks() const = 0;
     virtual const char *name() const = 0;
 };

@@ -246,6 +246,7 @@ struct EllFormat : Format {
         return B200SPMV_OK;
     }
     bool has_rows() const override { return !(cb != nullptr) && !prec; }   // a row chunk would pay every column-block switch again
+    int prepare_rows(int rb, int re) override { return cb != nullptr ? cb->prepare(rb, re) : B200SPMV_OK; }
     int col_extent(int rb, int re, int *cmin, int *cmax) override
     {
         if (rb < 0 || re > nRow || rb > re) { set_error("col_extent: bad row range [%d,%d)", rb, re); return B200SPMV_ERR_INVALID; }

@@ -325,7 +325,12 @@ struct SsFormat : Format {
     }
 
     bool has_rows() const override { return !faithful && !(cb != nullptr); }
-    int prepare_rows(int rb, int re) override { return (faithful || short_rows || (cb != nullptr)) ? B200SPMV_OK : ts.prepare(rb, re); }
+    int prepare_rows(int rb, int re) override
+    {
+        if (faithful) return B200SPMV_OK;
+        if (cb != nullptr) return cb->prepare(rb, re);
+        return short_rows ? B200SPMV_OK : ts.prepare(rb, re);
+    }
     int col_extent(int rb, int re, int *cmin, int *cmax) override
     {
         if (rb < 0 || re > nRow || rb > re) { set_error("col_extent: bad row range [%d,%d)", rb, re); return B200SPMV_ERR_INVALID; }
@@ -352,6 +357,7 @@ struct SsFormat : Format {
         if (prof.scalar(n, out)) return true;
         if (n == "col_blocks") { *out = (cb != nullptr) ? cb->n_blocks() : 0; return true; }
         if (n == "col_block_engine") { *out = (cb == nullptr) ? 0 : (cb->name()[0] == 'e' ? 1 : 2); return true; }   // 1 = sliced ELL per block, 2 = tile-stream
+        if (n == "short_row_path") { *out = short_rows ? 1 : 0; return true; }   // 1 = row-chunk / row-block stream, 0 = tile-stream
         if (n == "H") { *out = H; return true; }
         if (n == "nStep") { *out = nStep; return true; }
         if (n == "W") { *out = W; return true; }
@@ -610,8 +616,8 @@ struct CssFormat : Format {
     bool has_rows() const override { return !faithful; }
     int prepare_rows(int rb, int re) override
     {
-        if (faithful || (rb == 0 && re == nRow)) return B200SPMV_OK;
-        for (auto &k : blocks) if (!k->cs.ok) B2_TRY(k->ts.prepare(rb, re));
+        if (faithful || ellb || (rb == 0 && re == nRow)) return B200SPMV_OK;
+        for (auto &k : blocks) if (!k->cs.ok || gather_bound) B2_TRY(k->ts.prepare(rb, re));     // the blocks CssBlock::run gives to the tile-stream
         return B200SPMV_OK;
     }
     int multiply_rows(int rb, int re, const double *x, double *y, cudaStream_t s) override
@@ -718,6 +724,7 @@ struct CrsColBlocks : ColBlockEngine {
     CssFormat css;
     explicit CrsColBlocks(const b200spmv_options &o) : css(o) { css.lean = true; css.input_checked = true; }
     int run(const double *x, double *y, int rb, int re, cudaStream_t s) override { return css.multiply_continue(rb, re, x, y, s); }
+    int prepare(int rb, int re) override { return css.prepare_rows(rb, re); }
     int n_blocks() const override { return css.nBlock; }
     const char *name() const override { return "crs"; }
 };

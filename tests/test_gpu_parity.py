@@ -199,8 +199,8 @@ def test_crs_paths_agree(sp, oracle):
         for fmt in ("crs", "ss"):
             A_auto, y_auto = run_host(sp, fmt, nr, nc, row, col, val, x)
             A_tile, y_tile = run_host(sp, fmt, nr, nc, row, col, val, x, crs_path=1)
+            assert A_auto.scalar("short_row_path") == 1 and A_tile.scalar("short_row_path") == 0
             if fmt == "crs":
-                assert A_auto.scalar("short_row_path") == 1 and A_tile.scalar("short_row_path") == 0
                 assert A_auto.scalar("launches") == 1 and A_tile.scalar("launches") == 2
             assert np.array_equal(y_auto, y_ref) and np.array_equal(y_tile, y_ref)
     # longer rows: the short-row kernels do not apply
