@@ -187,7 +187,7 @@ struct CrsFormat : Format {
         if (use_rbs) return rowblock_spmv(ptr.p, idx.p, f32 ? (const void *)val32.p : (const void *)val.p, f32, maxLen, rb, re, x, y, s);
         return cs.run(x, y, rb, re, CS_OVERWRITE, s);
     }
-    bool has_rows() const override { return true; }
+    bool has_rows() const override { return !prec; }   // multiply_rows has no fp32-vector variant
     int prepare_rows(int rb, int re) override { return short_rows ? B200SPMV_OK : use_es ? es.prepare(rb, re) : ts.prepare(rb, re); }
     int col_extent(int rb, int re, int *cmin, int *cmax) override
     {

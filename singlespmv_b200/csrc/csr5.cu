@@ -21,6 +21,7 @@
 //              tile as plain CSR, one thread per row (sequential, reference order).
 //   calibrate: one thread per tile; the first tile of each row adds that row's carries in tile order.
 #include <cub/cub.cuh>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -284,6 +285,10 @@ c5_compute_kernel(const int *__restrict__ col, const VT *__restrict__ val, const
 
     if (direct) yt[off ? off[y_offset] : y_offset] = (XT)last_sum;                    // csr5_spmv_cuda.h:193-195
     if (lane == 0) carry[t] = (double)(direct ? first_sum : last_sum);                      // :198-199
+    // fp32 vectors: the tile's last segment, whose row may go on into the next tile, also in fp64 for the calibration, so
+    // that a row of fp64 sums (precision 2) is rounded to fp32 once
+    if constexpr (std::is_same<XT, float>::value)
+        if (direct && (present >> lane) == 1u) carry[p + t] = (double)last_sum;
 }
 
 // one thread per tile; the first tile of row R adds R's carries in tile order.  R's entries before that
@@ -301,7 +306,8 @@ __global__ void c5_calibrate_kernel(const int *__restrict__ row_ptr, const uint3
     if (t > 0 && (tile_ptr[t - 1] & C5_MASK) == R) return;
     double sum = 0.0;
     for (int u = t; u < p && (tile_ptr[u] & C5_MASK) == R; u++) sum += carry[u];
-    y[R] = (XT)(row_ptr[R] == t * T ? sum : (double)y[R] + sum);
+    if constexpr (std::is_same<XT, float>::value) y[R] = (XT)(row_ptr[R] == t * T ? sum : carry[p + t - 1] + sum);
+    else y[R] = (XT)(row_ptr[R] == t * T ? sum : (double)y[R] + sum);
 }
 
 struct Csr5Format : Format {
@@ -341,7 +347,7 @@ struct Csr5Format : Format {
         B2_TRY(col.alloc((size_t)nnz));
         if (prec) B2_TRY(val32.alloc((size_t)nnz));
         else B2_TRY(val.alloc((size_t)nnz));
-        B2_TRY(carry.alloc((size_t)p));
+        B2_TRY(carry.alloc((size_t)p * (prec ? 2 : 1)));   // fp32 vectors: [p + t] = fp64 last segment of tile t
         B2_CUDA(cudaMemsetAsync(desc.p, 0, desc.bytes() ? desc.bytes() : 4, s));
         DevBuf<int> cnt;
         B2_TRY(cnt.alloc((size_t)p + 1));

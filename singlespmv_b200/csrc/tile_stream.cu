@@ -2,10 +2,17 @@
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
+#include <type_traits>
 
 #include "tile_stream.cuh"
 
 namespace b2 {
+
+// fp64 slots per tile in `carry` (s = ts_slots): carry[s t] holds the piece of a row carried in from earlier tiles; with
+// fp32 vectors carry[2 t + 1] also holds the partial of the row that runs on past the tile's end.  That partial stays in
+// fp64 until the fix-up kernel has added the carries, so a row of fp64 sums (precision 2) is rounded to fp32 once.  fp64
+// vectors keep the partial in y.
+template <typename XT> __host__ __device__ constexpr int ts_slots() { return std::is_same<XT, float>::value ? 2 : 1; }
 
 // tile_row[t] = first row r with row_ptr[r] >= t*TS_TILE (lower bound over row_ptr[0..nRow]).
 // Rows [tile_row[t], tile_row[t+1]) are OWNED by tile t: their first entry lies in it.  Empty
@@ -130,6 +137,12 @@ tile_stream_kernel(const int *__restrict__ row_ptr, const int *__restrict__ col,
         }
         AT acc = accumulate == CS_CONTINUE ? (AT)y[r] : (AT)0;    // CONTINUE: the running sum of the earlier column blocks
         for (int j = b; j < e; j++) acc = Arith<AT>::add(acc, prod[j - t0]);
+        if constexpr (ts_slots<XT>() == 2) {
+            if (e_full > t1) {
+                carry[2 * t + 1] = (double)(accumulate == CS_ADD ? Arith<AT>::add((AT)y[r], acc) : acc);
+                continue;
+            }
+        }
         y[r] = (XT)(accumulate == CS_ADD ? Arith<AT>::add((AT)y[r], acc) : acc);
     }
     if (tid == 0 && cin_end > t0) {
@@ -156,7 +169,8 @@ tile_stream_kernel(const int *__restrict__ row_ptr, const int *__restrict__ col,
         for (int j = b + lane; j < e; j += 32) acc += (double)prod[j - t0];
         acc = warp_sum(acc);
         if (lane == 0) {
-            if (r < 0) carry[t] = acc;
+            if (r < 0) carry[ts_slots<XT>() * t] = acc;
+            else if (ts_slots<XT>() == 2 && row_ptr[r + 1] > t1) carry[2 * t + 1] = accumulate ? (double)y[r] + acc : acc;
             else y[r] = (XT)(accumulate ? (double)y[r] + acc : acc);
         }
     }
@@ -188,8 +202,9 @@ __global__ void tile_fixup_kernel(const int *__restrict__ row_ptr, const int *__
     } else {
         const int last = (e - 1) / tile;
         double sum = 0.0;
-        for (int u = t; u <= last; u++) sum += carry[u];
-        y[rc] = (XT)((double)y[rc] + sum);
+        for (int u = t; u <= last; u++) sum += carry[ts_slots<XT>() * u];
+        if constexpr (ts_slots<XT>() == 2) y[rc] = (XT)(carry[2 * (t - 1) + 1] + sum);     // rc starts in tile t - 1
+        else y[rc] = (XT)((double)y[rc] + sum);
     }
 }
 
@@ -207,7 +222,7 @@ int TileStream::build(const int *row_ptr_d, const int *col_d, const void *val_d,
     tile = threads * TS_IPT;
     nTiles = ceil_div(nnz, tile);
     B2_TRY(tile_row.alloc((size_t)nTiles + 1));
-    B2_TRY(carry.alloc((size_t)nTiles));
+    B2_TRY(carry.alloc((size_t)nTiles * (f32 ? 2 : 1)));   // fp32 values: the fp32-vector kernels may run (ts_slots)
     tile_row_kernel<<<ceil_div(nTiles + 1, 256), 256, 0, s>>>(row_ptr, nRow, nTiles, tile, tile_row.p);
     B2_KERNEL_CHECK();
     range_cache.clear();

@@ -45,7 +45,7 @@ struct TileStream {
     int nTiles = 0;
     int threads = TS_THREADS, tile = TS_TILE;   // CTA width and entries per tile of this instance
     DevBuf<int> tile_row;           // [nTiles+1]: first row whose first entry is >= tile start
-    DevBuf<double> carry;           // [nTiles]
+    DevBuf<double> carry;           // [nTiles], [2 nTiles] when f32 (tile_stream.cu ts_slots)
 
     int build(const int *row_ptr_d, const int *col_d, const void *val_d, bool val_is_f32, int nRow_, int nnz_,
               cudaStream_t s);

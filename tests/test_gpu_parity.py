@@ -1212,8 +1212,8 @@ def test_fp32_variant(sp, oracle, all_cases, fmt, precision):
         tol = np.full(nRow, 1e-5)
         if precision == 1:
             tol = np.maximum(tol, lens * 2.0 ** -23)
-        if fmt == "csr5":
-            tol = np.maximum(tol, 3e-7 * np.sqrt(np.maximum(lens, 1)))      # segment partials are rounded to fp32 before the fp64 carries
+        if fmt == "csr5" and precision == 1:
+            tol = np.maximum(tol, 3e-7 * np.sqrt(np.maximum(lens, 1)))      # fp32 segment sums; precision 2 rounds once
         ok = (err <= tol * np.abs(y_ref)) | (err <= tol * mag)
         assert np.all(ok), (name, int((~ok).sum()), float(np.max(err / np.maximum(mag, 1e-300))))
         with pytest.raises(sp.B200SpmvError) as e:                        # fp64 entry on an fp32 handle
