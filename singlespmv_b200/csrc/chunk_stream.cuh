@@ -22,13 +22,26 @@ constexpr int CS_MAXLEN = 16;      // longest row the row-chunk stream takes (lo
 constexpr int CS_SLACK = 8;        // entries of allocation slack the caller keeps behind idx / val (copies end on 16 bytes)
 constexpr int CS_MAXSTAGES = 4;
 
+// Column feed "offset dictionary" (multiply-only metadata, built at conversion): on stencils and other banded matrices a
+// row's columns are the row number plus a few offsets that repeat from row to row.  Each chunk stores its distinct
+// col - row offsets once (ascending, at most CS_DICT), and each row a bitmask of the offsets it uses; bit j of row r
+// stands for column r + dict[j].  Walking the set bits from low to high visits a row's entries in idx order, so the
+// sums are the same as with the idx feed, bit for bit.  A chunk's record, CS_META_INTS(TH) ints:
+//   dict[CS_DICT] | wbase[TH / 32]: ptr of the first row of every warp | mask[TH]: uint16 per row (0 past nRow)
+// It replaces 4 B/entry of idx and 4 B/row of ptr with (64 + TH / 8 + 2 TH) B per chunk: on c5 0.32 GB instead of 4.29 GB.
+constexpr int CS_DICT = 16;
+__host__ __device__ constexpr int CS_META_INTS(int th) { return CS_DICT + th / 32 + th / 2; }
+enum { CS_FEED_IDX = 0, CS_FEED_DICT = 1 };
+
 struct ChunkStream {
     const int *ptr = nullptr, *idx = nullptr;
     const void *val = nullptr;
     bool f32 = false, ok = false;
     int nRow = 0, maxLen = 0, th = 0, cap = 0;
+    int feed = CS_FEED_IDX;            // CS_FEED_DICT when every chunk fits CS_DICT offsets (and B200SPMV_CS_FEED != idx)
+    DevBuf<int> meta;                  // CS_FEED_DICT: nChunks records of CS_META_INTS(th) ints, then CS_SLACK zeroed ints
 
-    // ok = the matrix qualifies (0 < longest row <= CS_MAXLEN); synchronises s
+    // ok = the matrix qualifies (0 < longest row <= CS_MAXLEN); also picks the feed; synchronises s (once)
     int build(const int *ptr_d, const int *idx_d, const void *val_d, bool val_is_f32, int nRow_, int nnz, int maxLen_,
               cudaStream_t s);
     int run(const double *x, double *y, int rb, int re, int acc, cudaStream_t s) const;

@@ -209,6 +209,7 @@ struct CrsFormat : Format {
         if (n == "crs_kernel") { *out = short_rows ? 1 : use_es ? (es.tma ? 2 : 3) : 0; return true; }   // 0 tile-stream, 1 row-chunk stream, 2 / 3 entry stream (TMA- / load-fed)
         if (n == "maxLength") { *out = maxLen; return true; }
         if (n == "short_row_path") { *out = short_rows ? 1 : 0; return true; }
+        if (n == "chunk_feed") { *out = short_rows && !use_rbs ? cs.feed : CS_FEED_IDX; return true; }   // row-chunk stream: 0 idx / ptr, 1 offset dictionary
         if (n == "nTiles") { *out = ts.nTiles; return true; }
         if (n == "value_f32") { *out = f32 ? 1 : 0; return true; }
         if (n == "precision") { *out = prec; return true; }

@@ -358,6 +358,7 @@ struct SsFormat : Format {
         if (n == "col_blocks") { *out = (cb != nullptr) ? cb->n_blocks() : 0; return true; }
         if (n == "col_block_engine") { *out = (cb == nullptr) ? 0 : (cb->name()[0] == 'e' ? 1 : 2); return true; }   // 1 = sliced ELL per block, 2 = tile-stream
         if (n == "short_row_path") { *out = short_rows ? 1 : 0; return true; }   // 1 = row-chunk / row-block stream, 0 = tile-stream
+        if (n == "chunk_feed") { *out = !faithful && cb == nullptr && short_rows && !use_rbs ? cs.feed : CS_FEED_IDX; return true; }   // see crs.cu
         if (n == "H") { *out = H; return true; }
         if (n == "nStep") { *out = nStep; return true; }
         if (n == "W") { *out = W; return true; }
@@ -667,6 +668,13 @@ struct CssFormat : Format {
         if (n == "B") { *out = B; return true; }
         if (n == "col_block_engine") { *out = ellb ? 1 : (gather_bound ? 2 : 0); return true; }
         if (n == "nBlock") { *out = nBlock; return true; }
+        if (n == "chunk_feed") {   // 1: every block on the row-chunk stream reads the offset dictionary (and there is one)
+            bool any = false, all = true;
+            if (!faithful && !ellb && !gather_bound)
+                for (auto &k : blocks) if (k->cs.ok) { any = true; all = all && k->cs.feed == CS_FEED_DICT; }
+            *out = any && all ? CS_FEED_DICT : CS_FEED_IDX;
+            return true;
+        }
         if (n == "totalH") { *out = totalH; return true; }
         if (n == "W") { *out = W; return true; }
         if (n == "alg_bytes") {   // SS bytes with one row_ptr per block
