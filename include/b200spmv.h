@@ -78,8 +78,8 @@ typedef struct {
     int crs_path;        /* CRS / SS: 0 = choose from the matrix (longest row <= 16 and banded: TMA-fed row-chunk stream; CRS on matrices
                             whose gathers range over > 32 MB of x: the entry stream, sums re-associated within 1e-12; else the
                             tile-stream), 1 = always the tile-stream kernel (rows of up to 64 entries summed in the reference's
-                            order); when the short-row path applies: 2 = the warp-per-32-rows row-block stream of round 1, 3 = the
-                            TMA-fed row-chunk stream; CRS: 4 = always the entry stream */
+                            order); 3 = the TMA-fed row-chunk stream wherever it applies; CRS: 4 = always the entry stream.
+                            2 (round 1's row-block stream) was removed and is rejected, like any value outside 0..4 */
     int profile;         /* SS/CSS with ss_faithful: time the Mul and the Sum phase of every multiply with CUDA events
                             (the reference's -DPROFILING, src/util.h:59-65); the multiply then synchronises and the
                             scalars MulTime_ns / SumTime_ns hold the last call's phases */
@@ -95,7 +95,8 @@ typedef struct {
     int hyb_k;           /* HYB: width of the ELL part; 0 = the largest width that max(4096, nRow/3) rows still fill */
     int coo_path;        /* COO: 0 = entry stream (segmented warp scans; sums re-associated within 1e-12), fed by TMA bulk copies or
                             by the lanes' own loads, whichever suits the matrix; 1 = the order-preserving tile kernel (rows <= 64
-                            entries bit-identical to the CRS result); 2 / 3 = force the load-fed / the TMA-fed entry stream */
+                            entries bit-identical to the CRS result); 2 / 3 = force the load-fed / the TMA-fed entry stream;
+                            other values are rejected */
     int reserved[5];
 } b200spmv_options;
 

@@ -9,7 +9,6 @@ cap() { # name kernel-regex skip args...
   echo "$n rc=$?"
 }
 if [ "${1:-all}" = "late" ]; then   # kernels changed after the first capture round
-cap crsrows_c5 crs_rowblock_kernel 3 --workload c5 --format crs
 cap dia7_c4    dia_spmv_tma       3 --workload c4 --format dia
 cap dia3_c5    dia_spmv_tma       3 --workload c5 --format dia
 cap csr5s16_c5 c5_compute_kernel  3 --workload c5 --format csr5

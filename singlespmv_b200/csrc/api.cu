@@ -14,15 +14,8 @@ long long row_block_limit();
 }
 using namespace b2;
 
-int b2::xload_mode()
-{
-    static int m = -1;
-    if (m < 0) { const char *e = getenv("B200SPMV_XLOAD"); m = e ? atoi(e) : 0; if (m < 0 || m > 5) m = 0; }
-    return m;
-}
-
-constexpr int B200SPMV_HOST_CHUNKS = 32;
-constexpr int B200SPMV_HOST_SLICES = 64;
+constexpr int MAX_HOST_CHUNKS = 32;
+constexpr int MAX_HOST_SLICES = 64;
 
 struct b200spmv_matrix {
     int format = 0;
@@ -31,14 +24,14 @@ struct b200spmv_matrix {
     bool converted = false, blocked = false;
     // plan of the host-semantics pipeline (built on first use)
     int plan_chunks = 0, plan_pieces = 0;
-    int chunk_rb[B200SPMV_HOST_CHUNKS + 1] = {}, chunk_need[B200SPMV_HOST_CHUNKS] = {};
-    long long piece_c0[B200SPMV_HOST_SLICES + 1] = {};
+    int chunk_rb[MAX_HOST_CHUNKS + 1] = {}, chunk_need[MAX_HOST_CHUNKS] = {};
+    long long piece_c0[MAX_HOST_SLICES + 1] = {};
     // staging for host-semantics multiply
     DevBuf<double> x_stage, y_stage;
     DevBuf<float> x_stage32, y_stage32;
     cudaStream_t stream = nullptr, copy_stream = nullptr, in_stream = nullptr;
-    cudaEvent_t chunk_done[B200SPMV_HOST_CHUNKS] = {};
-    cudaEvent_t slice_in[B200SPMV_HOST_SLICES] = {};
+    cudaEvent_t chunk_done[MAX_HOST_CHUNKS] = {};
+    cudaEvent_t slice_in[MAX_HOST_SLICES] = {};
     ~b200spmv_matrix()
     {
         if (stream) cudaStreamDestroy(stream);
@@ -74,16 +67,6 @@ static int require_device()
         set_error("no CUDA device available (%s); libb200spmv has no CPU fallback",
                   e == cudaSuccess ? "device count 0" : cudaGetErrorString(e));
         return B200SPMV_ERR_CUDA;
-    }
-    // L2 fetch granularity: a missing 32-byte sector normally pulls 64 bytes from HBM, which doubles
-    // the DRAM traffic of random x gathers.  B200SPMV_L2_FETCH=32|64|128 sets the device limit once.
-    static bool limit_done = false;
-    if (!limit_done) {
-        limit_done = true;
-        const char *g = getenv("B200SPMV_L2_FETCH");
-        if (g && atoi(g) > 0) {
-            if (cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)atoi(g)) != cudaSuccess) cudaGetLastError();
-        }
     }
     return B200SPMV_OK;
 }
@@ -125,6 +108,14 @@ int b200spmv_create(int format, const b200spmv_options *opts, b200spmv_matrix **
     }
     if (o.n_block < 1 || o.csr5_sigma < -1 || o.csr5_sigma > 32) {
         set_error("create: bad option (n_block=%d csr5_sigma=%d)", o.n_block, o.csr5_sigma);
+        return B200SPMV_ERR_INVALID;
+    }
+    if (o.crs_path == 2) {
+        set_error("create: crs_path=2 selected round 1's row-block stream, which was removed; 3 selects the row-chunk stream");
+        return B200SPMV_ERR_INVALID;
+    }
+    if (o.crs_path < 0 || o.crs_path > 4 || o.coo_path < 0 || o.coo_path > 3) {
+        set_error("create: bad option (crs_path=%d, 0..4 without 2; coo_path=%d, 0..3)", o.crs_path, o.coo_path);
         return B200SPMV_ERR_INVALID;
     }
     if (o.value_f32 && format != B200SPMV_CRS) {
@@ -348,9 +339,6 @@ int b200spmv_multiply_host(b200spmv_matrix *m, const double *x_h, double *y_h)
     //     multiply on a third stream (PCIe is full duplex).
     // The pipeline needs true asynchronous copies: with pageable vectors every cudaMemcpyAsync is staged and the D2H
     // blocks the host, so the chunks would only add launches -> one H2D, one multiply, one D2H instead.
-    static const int env_chunks = getenv("B200SPMV_HOST_CHUNKS") ? atoi(getenv("B200SPMV_HOST_CHUNKS")) : 0;
-    static const int env_pieces = getenv("B200SPMV_HOST_PIECES") ? atoi(getenv("B200SPMV_HOST_PIECES")) : 0;
-    static const int env_slices = getenv("B200SPMV_HOST_SLICES") ? atoi(getenv("B200SPMV_HOST_SLICES")) : 1;
     const bool big = f->nRow >= (1 << 20) && f->has_rows() && host_pinned(x_h) && host_pinned(y_h);
     if (!big) {
         B2_CUDA(cudaMemcpyAsync(m->x_stage.p, x_h, sizeof(double) * (size_t)f->nCol, cudaMemcpyHostToDevice, m->stream));
@@ -359,13 +347,12 @@ int b200spmv_multiply_host(b200spmv_matrix *m, const double *x_h, double *y_h)
         B2_CUDA(cudaStreamSynchronize(m->stream));
         return B200SPMV_OK;
     }
-    const bool sliced = env_slices && f->n_x_slices() > 1 && f->n_x_slices() <= B200SPMV_HOST_SLICES;   // CSS
+    const bool sliced = f->n_x_slices() > 1 && f->n_x_slices() <= MAX_HOST_SLICES;   // CSS
     // chunks of at least 4 MB of y; measured on c2 (profiles/r1_experiments.md): CSS pays for every chunk with another
     // round of x-slice switches in L2 and is best with 2
     const int byBytes = (int)std::max<long long>(2, std::min<long long>(16, (long long)f->nRow * 8 / (4 << 20)));
-    const int nChunks = std::max(1, std::min(env_chunks > 0 ? env_chunks : (sliced ? 2 : byBytes), B200SPMV_HOST_CHUNKS));
-    const int nPieces = sliced ? f->n_x_slices()
-                               : std::max(1, std::min(env_pieces > 0 ? env_pieces : nChunks, B200SPMV_HOST_SLICES));
+    const int nChunks = std::min(sliced ? 2 : byBytes, MAX_HOST_CHUNKS);
+    const int nPieces = sliced ? f->n_x_slices() : std::min(nChunks, MAX_HOST_SLICES);
     B2_TRY(plan_host_pipeline(m, nChunks, sliced ? 1 : nPieces));
     for (int i = 0; i < nPieces; i++) {
         long long c0 = m->piece_c0[i], c1 = m->piece_c0[i + 1];

@@ -209,18 +209,6 @@ __device__ __forceinline__ double ld_x(const double *p, uint64_t pol)
     asm volatile("ld.global.nc.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(r) : "l"(p), "l"(pol));
     return r;
 }
-// Experiment hook (B200SPMV_XLOAD=0..5): how a random x gather is issued.  0 is the shipped choice.
-template <int XM> __device__ __forceinline__ double ld_x_mode(const double *p, uint64_t pol)
-{
-    double r;
-    if (XM == 0) asm volatile("ld.global.nc.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(r) : "l"(p), "l"(pol));
-    else if (XM == 1) asm volatile("ld.global.f64 %0, [%1];" : "=d"(r) : "l"(p));
-    else if (XM == 2) asm volatile("ld.global.nc.f64 %0, [%1];" : "=d"(r) : "l"(p));
-    else if (XM == 3) asm volatile("ld.global.L1::no_allocate.f64 %0, [%1];" : "=d"(r) : "l"(p));
-    else if (XM == 4) asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(r) : "l"(p), "l"(pol));
-    else asm volatile("ld.global.L1::evict_last.f64 %0, [%1];" : "=d"(r) : "l"(p));
-    return r;
-}
 // ---------------------------------------------------------------- mbarrier / TMA (sm_90+ PTX)
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count)
@@ -269,7 +257,6 @@ __device__ __forceinline__ float ld_x(const float *p, uint64_t pol)
     return r;
 }
 
-int xload_mode();   // value of B200SPMV_XLOAD (api.cu)
 __device__ __forceinline__ double warp_sum(double v)
 {
 #pragma unroll

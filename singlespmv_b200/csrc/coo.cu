@@ -13,7 +13,6 @@
 //    crossing a tile boundary are finished by a second tiny kernel (short: recomputed sequentially; long: per-tile carries
 //    added in tile order -> deterministic).
 #include <algorithm>
-#include <cstdlib>
 #include <map>
 
 #include "common.cuh"
@@ -415,12 +414,15 @@ __global__ void coo_stream_fixup_kernel(const int *__restrict__ row, double *__r
     y[rc] = __dadd_rn(y[rc], sum);
 }
 
+// entry-stream tiles: 1024 entries TMA-fed (6 CTAs per SM against 3 with 2048; c5 0.85 against 0.74 of the roofline); load-fed,
+// a warp's 256 consecutive entries of a 2048 tile (c3 410 against 385 GFLOP/s)
+constexpr int COO_E_TMA = 1024, COO_E_LDG = 2048;
+
 struct CooFormat : Format {
     DevBuf<int> row, col;
     DevBuf<double> val, carry;
     int nTiles = 0;
     int path = 0;                                             // 0 = entry stream fed by TMA, 1 = order-preserving tile kernel, 2 = entry stream fed by LDG
-    int E = 2048;                                             // entry stream: entries per tile
     int want = 0;                                             // options.coo_path (0 = choose the feed from the matrix)
     explicit CooFormat(int path_) : want(path_) {}
 
@@ -438,10 +440,7 @@ struct CooFormat : Format {
         B2_CUDA(cudaMemcpyAsync(row.p, A.row, sizeof(int) * (size_t)nnz, cudaMemcpyDeviceToDevice, s));   // opt_coo.cpp:14-19
         B2_CUDA(cudaMemcpyAsync(col.p, A.col, sizeof(int) * (size_t)nnz, cudaMemcpyDeviceToDevice, s));
         B2_CUDA(cudaMemcpyAsync(val.p, A.val, sizeof(double) * (size_t)nnz, cudaMemcpyDeviceToDevice, s));
-        static const char *env_path = getenv("B200SPMV_COO_PATH");
-        static const int env_e = getenv("B200SPMV_COO_E") ? atoi(getenv("B200SPMV_COO_E")) : 0;
         path = want;
-        if (env_path) path = strcmp(env_path, "tile") == 0 ? 1 : strcmp(env_path, "ldg") == 0 ? 2 : strcmp(env_path, "tma") == 0 ? 3 : 0;
         if (path == 0 || path == 3) {
             // Entry stream: who feeds it?  Banded matrices (stencils: the x entries a tile touches are a few MB that L1 / L2 hold
             // whatever else streams by) take the TMA-fed persistent kernel: c5 607 GFLOP/s against 530 with loads.  Matrices whose
@@ -451,10 +450,7 @@ struct CooFormat : Format {
             if (path == 0) B2_TRY(max_band(A.row, A.col, nnz, A.rowOffset, &band, s));
             path = (path == 0 && gathers_need_l2(band)) ? 2 : 0;
         }
-        // tiles of 1024 entries (TMA-fed: 6 CTAs per SM against 3 with 2048; c5 0.85 against 0.74 of the roofline); load-fed: a
-        // warp's 256 consecutive entries of a 2048 tile (c3 410 against 385 GFLOP/s)
-        E = env_e == 2048 || env_e == 1024 ? env_e : (path == 2 ? 2048 : 1024);
-        nTiles = ceil_div(nnz, path == 1 ? COO_TILE : E);
+        nTiles = ceil_div(nnz, path == 1 ? COO_TILE : path == 2 ? COO_E_LDG : COO_E_TMA);
         B2_TRY(carry.alloc((size_t)nTiles));
         B2_CUDA(cudaStreamSynchronize(s));
         return B200SPMV_OK;
@@ -467,8 +463,8 @@ struct CooFormat : Format {
             B2_CUDA(cudaMemsetAsync(y, 0, sizeof(double) * (size_t)nRow, s));
             return B200SPMV_OK;
         }
-        if (path == 2) return E == 1024 ? stream_multiply<1024, false>(x, y, s) : stream_multiply<2048, false>(x, y, s);
-        if (path != 1) return E == 1024 ? stream_multiply<1024, true>(x, y, s) : stream_multiply<2048, true>(x, y, s);
+        if (path == 2) return stream_multiply<COO_E_LDG, false>(x, y, s);
+        if (path != 1) return stream_multiply<COO_E_TMA, true>(x, y, s);
         coo_tile_kernel<false><<<nTiles, COO_THREADS, 0, s>>>(row.p, col.p, val.p, x, y, carry.p, nnz, nRow, 1);
         B2_KERNEL_CHECK();
         if (nTiles > 1) {
@@ -484,7 +480,6 @@ struct CooFormat : Format {
         auto kern = coo_stream_kernel<TE, TMA>;
         static std::map<int, int> per_sm;                      // resident CTAs per SM of this instantiation, by device
         static int sms = 0;
-        static const int env_b = getenv("B200SPMV_COO_CTAS") ? atoi(getenv("B200SPMV_COO_CTAS")) : 0;
         int dev = 0;
         B2_CUDA(cudaGetDevice(&dev));
         if (!sms) B2_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
@@ -496,7 +491,7 @@ struct CooFormat : Format {
             if (n < 1) { set_error("COO entry stream: %zu bytes of shared memory do not fit", smem); return B200SPMV_ERR_UNSUPPORTED; }
             it = per_sm.emplace(dev, n).first;
         }
-        const int perSm = env_b > 0 ? std::min(env_b, it->second) : std::min(it->second, 6);
+        const int perSm = std::min(it->second, 6);
         const int grid = TMA ? std::min(nTiles, sms * perSm) : nTiles;
         kern<<<grid, CS_THREADS, smem, s>>>(row.p, col.p, val.p, x, y, carry.p, nnz, nRow, nTiles);
         B2_KERNEL_CHECK();

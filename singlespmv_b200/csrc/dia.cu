@@ -13,7 +13,6 @@
 // windows from L2 instead of 27.  Per row the diagonals are accumulated in ascending order with
 // unfused mul/add = the reference's order (and, padding zeros aside, opt_crs.cpp's) -> bit-identical y.
 #include <algorithm>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -341,7 +340,6 @@ struct DiaFormat : Format {
             else if (smem_bytes > 48 * 1024) {
                 B2_CUDA(cudaFuncSetAttribute(dia_spmv_tma_kernel<5, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
                 B2_CUDA(cudaFuncSetAttribute(dia_spmv_tma_kernel<7, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
-                B2_CUDA(cudaFuncSetAttribute(dia_spmv_tma_kernel<9, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
                 B2_CUDA(cudaFuncSetAttribute(dia_spmv_tma_kernel<3, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
             }
         }
@@ -381,12 +379,10 @@ struct DiaFormat : Format {
         }
         // diagonals per load round, measured (profiles/r1_experiments.md): 27 diagonals want 7 (c4: 0.99 of the copy
         // peak, 5 gives 0.88), 7 diagonals want 3 (c5: 1.06 vs 0.99), up to 5 diagonals go in one round
-        static const int du_env = getenv("B200SPMV_DIA_U") ? atoi(getenv("B200SPMV_DIA_U")) : 0;
-        const int du = du_env ? du_env : (nDiag >= 16 ? 7 : nDiag <= 5 ? 5 : 3);
+        const int du = nDiag >= 16 ? 7 : nDiag <= 5 ? 5 : 3;
         if (tma_ok && (reinterpret_cast<uintptr_t>(x) & 15) == 0) {
             const int grid = ceil_div(re - rb, DIA_R);
             if (du == 7) dia_spmv_tma_kernel<7, 5><<<grid, DIA_THREADS, smem_bytes, s>>>(diag.p, ld, nDiag, runs, x, y, rb, re, nCol);
-            else if (du == 9) dia_spmv_tma_kernel<9, 4><<<grid, DIA_THREADS, smem_bytes, s>>>(diag.p, ld, nDiag, runs, x, y, rb, re, nCol);
             else if (du == 3) dia_spmv_tma_kernel<3, 8><<<grid, DIA_THREADS, smem_bytes, s>>>(diag.p, ld, nDiag, runs, x, y, rb, re, nCol);
             else dia_spmv_tma_kernel<5, 6><<<grid, DIA_THREADS, smem_bytes, s>>>(diag.p, ld, nDiag, runs, x, y, rb, re, nCol);
         }

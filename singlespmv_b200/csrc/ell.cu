@@ -97,22 +97,9 @@ __device__ __forceinline__ void ell_load(EllGroup<V, float> &g, const int *ecol,
 // One lane per row; the K-loop runs in ascending slot order with unfused mul/add, i.e. the
 // reference's own order -> y is bit-identical to opt_ell.cpp / opt_crs.cpp (fp64).
 // VT = stored value type, XT = type of x and y, AT = type of the products and the row sum.
-__device__ __forceinline__ double ell_gather(const double *p, uint64_t pol, int xm)
-{
-    switch (xm) {
-    case 1: return ld_x_mode<1>(p, pol);
-    case 2: return ld_x_mode<2>(p, pol);
-    case 3: return ld_x_mode<3>(p, pol);
-    case 4: return ld_x_mode<4>(p, pol);
-    case 5: return ld_x_mode<5>(p, pol);
-    default: return ld_x_mode<0>(p, pol);
-    }
-}
-__device__ __forceinline__ float ell_gather(const float *p, uint64_t pol, int) { return ld_x(p, pol); }
-
 // ACC = CS_CONTINUE: the row sums continue what y holds (acc = y[r]; ...; y[r] = acc): the next column block of the same
 // running sum.  ACC = CS_ADD: y[r] = y[r] + sum (CSS adds its block sums, src/opt_css.cpp:298).
-template <int V, int XM, typename VT, typename XT, typename AT, int ACC = CS_OVERWRITE>
+template <int V, typename VT, typename XT, typename AT, int ACC = CS_OVERWRITE>
 __global__ void __launch_bounds__(256)
 ell_spmv_kernel(const long long *__restrict__ slice_off, const int *__restrict__ ecol,
                 const VT *__restrict__ eval, const XT *__restrict__ x, XT *__restrict__ y,
@@ -134,9 +121,9 @@ ell_spmv_kernel(const long long *__restrict__ slice_off, const int *__restrict__
         ell_load<V>(b, ecol, eval, ((size_t)(g + 1) * 32 + lane) * V, pol_stream);
         XT xa[V], xb[V];
 #pragma unroll
-        for (int j = 0; j < V; j++) xa[j] = ell_gather(x + a.c[j], pol_x, XM);
+        for (int j = 0; j < V; j++) xa[j] = ld_x(x + a.c[j], pol_x);
 #pragma unroll
-        for (int j = 0; j < V; j++) xb[j] = ell_gather(x + b.c[j], pol_x, XM);
+        for (int j = 0; j < V; j++) xb[j] = ld_x(x + b.c[j], pol_x);
 #pragma unroll
         for (int j = 0; j < V; j++) acc = Arith<AT>::add(acc, Arith<AT>::mul((AT)xa[j], (AT)a.v[j]));
 #pragma unroll
@@ -147,7 +134,7 @@ ell_spmv_kernel(const long long *__restrict__ slice_off, const int *__restrict__
         ell_load<V>(a, ecol, eval, ((size_t)g * 32 + lane) * V, pol_stream);
         XT xa[V];
 #pragma unroll
-        for (int j = 0; j < V; j++) xa[j] = ell_gather(x + a.c[j], pol_x, XM);
+        for (int j = 0; j < V; j++) xa[j] = ld_x(x + a.c[j], pol_x);
 #pragma unroll
         for (int j = 0; j < V; j++) acc = Arith<AT>::add(acc, Arith<AT>::mul((AT)xa[j], (AT)a.v[j]));
     }
@@ -238,10 +225,10 @@ struct EllFormat : Format {
         if (!prec) { set_error("multiply_f32: the handle was created with precision = 0 (fp64 vectors)"); return B200SPMV_ERR_STATE; }
         if (nRow == 0) return B200SPMV_OK;
         const int blocks = ceil_div((long long)nSlices * 32, 256);
-        if (V == 4 && prec == 1) ell_spmv_kernel<4, 0, float, float, float><<<blocks, 256, 0, s>>>(slice_off.p, ecol.p, eval32.p, x, y, 0, nRow, 0, nSlices);
-        else if (V == 4) ell_spmv_kernel<4, 0, float, float, double><<<blocks, 256, 0, s>>>(slice_off.p, ecol.p, eval32.p, x, y, 0, nRow, 0, nSlices);
-        else if (prec == 1) ell_spmv_kernel<2, 0, float, float, float><<<blocks, 256, 0, s>>>(slice_off.p, ecol.p, eval32.p, x, y, 0, nRow, 0, nSlices);
-        else ell_spmv_kernel<2, 0, float, float, double><<<blocks, 256, 0, s>>>(slice_off.p, ecol.p, eval32.p, x, y, 0, nRow, 0, nSlices);
+        if (V == 4 && prec == 1) ell_spmv_kernel<4, float, float, float><<<blocks, 256, 0, s>>>(slice_off.p, ecol.p, eval32.p, x, y, 0, nRow, 0, nSlices);
+        else if (V == 4) ell_spmv_kernel<4, float, float, double><<<blocks, 256, 0, s>>>(slice_off.p, ecol.p, eval32.p, x, y, 0, nRow, 0, nSlices);
+        else if (prec == 1) ell_spmv_kernel<2, float, float, float><<<blocks, 256, 0, s>>>(slice_off.p, ecol.p, eval32.p, x, y, 0, nRow, 0, nSlices);
+        else ell_spmv_kernel<2, float, float, double><<<blocks, 256, 0, s>>>(slice_off.p, ecol.p, eval32.p, x, y, 0, nRow, 0, nSlices);
         B2_KERNEL_CHECK();
         return B200SPMV_OK;
     }
@@ -267,17 +254,8 @@ struct EllFormat : Format {
         if ((cb != nullptr)) return cb->run(x, y, rb, re, s);
         const int sb = rb / 32, se = ceil_div(re, 32);
         const int blocks = ceil_div((long long)(se - sb) * 32, 256);
-#define ELL_LAUNCH(VV, XM) ell_spmv_kernel<VV, XM, double, double, double><<<blocks, 256, 0, s>>>(slice_off.p, ecol.p, eval.p, x, y, rb, re, sb, se)
-#define ELL_LAUNCH_V(VV)                                   \
-    switch (xload_mode()) {                                \
-    case 1: ELL_LAUNCH(VV, 1); break;                      \
-    case 2: ELL_LAUNCH(VV, 2); break;                      \
-    case 3: ELL_LAUNCH(VV, 3); break;                      \
-    case 4: ELL_LAUNCH(VV, 4); break;                      \
-    case 5: ELL_LAUNCH(VV, 5); break;                      \
-    default: ELL_LAUNCH(VV, 0); break;                     \
-    }
-        if (V == 4) { ELL_LAUNCH_V(4) } else { ELL_LAUNCH_V(2) }
+        if (V == 4) ell_spmv_kernel<4, double, double, double><<<blocks, 256, 0, s>>>(slice_off.p, ecol.p, eval.p, x, y, rb, re, sb, se);
+        else ell_spmv_kernel<2, double, double, double><<<blocks, 256, 0, s>>>(slice_off.p, ecol.p, eval.p, x, y, rb, re, sb, se);
         B2_KERNEL_CHECK();
         return B200SPMV_OK;
     }
@@ -401,9 +379,9 @@ struct EllColBlocks : ColBlockEngine {
         const int sb = rb / 32, se = ceil_div(re, 32);
         const int blocks = ceil_div((long long)(se - sb) * 32, 256);
         const Blk &k = *blk[(size_t)b];
-        if (b == 0) ell_spmv_kernel<2, 0, double, double, double, CS_OVERWRITE><<<blocks, 256, 0, s>>>(k.slice_off.p, k.ecol.p, k.eval.p, x, y, rb, re, sb, se);
-        else if (later == CS_ADD) ell_spmv_kernel<2, 0, double, double, double, CS_ADD><<<blocks, 256, 0, s>>>(k.slice_off.p, k.ecol.p, k.eval.p, x, y, rb, re, sb, se);
-        else ell_spmv_kernel<2, 0, double, double, double, CS_CONTINUE><<<blocks, 256, 0, s>>>(k.slice_off.p, k.ecol.p, k.eval.p, x, y, rb, re, sb, se);
+        if (b == 0) ell_spmv_kernel<2, double, double, double, CS_OVERWRITE><<<blocks, 256, 0, s>>>(k.slice_off.p, k.ecol.p, k.eval.p, x, y, rb, re, sb, se);
+        else if (later == CS_ADD) ell_spmv_kernel<2, double, double, double, CS_ADD><<<blocks, 256, 0, s>>>(k.slice_off.p, k.ecol.p, k.eval.p, x, y, rb, re, sb, se);
+        else ell_spmv_kernel<2, double, double, double, CS_CONTINUE><<<blocks, 256, 0, s>>>(k.slice_off.p, k.ecol.p, k.eval.p, x, y, rb, re, sb, se);
         B2_KERNEL_CHECK();
         return B200SPMV_OK;
     }

@@ -1,6 +1,5 @@
 // entry_stream.cu -- kernels and launcher of the CRS entry stream (see entry_stream.cuh).
 #include <algorithm>
-#include <cstdlib>
 
 #include "entry_stream.cuh"
 
@@ -69,12 +68,13 @@ struct EsChunkRec {
 
 // TMA = true: persistent CTAs, (idx, val) of tile k+1 arriving by two bulk copies while tile k is reduced.
 // TMA = false: one tile per CTA, the lanes load their entries themselves (gather-bound matrices: x must stay in L2).
-template <int E, bool TMA>
+template <bool TMA>
 __global__ void __launch_bounds__(ES_THREADS)
 entry_stream_kernel(const int *__restrict__ idx, const double *__restrict__ val, const unsigned *__restrict__ bits,
                     const int *__restrict__ grpRun, const int *__restrict__ nzrow, const double *__restrict__ x,
                     double *__restrict__ y, double *__restrict__ carry, int nnz, int tileLo, int tileHi, int rowLo, int rowHi)
 {
+    constexpr int E = ES_E;
     constexpr int CHUNK = E / ES_WARPS;
     constexpr int GROUPS = CHUNK / 128;
     static_assert(GROUPS >= 1, "a warp pass covers 128 entries");
@@ -275,10 +275,8 @@ int EntryStream::build(const int *ptr_d, const int *idx_d, const double *val_d, 
     range_cache.clear();
     if (nnz <= 0 || nRow <= 0) return B200SPMV_OK;
     tma = !gather_bound;
-    static const int env_e = getenv("B200SPMV_ES_E") ? atoi(getenv("B200SPMV_ES_E")) : 0;
-    E = env_e == 1024 || env_e == 2048 ? env_e : 2048;        // c4 (TMA-fed) 659 against 620 GFLOP/s with 1024; c3 (load-fed) 418 against 411
-    nTiles = ceil_div(nnz, E);
-    const int nGroups = ceil_div((long long)nTiles * E, 128);
+    nTiles = ceil_div(nnz, ES_E);
+    const int nGroups = ceil_div((long long)nTiles * ES_E, 128);
     B2_TRY(bits.alloc((size_t)nGroups * 4 + 4));
     B2_TRY(grpRun.alloc((size_t)nGroups + 1));
     B2_TRY(carry.alloc((size_t)nTiles));
@@ -317,19 +315,18 @@ int EntryStream::prepare(int rb, int re)
     int pb = 0, pe = 0;
     B2_CUDA(cudaMemcpy(&pb, ptr + rb, sizeof(int), cudaMemcpyDeviceToHost));
     B2_CUDA(cudaMemcpy(&pe, ptr + re, sizeof(int), cudaMemcpyDeviceToHost));
-    const int lo = pb / E, hi = pe > pb ? (pe - 1) / E + 1 : lo;           // tiles that hold an entry of the rows
+    const int lo = pb / ES_E, hi = pe > pb ? (pe - 1) / ES_E + 1 : lo;           // tiles that hold an entry of the rows
     range_cache.emplace(key, std::make_pair(lo, hi));
     return B200SPMV_OK;
 }
 
-template <int E, bool TMA>
+template <bool TMA>
 static int es_launch(EntryStream &T, const double *x, double *y, int tileLo, int tileHi, int rb, int re, cudaStream_t s)
 {
-    constexpr size_t smem = TMA ? 24 * (size_t)E : 0;
-    auto kern = entry_stream_kernel<E, TMA>;
+    constexpr size_t smem = TMA ? 24 * (size_t)ES_E : 0;
+    auto kern = entry_stream_kernel<TMA>;
     static std::map<int, int> per_sm;
     static int sms = 0;
-    static const int env_b = getenv("B200SPMV_ES_CTAS") ? atoi(getenv("B200SPMV_ES_CTAS")) : 0;
     int dev = 0;
     B2_CUDA(cudaGetDevice(&dev));
     if (!sms) B2_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
@@ -342,13 +339,13 @@ static int es_launch(EntryStream &T, const double *x, double *y, int tileLo, int
         it = per_sm.emplace(dev, n).first;
     }
     const int nT = tileHi - tileLo;
-    const int perSm = env_b > 0 ? std::min(env_b, it->second) : std::min(it->second, 6);
+    const int perSm = std::min(it->second, 6);
     const int grid = TMA ? std::min(nT, sms * perSm) : nT;
     kern<<<grid, ES_THREADS, smem, s>>>(T.idx, T.val, T.bits.p, T.grpRun.p, T.nEmpty ? T.nzrow.p : nullptr, x, y, T.carry.p, T.nnz, tileLo,
                                         tileHi, rb, re);
     B2_KERNEL_CHECK();
     if (nT > 1) {
-        entry_stream_fixup_kernel<<<ceil_div(nT - 1, 256), 256, 0, s>>>(T.bits.p, T.grpRun.p, T.nEmpty ? T.nzrow.p : nullptr, y, T.carry.p, E,
+        entry_stream_fixup_kernel<<<ceil_div(nT - 1, 256), 256, 0, s>>>(T.bits.p, T.grpRun.p, T.nEmpty ? T.nzrow.p : nullptr, y, T.carry.p, ES_E,
                                                                        tileLo, tileHi, rb, re);
         B2_KERNEL_CHECK();
     }
@@ -379,8 +376,8 @@ int EntryStream::run_rows(const double *x, double *y, int rb, int re, cudaStream
         B2_KERNEL_CHECK();
     }
     if (hi <= lo) return B200SPMV_OK;
-    if (tma) return E == 1024 ? es_launch<1024, true>(*this, x, y, lo, hi, rb, re, s) : es_launch<2048, true>(*this, x, y, lo, hi, rb, re, s);
-    return E == 1024 ? es_launch<1024, false>(*this, x, y, lo, hi, rb, re, s) : es_launch<2048, false>(*this, x, y, lo, hi, rb, re, s);
+    if (tma) return es_launch<true>(*this, x, y, lo, hi, rb, re, s);
+    return es_launch<false>(*this, x, y, lo, hi, rb, re, s);
 }
 
 }  // namespace b2

@@ -267,7 +267,6 @@ struct SsFormat : Format {
     std::vector<int> counts;
     TileStream ts;
     ChunkStream cs;
-    bool use_rbs = false;
     PhaseTimer prof;
     std::unique_ptr<ColBlockEngine> cb;   // column-blocked multiply layout when x does not fit L2 (colblocks.cuh)
     int cbs_want;
@@ -295,10 +294,9 @@ struct SsFormat : Format {
         B2_TRY(ts.build(row_ptr.p, col2d.p, val2d.p, false, nRow, nnz, s));
         B2_TRY(max_row_length(row_ptr.p, nRow, &maxLen, s));
         B2_TRY(cs.build(row_ptr.p, col2d.p, val2d.p, false, nRow, nnz, maxLen, s));
-        use_rbs = path_opt == 2 && rowblock_applies(maxLen, nnz);
         int band = 0;
         if (path_opt == 0 && cs.ok) B2_TRY(max_band(A.row, A.col, nnz, A.rowOffset, &band, s));
-        short_rows = path_opt != 1 && (use_rbs || (cs.ok && !gathers_need_l2(band)));   // see crs.cu
+        short_rows = path_opt != 1 && cs.ok && !gathers_need_l2(band);   // see crs.cu
         cb.reset();
         if (!faithful) B2_TRY(make_col_block_engine(A, row_ptr.p, cbs_want, s, &cb));
         if (faithful) B2_TRY(val_buf.alloc((size_t)slots));
@@ -344,9 +342,8 @@ struct SsFormat : Format {
     {
         if (faithful) return Format::multiply_rows(rb, re, x, y, s);
         if ((cb != nullptr)) return cb->run(x, y, rb, re, s);
-        if (short_rows) {        // same fused product+sum, warp-per-32-rows stream (crs.cu)
+        if (short_rows) {        // same fused product+sum, TMA-fed row-chunk stream (crs.cu)
             if (rb < 0 || re > nRow || rb > re) { set_error("multiply_rows: bad row range [%d,%d)", rb, re); return B200SPMV_ERR_INVALID; }
-            if (use_rbs) return rowblock_spmv(row_ptr.p, col2d.p, val2d.p, false, maxLen, rb, re, x, y, s);
             return cs.run(x, y, rb, re, CS_OVERWRITE, s);
         }
         return ts.run_rows(x, y, CS_OVERWRITE, rb, re, s);
@@ -357,8 +354,8 @@ struct SsFormat : Format {
         if (prof.scalar(n, out)) return true;
         if (n == "col_blocks") { *out = (cb != nullptr) ? cb->n_blocks() : 0; return true; }
         if (n == "col_block_engine") { *out = (cb == nullptr) ? 0 : (cb->name()[0] == 'e' ? 1 : 2); return true; }   // 1 = sliced ELL per block, 2 = tile-stream
-        if (n == "short_row_path") { *out = short_rows ? 1 : 0; return true; }   // 1 = row-chunk / row-block stream, 0 = tile-stream
-        if (n == "chunk_feed") { *out = !faithful && cb == nullptr && short_rows && !use_rbs ? cs.feed : CS_FEED_IDX; return true; }   // see crs.cu
+        if (n == "short_row_path") { *out = short_rows ? 1 : 0; return true; }   // 1 = row-chunk stream, 0 = tile-stream
+        if (n == "chunk_feed") { *out = !faithful && cb == nullptr && short_rows ? cs.feed : CS_FEED_IDX; return true; }   // see crs.cu
         if (n == "H") { *out = H; return true; }
         if (n == "nStep") { *out = nStep; return true; }
         if (n == "W") { *out = W; return true; }
@@ -739,8 +736,6 @@ struct CrsColBlocks : ColBlockEngine {
 int make_col_block_engine(const CooView &A, const int *row_ptr, int want, cudaStream_t s, std::unique_ptr<ColBlockEngine> *out)
 {
     out->reset();
-    static const char *env_n = getenv("B200SPMV_COL_BLOCKS");           // experiments: 0 = never, n = n blocks
-    if (env_n) want = atoi(env_n) == 0 ? -1 : atoi(env_n);
     if (want < 0 || A.nnz == 0 || A.nRow == 0 || A.nCol == 0) return B200SPMV_OK;
     int nb = want;
     if (want == 0) {

@@ -1,7 +1,5 @@
 // tile_stream.cu -- kernels of the tile-stream multiply (see tile_stream.cuh).
 #include <algorithm>
-#include <cstdlib>
-#include <cstring>
 #include <type_traits>
 
 #include "tile_stream.cuh"
@@ -70,14 +68,14 @@ __device__ __forceinline__ void st_prod4(float *p, float a, float b, float c, fl
 // path, which the x gathers saturate on gather-bound matrices) was measured and removed: with bulk copies in flight the
 // x slice no longer stays L2-resident, whatever cache policy the copies carry (c2 4.4-7.4 ms against 2.9, profiles/r2_experiments.md).
 // VT = stored value type, XT = type of x and y, AT = type of the products and sums.
-template <typename VT, typename XT, typename AT, int TH>
-__global__ void __launch_bounds__(TH)
+template <typename VT, typename XT, typename AT>
+__global__ void __launch_bounds__(TS_THREADS)
 tile_stream_kernel(const int *__restrict__ row_ptr, const int *__restrict__ col,
                    const VT *__restrict__ val, const int *__restrict__ tile_row,
                    const XT *__restrict__ x, XT *__restrict__ y, double *__restrict__ carry,
                    int nnz, int tileLo, int rowLo, int rowHi, int accumulate, int vec_ok)
 {
-    constexpr int TILE = TH * TS_IPT;
+    constexpr int TH = TS_THREADS, TILE = TS_TILE;
     __shared__ __align__(16) AT prod[TILE];
     __shared__ int long_row[TILE / TS_LONG + 2];
     __shared__ int n_long;
@@ -217,13 +215,10 @@ int TileStream::build(const int *row_ptr_d, const int *col_d, const void *val_d,
     val = val_d;
     nRow = nRow_;
     nnz = nnz_;
-    static const int env_threads = getenv("B200SPMV_TS_THREADS") ? atoi(getenv("B200SPMV_TS_THREADS")) : 256;
-    threads = (env_threads == 128 || env_threads == 512) ? env_threads : 256;
-    tile = threads * TS_IPT;
-    nTiles = ceil_div(nnz, tile);
+    nTiles = ceil_div(nnz, TS_TILE);
     B2_TRY(tile_row.alloc((size_t)nTiles + 1));
     B2_TRY(carry.alloc((size_t)nTiles * (f32 ? 2 : 1)));   // fp32 values: the fp32-vector kernels may run (ts_slots)
-    tile_row_kernel<<<ceil_div(nTiles + 1, 256), 256, 0, s>>>(row_ptr, nRow, nTiles, tile, tile_row.p);
+    tile_row_kernel<<<ceil_div(nTiles + 1, 256), 256, 0, s>>>(row_ptr, nRow, nTiles, TS_TILE, tile_row.p);
     B2_KERNEL_CHECK();
     range_cache.clear();
     return B200SPMV_OK;
@@ -266,8 +261,8 @@ int TileStream::prepare(int rb, int re)
     int pb = 0, pe = 0;
     B2_CUDA(cudaMemcpy(&pb, row_ptr + rb, sizeof(int), cudaMemcpyDeviceToHost));
     B2_CUDA(cudaMemcpy(&pe, row_ptr + re, sizeof(int), cudaMemcpyDeviceToHost));
-    const int lo = nTiles ? std::min(pb / tile, nTiles - 1) : 0;
-    const int hi = std::min(nTiles, pe / tile + 1);
+    const int lo = nTiles ? std::min(pb / TS_TILE, nTiles - 1) : 0;
+    const int hi = std::min(nTiles, pe / TS_TILE + 1);
     range_cache.emplace(key, std::make_pair(lo, hi));
     return B200SPMV_OK;
 }
@@ -279,14 +274,11 @@ static int ts_launch(const TileStream &T, const XT *x, XT *y, int acc, int rowLo
     const int vec_ok = ((reinterpret_cast<uintptr_t>(T.col) | reinterpret_cast<uintptr_t>(T.val)) & 15) == 0;
     const int nT = tileHi - tileLo;
     const bool fix = nT > 1 || tileLo > 0;
-#define TS_ARGS T.row_ptr, T.col, v, T.tile_row.p, x, y, T.carry.p, T.nnz, tileLo, rowLo, rowHi, acc, vec_ok
-    if (T.threads == 128) tile_stream_kernel<VT, XT, AT, 128><<<nT, 128, 0, s>>>(TS_ARGS);
-    else if (T.threads == 512) tile_stream_kernel<VT, XT, AT, 512><<<nT, 512, 0, s>>>(TS_ARGS);
-    else tile_stream_kernel<VT, XT, AT, 256><<<nT, 256, 0, s>>>(TS_ARGS);
-#undef TS_ARGS
+    tile_stream_kernel<VT, XT, AT><<<nT, TS_THREADS, 0, s>>>(T.row_ptr, T.col, v, T.tile_row.p, x, y, T.carry.p, T.nnz, tileLo, rowLo,
+                                                             rowHi, acc, vec_ok);
     if (fix)
         tile_fixup_kernel<VT, XT, AT><<<ceil_div(nT, 256), 256, 0, s>>>(T.row_ptr, T.col, v, T.tile_row.p, x, y, T.carry.p, tileLo,
-                                                                        tileHi, rowLo, rowHi, acc, T.tile);
+                                                                        tileHi, rowLo, rowHi, acc, TS_TILE);
     B2_KERNEL_CHECK();
     return B200SPMV_OK;
 }

@@ -43,7 +43,6 @@ struct TileStream {
     int nRow = 0, nnz = 0;
     // owned
     int nTiles = 0;
-    int threads = TS_THREADS, tile = TS_TILE;   // CTA width and entries per tile of this instance
     DevBuf<int> tile_row;           // [nTiles+1]: first row whose first entry is >= tile start
     DevBuf<double> carry;           // [nTiles], [2 nTiles] when f32 (tile_stream.cu ts_slots)
 
@@ -64,11 +63,5 @@ struct TileStream {
     size_t meta_bytes() const { return tile_row.bytes(); }
     std::map<std::pair<int, int>, std::pair<int, int>> range_cache;
 };
-
-// round 1's short-row alternative to the tile-stream (crs.cu): warp-per-32-rows stream, no tiles, one launch.  Kept
-// as options.crs_path = 2 for A/B runs; the default short-row kernel is the TMA-fed row-chunk stream (chunk_stream.cuh)
-int rowblock_spmv(const int *ptr, const int *idx, const void *val, bool f32, int maxLen, int rb, int re, const double *x,
-                  double *y, cudaStream_t s);
-bool rowblock_applies(int maxLen, long long nnz);
 
 }  // namespace b2

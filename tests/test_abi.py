@@ -51,6 +51,41 @@ def test_argument_validation_without_gpu():
     assert e.value.status == -4 or e.value.status == -1
 
 
+def test_create_rejects_unknown_kernel_paths():
+    """crs_path = 2 selected round 1's row-block stream, which was removed; it and every other value outside the documented
+    crs_path / coo_path sets are refused at create instead of silently running some other kernel."""
+    import singlespmv_b200 as sp
+    for fmt, opt in (("crs", {"crs_path": 2}), ("ss", {"crs_path": 2}), ("crs", {"crs_path": 5}), ("crs", {"crs_path": -1}),
+                     ("coo", {"coo_path": 4}), ("coo", {"coo_path": -1})):
+        with pytest.raises(sp.B200SpmvError) as e:
+            sp.SpMatOpt(fmt, **opt)
+        assert e.value.status == -1, (fmt, opt)
+        if opt.get("crs_path") == 2:
+            assert "row-block stream" in str(e.value)
+    for fmt, opt in (("crs", {"crs_path": 1}), ("crs", {"crs_path": 3}), ("crs", {"crs_path": 4}), ("ss", {"crs_path": 3}),
+                     ("coo", {"coo_path": 1}), ("coo", {"coo_path": 3})):
+        sp.SpMatOpt(fmt, **opt)
+
+
+def test_environment_hooks_match_design_table():
+    """The B200SPMV_* variables the library reads are exactly the ones DESIGN.md section 5c documents."""
+    read = set()
+    for dp, dns, fns in os.walk(os.path.join(ROOT, "singlespmv_b200")):
+        dns[:] = [d for d in dns if d not in ("build", "__pycache__")]
+        for fn in fns:
+            if fn.endswith((".cu", ".cuh", ".cpp", ".h")):
+                src = open(os.path.join(dp, fn), errors="replace").read()
+                read |= set(re.findall(r'getenv\(\s*"(B200SPMV_\w+)"', src))
+            elif fn.endswith(".py"):
+                src = open(os.path.join(dp, fn), errors="replace").read()
+                read |= set(re.findall(r'(?:os\.environ\.get\(|os\.environ\[|os\.getenv\()\s*["\'](B200SPMV_\w+)', src))
+    design = open(os.path.join(ROOT, "DESIGN.md")).read()
+    section = design.split("\n## 5c.", 1)[1].split("\n## ", 1)[0]
+    documented = set(re.findall(r"B200SPMV_\w+", section))
+    assert "B200SPMV_DIST_EXCHANGE" in read and "B200SPMV_TMA_R" in read
+    assert read == documented, {"read, not documented": sorted(read - documented), "documented, not read": sorted(documented - read)}
+
+
 def test_no_cpu_fallback():
     """Without a device, conversion and multiply must fail loudly -- never compute on the host."""
     import singlespmv_b200 as sp

@@ -190,7 +190,7 @@ def test_crs_entry_stream(sp, oracle, all_cases):
 
 
 def test_crs_paths_agree(sp, oracle):
-    """Short-row matrices take the row-block stream by default; crs_path=1 forces the tile-stream.  Both sum every
+    """Short-row matrices take the TMA-fed row-chunk stream by default; crs_path=1 forces the tile-stream.  Both sum every
     row in the reference's order -> identical y, and both equal the reference CRS result bit for bit."""
     for kind, n in (("lap3d7", 21), ("lap2d5", 130)):
         nr, nc, row, col, val = oracle.stencil(kind, n)
@@ -906,11 +906,13 @@ def _short_row_matrix(rng, nRow, nCol, max_len):
     return row, col, rng.standard_normal(len(row))
 
 
-@pytest.mark.parametrize("max_len", [1, 5, 8, 9, 16])
+@pytest.mark.parametrize("max_len", [1, 5, 8, 9, 16, 17, 24, 32, 63, 64])
 def test_crs_short_row_kernels_bit_exact(sp, oracle, max_len):
-    """The three CRS kernels that can take a short-row matrix -- tile-stream (crs_path=1), row-block stream (2), TMA-fed
-    row-chunk stream (3, the default) -- all sum every row in the reference's order: bit-identical y, also on row
-    ranges that start and end off the kernels' chunk / 16-byte boundaries, with empty rows and an empty tail."""
+    """The two CRS kernels that can take a short-row matrix -- tile-stream (crs_path=1) and TMA-fed row-chunk stream
+    (3, the default) -- both sum every row in the reference's order: bit-identical y, also on row
+    ranges that start and end off the kernels' chunk / 16-byte boundaries, with empty rows and an empty tail.
+    Rows longer than the row-chunk stream takes (17 and up) send crs_path 3 and 0 to the tile-stream, which still sums
+    rows of up to 64 entries in the reference's order."""
     import torch
     rng = np.random.default_rng(100 + max_len)
     nRow, nCol = 5003, 4097
@@ -920,9 +922,10 @@ def test_crs_short_row_kernels_bit_exact(sp, oracle, max_len):
     x = rng.random(nCol)
     y_ref = oracle.crs_result(nRow, row, col, val, x)
     xd = torch.from_numpy(x).cuda()
-    for path in (1, 2, 3, 0):
+    for path in (1, 3, 0):
         for fmt in ("crs", "ss"):
             A_opt, y = run_host(sp, fmt, nRow, nCol, row, col, val, x, crs_path=path)
+            assert A_opt.scalar("short_row_path") == (1 if path != 1 and max_len <= 16 else 0), (fmt, path)
             assert np.array_equal(y, y_ref), (fmt, path)
             yd = torch.full((nRow,), float("nan"), dtype=torch.float64, device="cuda")
             cuts = [0, 3, 517, 518, 1031, 4000, nRow - 1, nRow]
