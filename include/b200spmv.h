@@ -126,6 +126,21 @@ B200SPMV_API int b200spmv_jds_set_perm_host(b200spmv_matrix *m, const int *perm_
 /* ---- multiply: replaces SpMV (src/opt_crs.cpp:45 etc.).  y := A*x, every y[0..nRow) is
  * overwritten (beta = 0); the call may be repeated any number of times (src/main.cpp:41-88). */
 B200SPMV_API int b200spmv_multiply(b200spmv_matrix *m, const double *x_d, double *y_d, void *stream);
+/* Y[:, 0..k) := A * X[:, 0..k) for k = 1..8 vectors; row-major: X[c*ldx + j], Y[r*ldy + j]; ldx, ldy >= k (in doubles).
+ * CRS handles with precision = 0 and value_f32 = 0.  Columns k..ld-1 of X are never read into a result; those of Y are
+ * never written.  beta = 0 for every Y[r, j], j < k.  Same one-stream-at-a-time rule per handle as b200spmv_multiply.
+ * The matrix is streamed once for all k vectors, and one gather fetches the k values of a column from one row of X.
+ * The kernel follows the one conversion chose (scalar multi_kernel: 1 row-chunk stream, 2 / 3 entry stream TMA- / load-fed):
+ *   - row-chunk stream and entry stream handles: column j of Y has the bits of b200spmv_multiply on column j of X;
+ *   - tile-stream handles (rows longer than 16 that are not gather-bound, e.g. 27-point stencils, and crs_path = 1) run
+ *     the entry stream, whose metadata the first call builds (it synchronises): rows of up to 64 entries are then summed
+ *     in another association than b200spmv_multiply sums them, within the entry stream's 1e-12 tolerance.
+ * The first call on an entry-stream or tile-stream handle allocates per-handle buffers: made inside a stream capture it is
+ * refused with B200SPMV_ERR_STATE; later calls can be captured.  Errors: B200SPMV_ERR_INVALID (NULL handle or vector,
+ * k outside 1..8, ldx or ldy < k), B200SPMV_ERR_UNSUPPORTED (formats other than CRS, value_f32), B200SPMV_ERR_STATE
+ * (before convert, precision 1 / 2, first call inside a capture). */
+B200SPMV_API int b200spmv_multiply_multi(b200spmv_matrix *m, int k, const double *X_d, long long ldx,
+                                         double *Y_d, long long ldy, void *stream);
 /* Host semantics (what SpMV(A_opt, x_opt, y) means to the reference's driver): copies x H2D,
  * multiplies, copies y D2H, synchronises -- like src/opt_cusparse.cpp:72-82. */
 B200SPMV_API int b200spmv_multiply_host(b200spmv_matrix *m, const double *x_h, double *y_h);

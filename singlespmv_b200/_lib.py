@@ -53,6 +53,7 @@ def _load():
     lib.b200spmv_jds_set_perm_host.argtypes = [vp, vp, ip]
     lib.b200spmv_multiply.argtypes = [vp, vp, vp, vp]
     lib.b200spmv_multiply_host.argtypes = [vp, vp, vp]
+    lib.b200spmv_multiply_multi.argtypes = [vp, ip, vp, ll, vp, ll, vp]
     lib.b200spmv_multiply_f32.argtypes = [vp, vp, vp, vp]
     lib.b200spmv_multiply_host_f32.argtypes = [vp, vp, vp]
     lib.b200spmv_multiply_rows.argtypes = [vp, ip, ip, vp, vp, vp]

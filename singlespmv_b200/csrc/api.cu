@@ -216,6 +216,25 @@ int b200spmv_multiply(b200spmv_matrix *m, const double *x_d, double *y_d, void *
     return m->impl->multiply(x_d, y_d, (cudaStream_t)stream);
 }
 
+int b200spmv_multiply_multi(b200spmv_matrix *m, int k, const double *X_d, long long ldx, double *Y_d, long long ldy,
+                            void *stream)
+{
+    clear_error();
+    if (!m) { set_error("multiply_multi: NULL handle"); return B200SPMV_ERR_INVALID; }
+    if (k < 1 || k > 8 || ldx < k || ldy < k) {
+        set_error("multiply_multi: k=%d (1..8), ldx=%lld, ldy=%lld (>= k)", k, ldx, ldy);
+        return B200SPMV_ERR_INVALID;
+    }
+    if (m->format != B200SPMV_CRS) { set_error("multiply_multi: CRS handles only (format %d)", m->format); return B200SPMV_ERR_UNSUPPORTED; }
+    if (m->opt.value_f32) { set_error("multiply_multi: value_f32 handles are not supported"); return B200SPMV_ERR_UNSUPPORTED; }
+    if (m->opt.precision) {
+        set_error("multiply_multi: the handle was created with precision = %d (fp32 vectors)", m->opt.precision);
+        return B200SPMV_ERR_STATE;
+    }
+    B2_TRY(check_ready(m, X_d, Y_d));
+    return m->impl->multiply_multi(k, X_d, ldx, Y_d, ldy, (cudaStream_t)stream);
+}
+
 int b200spmv_multiply_f32(b200spmv_matrix *m, const float *x_d, float *y_d, void *stream)
 {
     B2_TRY(check_ready(m, x_d, y_d));

@@ -103,6 +103,11 @@ struct RowBlocked : Format {
         for (size_t g = 0; g < blk.size(); g++) B2_TRY(blk[g]->multiply_f32(x, y + rb[g], s));
         return B200SPMV_OK;
     }
+    int multiply_multi(int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s) override
+    {
+        for (size_t g = 0; g < blk.size(); g++) B2_TRY(blk[g]->multiply_multi(k, X, ldx, Y + (long long)rb[g] * ldy, ldy, s));
+        return B200SPMV_OK;
+    }
     bool has_rows() const override
     {
         for (auto &b : blk) if (!b->has_rows()) return false;

@@ -130,6 +130,128 @@ chunk_stream_kernel(const int *__restrict__ ptr, const int *__restrict__ idx, co
     }
 }
 
+// The multi-vector form (fp64 values, overwrite): chunks arrive exactly as in chunk_stream_kernel, and the thread of row r
+// sums KP vectors (columns j < k of X; KP = k rounded up to 1, 2, 4, 8) over the row's entries in ascending column order,
+// each with the unfused mul / add of the single multiply.  W2: X rows gathered in 16-byte pairs (ld_xrow).
+template <int MAXL, int TH, bool DICT, int KP, bool W2>
+__global__ void __launch_bounds__(TH, 1)
+chunk_stream_multi_kernel(const int *__restrict__ ptr, const int *__restrict__ idx, const int *__restrict__ meta,
+                          const double *__restrict__ val, const double *__restrict__ X, long long ldx, double *__restrict__ Y,
+                          long long ldy, int kv, int rowBegin, int rowEnd, int chunk0, int nChunks, int capI, int capV, int S)
+{
+    constexpr int MI = CS_META_INTS(TH);
+    extern __shared__ __align__(128) unsigned char cs_smem[];
+    __shared__ __align__(8) uint64_t bar[CS_MAXSTAGES];
+    __shared__ int sbaseI[CS_MAXSTAGES], sbaseV[CS_MAXSTAGES];
+    int *sidx = reinterpret_cast<int *>(cs_smem);
+    double *sval = reinterpret_cast<double *>(cs_smem + (size_t)S * capI * sizeof(int));
+    const int tid = threadIdx.x;
+    const uint64_t pol_stream = policy_evict_first(), pol_x = policy_evict_last();
+
+    auto issue = [&](int s, long long g, int b, int e) {
+        const int *srcI = idx + b;
+        const double *srcV = val + b;
+        const int misI = (int)((reinterpret_cast<uintptr_t>(srcI) & 15) / sizeof(int));
+        const int misV = (int)((reinterpret_cast<uintptr_t>(srcV) & 15) / sizeof(double));
+        const int n = e - b;
+        const uint32_t bytesI = DICT ? (uint32_t)(MI * sizeof(int)) : n ? (uint32_t)(((n + misI) * (int)sizeof(int) + 15) & ~15) : 0u;
+        const uint32_t bytesV = n ? (uint32_t)(((n + misV) * (int)sizeof(double) + 15) & ~15) : 0u;
+        sbaseI[s] = b - misI;
+        sbaseV[s] = b - misV;
+        mbar_expect_tx(&bar[s], bytesI + bytesV);
+        if (DICT) tma_load_1d(sidx + (size_t)s * capI, meta + g * MI, bytesI, &bar[s], pol_stream);
+        if (n) {
+            if (!DICT) tma_load_1d(sidx + (size_t)s * capI, srcI - misI, bytesI, &bar[s], pol_stream);
+            tma_load_1d(sval + (size_t)s * capV, srcV - misV, bytesV, &bar[s], pol_stream);
+        }
+    };
+    auto lo_of = [&](long long g) { return (int)min((long long)rowEnd, max((long long)rowBegin, g * TH)); };
+
+    if (tid == 0)
+        for (int s = 0; s < S; s++) mbar_init(&bar[s], 1);
+    __syncthreads();
+    if (tid == 0) {
+        for (int s = 0; s < S; s++) {
+            const long long c = (long long)blockIdx.x + (long long)s * gridDim.x;
+            if (c < nChunks) issue(s, chunk0 + c, ptr[lo_of(chunk0 + c)], ptr[lo_of(chunk0 + c + 1)]);
+        }
+    }
+    long long g = (long long)chunk0 + blockIdx.x;
+    int r = (int)min(g * TH + tid, (long long)0x7fffffff);
+    bool valid = r >= rowBegin && r < rowEnd;
+    int p = 0, q = 0;
+    if (!DICT && valid) {
+        p = ptr[r];
+        q = ptr[r + 1];
+    }
+    int k = 0;
+    for (long long c = blockIdx.x; c < nChunks; c += gridDim.x, k++) {
+        const int s = k % S;
+        const long long cIssue = c + (long long)S * gridDim.x, cNext = c + gridDim.x;
+        int nb = 0, ne = 0, pn = 0, qn = 0;
+        if (tid == 0 && cIssue < nChunks) {
+            nb = ptr[lo_of(chunk0 + cIssue)];
+            ne = ptr[lo_of(chunk0 + cIssue + 1)];
+        }
+        const long long rnl = (chunk0 + cNext) * TH + tid;
+        const int rn = (int)min(rnl, (long long)0x7fffffff);
+        const bool validn = cNext < nChunks && rn >= rowBegin && rn < rowEnd;
+        if (!DICT && validn) {
+            pn = ptr[rn];
+            qn = ptr[rn + 1];
+        }
+        mbar_wait(&bar[s], (uint32_t)(k / S) & 1u);
+        const int *rec = sidx + (size_t)s * capI;
+        int len, vo, io = 0;
+        uint32_t m = 0;
+        if (DICT) {
+            const uint32_t mrow = reinterpret_cast<const uint16_t *>(rec + CS_DICT + TH / 32)[tid];
+            const int lane = tid & 31, cnt = __popc(mrow);
+            int inc = cnt;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int t = __shfl_up_sync(0xffffffffu, inc, o);
+                if (lane >= o) inc += t;
+            }
+            vo = s * capV + (rec[CS_DICT + (tid >> 5)] + inc - cnt - sbaseV[s]);
+            m = valid ? mrow : 0u;
+            len = __popc(m);
+        } else {
+            io = s * capI + (p - sbaseI[s]);
+            vo = s * capV + (p - sbaseV[s]);
+            len = q - p;
+        }
+        double acc[KP];
+#pragma unroll
+        for (int v = 0; v < KP; v++) acc[v] = 0.0;
+#pragma unroll
+        for (int j = 0; j < MAXL; j++)
+            if (j < len) {
+                int col;
+                if (DICT) {                                     // set bits low to high = ascending columns = idx order
+                    col = r + rec[__ffs(m) - 1];
+                    m &= m - 1;
+                } else {
+                    col = sidx[io + j];
+                }
+                double xv[KP];
+                ld_xrow<KP, W2>(xv, X + (long long)col * ldx, kv, pol_x);
+                const double a = sval[vo + j];
+#pragma unroll
+                for (int v = 0; v < KP; v++) acc[v] = __dadd_rn(acc[v], __dmul_rn(a, xv[v]));
+            }
+        if (valid) {
+            double *yr = Y + (long long)r * ldy;
+#pragma unroll
+            for (int v = 0; v < KP; v++)
+                if (v < kv) yr[v] = acc[v];
+        }
+        __syncthreads();
+        if (tid == 0 && cIssue < nChunks) issue(s, chunk0 + cIssue, nb, ne);
+        r = rn; p = pn; q = qn; valid = validn;
+    }
+}
+
 __global__ void chunk_cap_kernel(const int *__restrict__ ptr, int nRow, int th, int nChunks, int *__restrict__ out)
 {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
@@ -314,6 +436,65 @@ int ChunkStream::run_f32(const float *x, float *y, int rb, int re, int acc, bool
     if (rb == re) return B200SPMV_OK;
     if (acc64) return cs_dispatch<float, float, double>(*this, x, y, rb, re, acc, s);
     return cs_dispatch<float, float, float>(*this, x, y, rb, re, acc, s);
+}
+
+// the multi-vector launch: stages, grid and occupancy as in cs_launch
+template <int MAXL, int TH, bool DICT, int KP, bool W2>
+static int cs_multi_launch(const ChunkStream &c, int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s)
+{
+    constexpr int S = 2;
+    const int capI = DICT ? CS_META_INTS(TH) : (c.cap + 8) & ~3, capV = (c.cap + 4) & ~1;
+    const size_t smem = (size_t)S * ((size_t)capI * 4 + (size_t)capV * sizeof(double));
+    auto kern = chunk_stream_multi_kernel<MAXL, TH, DICT, KP, W2>;
+    static int sms = 0;
+    static std::map<std::pair<int, size_t>, int> per_sm;
+    int dev = 0;
+    B2_CUDA(cudaGetDevice(&dev));
+    if (!sms) B2_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const auto key = std::make_pair(dev, smem);
+    auto it = per_sm.find(key);
+    if (it == per_sm.end()) {
+        B2_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 200 * 1024)));
+        int n = 0;
+        B2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kern, TH, smem));
+        if (n < 1) { set_error("row-chunk stream: %zu bytes of shared memory do not fit", smem); return B200SPMV_ERR_UNSUPPORTED; }
+        it = per_sm.emplace(key, n).first;
+    }
+    const int nChunks = ceil_div(c.nRow, TH);
+    const int grid = std::min(nChunks, sms * it->second);
+    kern<<<grid, TH, smem, s>>>(c.ptr, c.idx, c.meta.p, static_cast<const double *>(c.val), X, ldx, Y, ldy, k, 0, c.nRow, 0,
+                                nChunks, capI, capV, S);
+    B2_KERNEL_CHECK();
+    return B200SPMV_OK;
+}
+
+template <int MAXL, int TH, bool DICT>
+static int cs_multi_k(const ChunkStream &c, int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s)
+{
+    const bool w2 = (ldx & 1) == 0 && (reinterpret_cast<uintptr_t>(X) & 15) == 0;
+#define CS_MK(KP)                                                                                              \
+    return w2 ? cs_multi_launch<MAXL, TH, DICT, KP, true>(c, k, X, ldx, Y, ldy, s)                             \
+              : cs_multi_launch<MAXL, TH, DICT, KP, false>(c, k, X, ldx, Y, ldy, s)
+    if (k == 1) return cs_multi_launch<MAXL, TH, DICT, 1, false>(c, k, X, ldx, Y, ldy, s);
+    if (k == 2) CS_MK(2);
+    if (k <= 4) CS_MK(4);
+    CS_MK(8);
+#undef CS_MK
+}
+
+template <int MAXL, int TH>
+static int cs_multi_feed(const ChunkStream &c, int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s)
+{
+    if (c.feed == CS_FEED_DICT) return cs_multi_k<MAXL, TH, true>(c, k, X, ldx, Y, ldy, s);
+    return cs_multi_k<MAXL, TH, false>(c, k, X, ldx, Y, ldy, s);
+}
+
+int ChunkStream::run_multi(int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s) const
+{
+    if (f32) { set_error("multiply_multi: the row-chunk stream holds fp32 values"); return B200SPMV_ERR_UNSUPPORTED; }
+    if (nRow == 0) return B200SPMV_OK;
+    if (th == 512) return maxLen <= 8 ? cs_multi_feed<8, 512>(*this, k, X, ldx, Y, ldy, s) : cs_multi_feed<16, 512>(*this, k, X, ldx, Y, ldy, s);
+    return maxLen <= 8 ? cs_multi_feed<8, 256>(*this, k, X, ldx, Y, ldy, s) : cs_multi_feed<16, 256>(*this, k, X, ldx, Y, ldy, s);
 }
 
 }  // namespace b2

@@ -46,6 +46,9 @@ struct ChunkStream {
               cudaStream_t s);
     int run(const double *x, double *y, int rb, int re, int acc, cudaStream_t s) const;
     int run_f32(const float *x, float *y, int rb, int re, int acc, bool acc64, cudaStream_t s) const;
+    // Y[:, 0..k) := A X[:, 0..k) (k <= 8, row-major with leading dimensions ldx, ldy; fp64 values): the same chunks, one
+    // thread per row summing every vector in the order of run(), so each column of Y has the bits of run() on that column
+    int run_multi(int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s) const;
 };
 
 }  // namespace b2

@@ -94,6 +94,12 @@ struct Format {
         set_error("multiply_f32: this format has no fp32 variant (CRS, ELL and DIA do)");
         return B200SPMV_ERR_UNSUPPORTED;
     }
+    // Y[:, 0..k) := A X[:, 0..k), X and Y row-major with leading dimensions ldx, ldy (b200spmv_multiply_multi)
+    virtual int multiply_multi(int, const double *, long long, double *, long long, cudaStream_t)
+    {
+        set_error("multiply_multi: this format has no multi-vector multiply (CRS has)");
+        return B200SPMV_ERR_UNSUPPORTED;
+    }
     virtual int multiply_rows(int, int, const double *, double *, cudaStream_t)
     {
         set_error("multiply_rows: this format does not support row ranges (CRS, SS, CSS, ELL, DIA do)");
@@ -145,6 +151,8 @@ int sum_i32_as_i64(const int *in_d, int n, long long *out_h, cudaStream_t s);
 int minmax_i32(const int *in_d, long long b, long long e, int *mn_h, int *mx_h);
 // largest |col - row| (synchronises); gathers_need_l2: the x entries a stretch of rows touches span more than 32 MB
 int max_band(const int *row_d, const int *col_d, int nnz, int rowOffset, int *band_h, cudaStream_t s);
+// the same from a CRS matrix (columns ascending within a row: a row's first and last entry are its extremes)
+int max_band_crs(const int *ptr_d, const int *idx_d, int nRow, int rowOffset, int *band_h, cudaStream_t s);
 bool gathers_need_l2(int band);
 // checks the input contract: sorted by (row, col), no duplicates, indices in range
 int validate_sorted_coo(const CooView &A, cudaStream_t s);
@@ -255,6 +263,41 @@ __device__ __forceinline__ float ld_x(const float *p, uint64_t pol)
     float r;
     asm volatile("ld.global.nc.L2::cache_hint.f32 %0, [%1], %2;" : "=f"(r) : "l"(p), "l"(pol));
     return r;
+}
+
+// Gathers of the multi-vector multiply (X row-major, X[c*ldx + j]): the hint of ld_x, but not volatile, so that the
+// compiler may batch the loads of several entries.  ld_xrow reads X[c*ldx + j0 + v] for v < min(KP, k - j0) (the other
+// slots read nothing and hold 0): with W2 (ldx even, X 16-byte aligned, j0 even) pairs of columns come in one 16-byte load.
+__device__ __forceinline__ double ld_xm(const double *p, uint64_t pol)
+{
+    double r;
+    asm("ld.global.nc.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(r) : "l"(p), "l"(pol));
+    return r;
+}
+__device__ __forceinline__ double2 ld_xm2(const double *p, uint64_t pol)
+{
+    double2 r;
+    asm("ld.global.nc.L2::cache_hint.v2.f64 {%0,%1}, [%2], %3;" : "=d"(r.x), "=d"(r.y) : "l"(p), "l"(pol));
+    return r;
+}
+template <int KP, bool W2>
+__device__ __forceinline__ void ld_xrow(double (&xv)[KP], const double *p, int n, uint64_t pol)
+{
+#pragma unroll
+    for (int v = 0; v < KP; v += W2 ? 2 : 1) {
+        if (W2 && v + 1 < KP) {
+            if (v + 1 < n) {
+                const double2 t = ld_xm2(p + v, pol);
+                xv[v] = t.x;
+                xv[v + 1] = t.y;
+            } else {
+                xv[v] = v < n ? ld_xm(p + v, pol) : 0.0;
+                xv[v + 1] = 0.0;
+            }
+        } else {
+            xv[v] = v < n ? ld_xm(p + v, pol) : 0.0;
+        }
+    }
 }
 
 __device__ __forceinline__ double warp_sum(double v)

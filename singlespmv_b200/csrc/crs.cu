@@ -33,12 +33,15 @@ struct CrsFormat : Format {
     EntryStream es;
     bool use_es = false;
     int path_opt;
+    int band = 0, rowOffset = 0;
+    bool band_known = false;              // conversion computes the band for crs_path 0 and 4 only
     int prec;                             // options.precision: 0 fp64 vectors, 1 fp32 vectors + sums, 2 fp32 vectors, fp64 sums
     explicit CrsFormat(const b200spmv_options &o) : f32(o.value_f32 != 0 || o.precision != 0), path_opt(o.crs_path), prec(o.precision) {}
 
     int convert(const CooView &A, cudaStream_t s) override
     {
         nRow = A.nRow; nCol = A.nCol; nnz = A.nnz;
+        rowOffset = A.rowOffset;
         B2_TRY(validate_sorted_coo(A, s));
         B2_TRY(ptr.alloc((size_t)nRow + 1));
         B2_TRY(idx.alloc((size_t)nnz + CS_SLACK));
@@ -60,8 +63,9 @@ struct CrsFormat : Format {
         // path: 1 = tile-stream always; otherwise the TMA-fed row-chunk stream when the rows are short enough, else the tile-stream
         // ... unless the gathers range over tens of MB (uniform random, R-MAT): x must stay in L2, which it does with the
         // tile-stream's evict-first loads and does not with bulk copies in flight (uniform 2^24 x 11: 40 G entries/s TMA-fed)
-        int band = 0;
-        if (path_opt == 0 || path_opt == 4) B2_TRY(max_band(A.row, A.col, nnz, A.rowOffset, &band, s));
+        band = 0;
+        band_known = path_opt == 0 || path_opt == 4;
+        if (band_known) B2_TRY(max_band(A.row, A.col, nnz, A.rowOffset, &band, s));
         short_rows = path_opt != 1 && path_opt != 4 && cs.ok && !gathers_need_l2(band);
         // gather-bound matrices (fp64): the load-fed entry stream (entry_stream.cuh) -- c3 441 GFLOP/s against 365 for the tile-stream
         // (cuSPARSE CSR: 405).  Banded matrices with medium rows keep the tile-stream: the TMA-fed entry stream is level with it
@@ -93,6 +97,30 @@ struct CrsFormat : Format {
         if (rb == re) return B200SPMV_OK;
         return cs.run(x, y, rb, re, CS_OVERWRITE, s);
     }
+    // Row-chunk stream and entry stream handles run their own kernel's K-vector form.  Tile-stream handles (rows longer
+    // than the row-chunk stream takes, crs_path = 1) run the entry stream's, whose metadata the first call builds.
+    int multiply_multi(int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s) override
+    {
+        if (f32) { set_error("multiply_multi: fp64 values and vectors only (value_f32 = 0, precision = 0)"); return B200SPMV_ERR_UNSUPPORTED; }
+        if (short_rows) return cs.run_multi(k, X, ldx, Y, ldy, s);
+        if (nnz == 0) return zero_rows_multi(nRow, k, Y, ldy, s);
+        if (!use_es && !es.ok) {
+            cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+            if (cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone) {
+                set_error("multiply_multi: first call on a tile-stream handle inside a stream capture; call it once outside the capture first");
+                return B200SPMV_ERR_STATE;
+            }
+            B2_TRY(ensure_band(s));
+            B2_TRY(es.build(ptr.p, idx.p, val.p, nRow, nnz, gathers_need_l2(band), s));
+        }
+        return es.run_multi(k, X, ldx, Y, ldy, s);
+    }
+    int ensure_band(cudaStream_t s)
+    {
+        if (!band_known) B2_TRY(max_band_crs(ptr.p, idx.p, nRow, rowOffset, &band, s));
+        band_known = true;
+        return B200SPMV_OK;
+    }
     bool has_rows() const override { return !prec; }   // multiply_rows has no fp32-vector variant
     int prepare_rows(int rb, int re) override { return short_rows ? B200SPMV_OK : use_es ? es.prepare(rb, re) : ts.prepare(rb, re); }
     int col_extent(int rb, int re, int *cmin, int *cmax) override
@@ -113,6 +141,16 @@ struct CrsFormat : Format {
         }
         if (n == "launches") { *out = short_rows ? 1 : use_es ? (es.nTiles > 1 ? 2 : 1) + (es.nEmpty ? 1 : 0) : (ts.nTiles > 1 ? 2 : 1); return true; }
         if (n == "crs_kernel") { *out = short_rows ? 1 : use_es ? (es.tma ? 2 : 3) : 0; return true; }   // 0 tile-stream, 1 row-chunk stream, 2 / 3 entry stream (TMA- / load-fed)
+        if (n == "multi_kernel") {   // b200spmv_multiply_multi: 1 row-chunk stream, 2 / 3 entry stream TMA- / load-fed, 0 none
+            if (f32) *out = 0;
+            else if (short_rows) *out = 1;
+            else if (use_es) *out = es.tma ? 2 : 3;
+            else {
+                if (ensure_band(nullptr) != B200SPMV_OK) return false;
+                *out = gathers_need_l2(band) ? 3 : 2;
+            }
+            return true;
+        }
         if (n == "maxLength") { *out = maxLen; return true; }
         if (n == "short_row_path") { *out = short_rows ? 1 : 0; return true; }
         if (n == "chunk_feed") { *out = short_rows ? cs.feed : CS_FEED_IDX; return true; }   // row-chunk stream: 0 idx / ptr, 1 offset dictionary

@@ -267,12 +267,274 @@ __global__ void entry_stream_fixup_kernel(const unsigned *__restrict__ bits, con
     if (r >= rowLo && r < rowHi) y[r] = __dadd_rn(y[r], sum);
 }
 
+// ---------------------------------------------------------------- multiply of k <= ES_KMAX vectors (X, Y row-major)
+// The kernel above with every sum carried for KP vectors at once: the entry stream, start bits, ballots and scans are
+// shared, the lane gathers the KP values of a column in one row of X (ld_xrow).  k > KP: the tile is reduced once per
+// group of KP vectors (TMA-fed from the same stage, load-fed from L2).  Carries: carry[t * k + j].
+template <bool TMA, int KP, bool W2>
+__global__ void __launch_bounds__(ES_THREADS)
+entry_stream_multi_kernel(const int *__restrict__ idx, const double *__restrict__ val, const unsigned *__restrict__ bits,
+                          const int *__restrict__ grpRun, const int *__restrict__ nzrow, const double *__restrict__ X,
+                          long long ldx, double *__restrict__ Y, long long ldy, int kv, double *__restrict__ carry, int nnz,
+                          int tileLo, int tileHi, int rowLo, int rowHi)
+{
+    constexpr int E = ES_E;
+    constexpr int CHUNK = E / ES_WARPS;
+    constexpr int GROUPS = CHUNK / 128;
+    extern __shared__ __align__(128) unsigned char es_smem[];
+    __shared__ __align__(8) uint64_t full[2];
+    __shared__ double rPiece[ES_WARPS][ES_KMAX], rTail[ES_WARPS][ES_KMAX];
+    __shared__ int rRun[ES_WARPS];
+    int *scol = reinterpret_cast<int *>(es_smem);
+    double *sval = reinterpret_cast<double *>(es_smem + 2 * E * sizeof(int));
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const uint64_t pol_stream = policy_evict_first(), pol_x = policy_evict_last();
+    const unsigned lt = (1u << lane) - 1u;
+
+    auto row_of = [&](int run) { return nzrow ? nzrow[run] : run; };
+    auto store = [&](int run, int j0, const double (&a)[KP]) {
+        const int r = row_of(run);
+        if (r >= rowLo && r < rowHi) {
+            double *yr = Y + (long long)r * ldy + j0;
+#pragma unroll
+            for (int v = 0; v < KP; v++)
+                if (j0 + v < kv) yr[v] = a[v];
+        }
+    };
+    auto issue = [&](int s, int t) {
+        const long long t0 = (long long)t * E;
+        const int n = (int)min((long long)E, (long long)nnz - t0);
+        const uint32_t b4 = (uint32_t)((n * 4 + 15) & ~15), b8 = (uint32_t)(n * 8 + 15) & ~15u;
+        mbar_expect_tx(&full[s], b4 + b8);
+        tma_load_1d(scol + s * E, idx + t0, b4, &full[s], pol_stream);
+        tma_load_1d(sval + s * E, val + t0, b8, &full[s], pol_stream);
+    };
+    const int first = tileLo + blockIdx.x;
+    if (TMA) {
+        if (tid == 0) { mbar_init(&full[0], 1); mbar_init(&full[1], 1); }
+        __syncthreads();
+        if (tid == 0) {
+            if (first < tileHi) issue(0, first);
+            if (first + (int)gridDim.x < tileHi) issue(1, first + gridDim.x);
+        }
+    }
+    int k = 0;
+    for (int t = first; t < tileHi; t += gridDim.x, k++) {
+        const int s = k & 1;
+        const long long t0 = (long long)t * E;
+        const int n = (int)min((long long)E, (long long)nnz - t0);
+        const int c0 = warp * CHUNK;
+        const int nGroups = c0 < n ? min(GROUPS, (n - c0 + 127) >> 7) : 0;
+        const int nw = min(ES_WARPS, (n + CHUNK - 1) / CHUNK);
+        if (TMA) mbar_wait(&full[s], (uint32_t)(k >> 1) & 1u);
+        const int *Cc = TMA ? scol + s * E : idx + t0;
+        const double *V = TMA ? sval + s * E : val + t0;
+        for (int j0 = 0; j0 < kv && nGroups > 0; j0 += KP) {
+            bool started = false;
+            double cin[KP], piece[KP];
+#pragma unroll
+            for (int v = 0; v < KP; v++) cin[v] = piece[v] = 0.0;
+            int lastRun = -1;
+#pragma unroll
+            for (int g = 0; g < GROUPS; g++) {
+                if (g >= nGroups) break;
+                const int e = c0 + g * 128 + 4 * lane;
+                const long long ge = t0 + e;
+                int4 c;
+                double2 v0, v1;
+                if (c0 + g * 128 + 128 <= n) {
+                    if (TMA) {
+                        c = *reinterpret_cast<const int4 *>(Cc + e);
+                        v0 = *reinterpret_cast<const double2 *>(V + e);
+                        v1 = *reinterpret_cast<const double2 *>(V + e + 2);
+                    } else {
+                        c = ld_stream_i4(Cc + e, pol_stream);
+                        v0 = ld_stream_d2(V + e, pol_stream);
+                        v1 = ld_stream_d2(V + e + 2, pol_stream);
+                    }
+                } else {
+                    c.x = e < n ? Cc[e] : 0; c.y = e + 1 < n ? Cc[e + 1] : 0; c.z = e + 2 < n ? Cc[e + 2] : 0; c.w = e + 3 < n ? Cc[e + 3] : 0;
+                    v0.x = e < n ? V[e] : 0.0; v0.y = e + 1 < n ? V[e + 1] : 0.0; v1.x = e + 2 < n ? V[e + 2] : 0.0; v1.y = e + 3 < n ? V[e + 3] : 0.0;
+                }
+                const unsigned word = __ldg(bits + (ge >> 5));
+                const unsigned b = (word >> (unsigned)(ge & 31)) & 0xFu;
+                const int base = __ldg(grpRun + (ge >> 7));
+                double p0[KP], p1[KP], p2[KP], p3[KP];
+                ld_xrow<KP, W2>(p0, X + (long long)c.x * ldx + j0, kv - j0, pol_x);
+                ld_xrow<KP, W2>(p1, X + (long long)c.y * ldx + j0, kv - j0, pol_x);
+                ld_xrow<KP, W2>(p2, X + (long long)c.z * ldx + j0, kv - j0, pol_x);
+                ld_xrow<KP, W2>(p3, X + (long long)c.w * ldx + j0, kv - j0, pol_x);
+#pragma unroll
+                for (int v = 0; v < KP; v++) {
+                    p0[v] = __dmul_rn(v0.x, p0[v]); p1[v] = __dmul_rn(v0.y, p1[v]);
+                    p2[v] = __dmul_rn(v1.x, p2[v]); p3[v] = __dmul_rn(v1.y, p3[v]);
+                }
+                const bool b0 = b & 1u, b1 = b & 2u, b2 = b & 4u, b3 = b & 8u;
+                const bool has = b != 0u;
+                const int nStarts = __popc(b);
+                const unsigned m = __ballot_sync(0xffffffffu, has);
+                int runOpen = base - 1 + __popc(m & lt);
+                double head[KP], acc[KP];
+                if (__any_sync(0xffffffffu, nStarts > 1)) {
+                    const unsigned m0 = __ballot_sync(0xffffffffu, b0), m1 = __ballot_sync(0xffffffffu, b1),
+                                   m2 = __ballot_sync(0xffffffffu, b2), m3 = __ballot_sync(0xffffffffu, b3);
+                    runOpen = base - 1 + __popc(m0 & lt) + __popc(m1 & lt) + __popc(m2 & lt) + __popc(m3 & lt);
+#pragma unroll
+                    for (int v = 0; v < KP; v++) head[v] = acc[v] = 0.0;
+                    bool seen = false;
+                    int run = runOpen;
+                    auto step = [&](bool st, const double (&p)[KP]) {
+                        if (st) {
+                            if (!seen) {
+#pragma unroll
+                                for (int v = 0; v < KP; v++) head[v] = acc[v];
+                            } else {
+                                store(run, j0, acc);
+                            }
+                            seen = true;
+                            run++;
+#pragma unroll
+                            for (int v = 0; v < KP; v++) acc[v] = p[v];
+                        } else {
+#pragma unroll
+                            for (int v = 0; v < KP; v++) acc[v] = __dadd_rn(acc[v], p[v]);
+                        }
+                    };
+                    step(b0, p0); step(b1, p1); step(b2, p2); step(b3, p3);
+                } else {
+                    const bool f0 = b0, f1 = f0 | b1, f2 = f1 | b2;
+#pragma unroll
+                    for (int v = 0; v < KP; v++) {
+                        head[v] = __dadd_rn(__dadd_rn((has && !f0) ? p0[v] : 0.0, (has && !f1) ? p1[v] : 0.0), (has && !f2) ? p2[v] : 0.0);
+                        acc[v] = __dadd_rn(__dadd_rn(__dadd_rn((!has || f0) ? p0[v] : 0.0, (!has || f1) ? p1[v] : 0.0), (!has || f2) ? p2[v] : 0.0), p3[v]);
+                    }
+                }
+                const unsigned below = m & (0xffffffffu >> (31 - lane));
+                const int seg = below ? 31 - __clz(below) : 0;
+                unsigned cov = m | 1u;
+                cov |= cov << 1;
+                int steps = 1;
+                if (cov != 0xffffffffu) {
+                    cov |= cov << 2; steps = 2;
+                    if (cov != 0xffffffffu) {
+                        cov |= cov << 4; steps = 3;
+                        if (cov != 0xffffffffu) { cov |= cov << 8; steps = cov != 0xffffffffu ? 5 : 4; }
+                    }
+                }
+                double sc[KP];                                  // the segmented scan, per vector
+#pragma unroll
+                for (int v = 0; v < KP; v++) sc[v] = acc[v];
+#pragma unroll
+                for (int i = 0; i < 5; i++) {
+                    if (i < steps) {
+                        const int d = 1 << i;
+#pragma unroll
+                        for (int v = 0; v < KP; v++) {
+                            const double u = __shfl_up_sync(0xffffffffu, sc[v], d);
+                            if (lane - d >= seg) sc[v] = __dadd_rn(sc[v], u);
+                        }
+                    }
+                }
+                const bool firstInChunk = !started && !(m & lt);
+                double tot[KP];
+#pragma unroll
+                for (int v = 0; v < KP; v++) {
+                    if (!below) sc[v] = __dadd_rn(sc[v], cin[v]);
+                    double excl = __shfl_up_sync(0xffffffffu, sc[v], 1);
+                    if (lane == 0) excl = cin[v];
+                    tot[v] = __dadd_rn(excl, head[v]);
+                    if (has && firstInChunk) piece[v] = tot[v];
+                }
+                if (has && !firstInChunk) store(runOpen, j0, tot);
+#pragma unroll
+                for (int v = 0; v < KP; v++) {
+                    if (!started && m) piece[v] = __shfl_sync(0xffffffffu, piece[v], __ffs(m) - 1);
+                    cin[v] = __shfl_sync(0xffffffffu, sc[v], 31);
+                }
+                lastRun = __shfl_sync(0xffffffffu, runOpen + nStarts, 31);
+                started = started || m != 0u;
+            }
+            if (lane == 0) {
+#pragma unroll
+                for (int v = 0; v < KP; v++)
+                    if (j0 + v < kv) {
+                        rPiece[warp][j0 + v] = started ? piece[v] : cin[v];
+                        rTail[warp][j0 + v] = cin[v];
+                    }
+                rRun[warp] = started ? lastRun : -1;
+            }
+        }
+        __syncthreads();                                    // every warp is done with stage s, the chunk records are in place
+        if (tid >= 32 && tid < 32 + kv) {                   // one thread per vector stitches the chunks of the tile
+            const int j = tid - 32;
+            double tilePiece = 0.0, a2 = 0.0;
+            int accRun = -1;
+            auto put = [&](int run, double v) {
+                const int r = row_of(run);
+                if (r >= rowLo && r < rowHi) Y[(long long)r * ldy + j] = v;
+            };
+            for (int w = 0; w < nw; w++) {
+                const double oPiece = rPiece[w][j], oTail = rTail[w][j];
+                const int oRun = rRun[w];
+                if (accRun >= 0) a2 = __dadd_rn(a2, oPiece);
+                else tilePiece = __dadd_rn(tilePiece, oPiece);
+                if (oRun >= 0) {
+                    if (accRun >= 0) put(accRun, a2);
+                    accRun = oRun;
+                    a2 = oTail;
+                }
+            }
+            if (accRun >= 0) put(accRun, a2);
+            carry[(long long)t * kv + j] = tilePiece;
+        }
+        __syncthreads();                                    // the records are read before the next tile's warps rewrite them
+        if (TMA && tid == 0 && t + 2 * (int)gridDim.x < tileHi) issue(s, t + 2 * gridDim.x);
+    }
+}
+
+// one thread per (tile, vector): entry_stream_fixup_kernel on column j of Y
+__global__ void entry_stream_multi_fixup_kernel(const unsigned *__restrict__ bits, const int *__restrict__ grpRun,
+                                                const int *__restrict__ nzrow, double *__restrict__ Y, long long ldy, int kv,
+                                                const double *__restrict__ carry, int E, int tileLo, int tileHi)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int t = tileLo + 1 + (int)(i / kv), j = (int)(i % kv);
+    if (t >= tileHi) return;
+    auto first_bit = [&](int u) { const long long e = (long long)u * E; return (bits[e >> 5] >> (unsigned)(e & 31)) & 1u; };
+    auto run_at = [&](int u) { return grpRun[((long long)u * E) >> 7] - 1 + (int)first_bit(u); };
+    if (first_bit(t)) return;
+    const int run = run_at(t);
+    if (!first_bit(t - 1) && run_at(t - 1) == run) return;
+    double sum = 0.0;
+    for (int u = t; u < tileHi && !first_bit(u) && run_at(u) == run; u++) sum = __dadd_rn(sum, carry[(long long)u * kv + j]);
+    double *yr = Y + (long long)(nzrow ? nzrow[run] : run) * ldy + j;
+    *yr = __dadd_rn(*yr, sum);
+}
+
+// Y[r, j] = 0 for the listed rows (all rows [0, n) when rows == NULL) and j < k
+__global__ void es_zero_rows_multi_kernel(const int *__restrict__ rows, int n, int kv, double *__restrict__ Y, long long ldy)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (long long)n * kv) return;
+    const int q = (int)(i / kv);
+    Y[(long long)(rows ? rows[q] : q) * ldy + (int)(i % kv)] = 0.0;
+}
+
+int zero_rows_multi(int nRow, int k, double *Y, long long ldy, cudaStream_t s)
+{
+    if (nRow <= 0) return B200SPMV_OK;
+    es_zero_rows_multi_kernel<<<ceil_div((long long)nRow * k, 256), 256, 0, s>>>(nullptr, nRow, k, Y, ldy);
+    B2_KERNEL_CHECK();
+    return B200SPMV_OK;
+}
+
 int EntryStream::build(const int *ptr_d, const int *idx_d, const double *val_d, int nRow_, int nnz_, bool gather_bound,
                        cudaStream_t s)
 {
     ptr = ptr_d; idx = idx_d; val = val_d; nRow = nRow_; nnz = nnz_;
     ok = false;
     range_cache.clear();
+    carryK.release();
     if (nnz <= 0 || nRow <= 0) return B200SPMV_OK;
     tma = !gather_bound;
     nTiles = ceil_div(nnz, ES_E);
@@ -378,6 +640,66 @@ int EntryStream::run_rows(const double *x, double *y, int rb, int re, cudaStream
     if (hi <= lo) return B200SPMV_OK;
     if (tma) return es_launch<true>(*this, x, y, lo, hi, rb, re, s);
     return es_launch<false>(*this, x, y, lo, hi, rb, re, s);
+}
+
+template <bool TMA, int KP, bool W2>
+static int es_multi_launch(EntryStream &T, int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s)
+{
+    constexpr size_t smem = TMA ? 24 * (size_t)ES_E : 0;
+    auto kern = entry_stream_multi_kernel<TMA, KP, W2>;
+    static std::map<int, int> per_sm;
+    static int sms = 0;
+    int dev = 0;
+    B2_CUDA(cudaGetDevice(&dev));
+    if (!sms) B2_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    auto it = per_sm.find(dev);
+    if (it == per_sm.end()) {
+        if (smem) B2_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        int n = 0;
+        B2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kern, ES_THREADS, smem));
+        if (n < 1) { set_error("entry stream: %zu bytes of shared memory do not fit", smem); return B200SPMV_ERR_UNSUPPORTED; }
+        it = per_sm.emplace(dev, n).first;
+    }
+    const int nT = T.nTiles;
+    const int grid = TMA ? std::min(nT, sms * std::min(it->second, 6)) : nT;
+    kern<<<grid, ES_THREADS, smem, s>>>(T.idx, T.val, T.bits.p, T.grpRun.p, T.nEmpty ? T.nzrow.p : nullptr, X, ldx, Y, ldy, k,
+                                        T.carryK.p, T.nnz, 0, nT, 0, T.nRow);
+    B2_KERNEL_CHECK();
+    if (nT > 1) {
+        entry_stream_multi_fixup_kernel<<<ceil_div((long long)(nT - 1) * k, 256), 256, 0, s>>>(
+            T.bits.p, T.grpRun.p, T.nEmpty ? T.nzrow.p : nullptr, Y, ldy, k, T.carryK.p, ES_E, 0, nT);
+        B2_KERNEL_CHECK();
+    }
+    return B200SPMV_OK;
+}
+
+template <bool TMA>
+static int es_multi_k(EntryStream &T, int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s)
+{
+    const bool w2 = (ldx & 1) == 0 && (reinterpret_cast<uintptr_t>(X) & 15) == 0;
+    if (k == 1) return es_multi_launch<TMA, 1, false>(T, k, X, ldx, Y, ldy, s);
+    if (k == 2) return w2 ? es_multi_launch<TMA, 2, true>(T, k, X, ldx, Y, ldy, s) : es_multi_launch<TMA, 2, false>(T, k, X, ldx, Y, ldy, s);
+    return w2 ? es_multi_launch<TMA, 4, true>(T, k, X, ldx, Y, ldy, s) : es_multi_launch<TMA, 4, false>(T, k, X, ldx, Y, ldy, s);
+}
+
+int EntryStream::run_multi(int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s)
+{
+    if (k < 1 || k > ES_KMAX) { set_error("multiply_multi: k=%d outside 1..%d", k, ES_KMAX); return B200SPMV_ERR_INVALID; }
+    if (!ok) return zero_rows_multi(nRow, k, Y, ldy, s);      // no entries
+    if (!carryK.p) {
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        if (cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone) {
+            set_error("multiply_multi: first call on this handle inside a stream capture; call it once outside the capture first");
+            return B200SPMV_ERR_STATE;
+        }
+        B2_TRY(carryK.alloc((size_t)nTiles * ES_KMAX));
+    }
+    if (nEmpty) {
+        es_zero_rows_multi_kernel<<<ceil_div((long long)nEmpty * k, 256), 256, 0, s>>>(empty.p, nEmpty, k, Y, ldy);
+        B2_KERNEL_CHECK();
+    }
+    if (tma) return es_multi_k<true>(*this, k, X, ldx, Y, ldy, s);
+    return es_multi_k<false>(*this, k, X, ldx, Y, ldy, s);
 }
 
 }  // namespace b2

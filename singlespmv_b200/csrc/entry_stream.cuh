@@ -22,6 +22,10 @@ namespace b2 {
 
 // entries per tile: c4 (TMA-fed) 659 against 620 GFLOP/s with 1024; c3 (load-fed) 418 against 411
 constexpr int ES_E = 2048;
+constexpr int ES_KMAX = 8;         // vectors of one multi-vector multiply
+
+// Y[r, j] = 0 for r < nRow, j < k (row-major Y): the multi-vector multiply of a matrix without entries
+int zero_rows_multi(int nRow, int k, double *Y, long long ldy, cudaStream_t s);
 
 struct EntryStream {
     // borrowed
@@ -34,12 +38,16 @@ struct EntryStream {
     DevBuf<unsigned> bits;
     DevBuf<int> grpRun, nzrow, empty;
     DevBuf<double> carry;
+    DevBuf<double> carryK;             // nTiles x ES_KMAX carries of run_multi, allocated by its first call
     std::map<std::pair<int, int>, std::pair<int, int>> range_cache;
 
     // gather_bound: the x gathers need L2 residency (primitives.cu gathers_need_l2) -> load-fed, else TMA-fed
     int build(const int *ptr_d, const int *idx_d, const double *val_d, int nRow_, int nnz_, bool gather_bound, cudaStream_t s);
     int prepare(int rb, int re);
     int run_rows(const double *x, double *y, int rb, int re, cudaStream_t s);
+    // Y[:, 0..k) := A X[:, 0..k) over all rows (k <= ES_KMAX, row-major); each column is summed as run_rows sums it.
+    // The first call allocates the carries: refused with B200SPMV_ERR_STATE inside a stream capture.
+    int run_multi(int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s);
 };
 
 }  // namespace b2

@@ -187,6 +187,31 @@ int max_band(const int *row_d, const int *col_d, int nnz, int rowOffset, int *ba
     B2_CUDA(cudaStreamSynchronize(s));
     return B200SPMV_OK;
 }
+__global__ void band_crs_kernel(const int *__restrict__ ptr, const int *__restrict__ idx, int nRow, int rowOffset,
+                                int *__restrict__ out)
+{
+    int m = 0;
+    for (int r = blockIdx.x * blockDim.x + threadIdx.x; r < nRow; r += gridDim.x * blockDim.x) {
+        const int b = ptr[r], e = ptr[r + 1];
+        if (e > b) m = max(m, max(abs(idx[b] - (r + rowOffset)), abs(idx[e - 1] - (r + rowOffset))));
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
+    if ((threadIdx.x & 31) == 0 && m > 0) atomicMax(out, m);
+}
+int max_band_crs(const int *ptr_d, const int *idx_d, int nRow, int rowOffset, int *band_h, cudaStream_t s)
+{
+    *band_h = 0;
+    if (nRow <= 0) return B200SPMV_OK;
+    DevBuf<int> b;
+    B2_TRY(b.alloc(1));
+    B2_CUDA(cudaMemsetAsync(b.p, 0, sizeof(int), s));
+    band_crs_kernel<<<std::min(ceil_div(nRow, 256), 4096), 256, 0, s>>>(ptr_d, idx_d, nRow, rowOffset, b.p);
+    B2_KERNEL_CHECK();
+    B2_CUDA(cudaMemcpyAsync(band_h, b.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+    B2_CUDA(cudaStreamSynchronize(s));
+    return B200SPMV_OK;
+}
 bool gathers_need_l2(int band) { return 8LL * band > (32LL << 20); }
 
 // ---------------------------------------------------------------- input contract

@@ -157,6 +157,11 @@ class SpMatOpt:
     def multiply(self, x_ptr, y_ptr, stream=None):
         check(lib.b200spmv_multiply(self.h, C.c_void_p(x_ptr), C.c_void_p(y_ptr), stream))
 
+    def multiply_multi(self, k, X_ptr, ldx, Y_ptr, ldy, stream=None):
+        """Y[:, :k] := A X[:, :k] for k = 1..8 device-resident row-major vectors (X[c*ldx + j], Y[r*ldy + j]): the matrix is
+        streamed once for all k.  CRS handles with fp64 values and vectors (b200spmv_multiply_multi)."""
+        check(lib.b200spmv_multiply_multi(self.h, k, C.c_void_p(X_ptr), ldx, C.c_void_p(Y_ptr), ldy, stream))
+
     def multiply_rows(self, row_begin, row_end, x_ptr, y_ptr, stream=None):
         check(lib.b200spmv_multiply_rows(self.h, row_begin, row_end, C.c_void_p(x_ptr), C.c_void_p(y_ptr), stream))
 
