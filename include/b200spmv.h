@@ -148,6 +148,24 @@ B200SPMV_API int b200spmv_multiply_host(b200spmv_matrix *m, const double *x_h, d
  * vendors does: CSR5_cuda/Makefile:4 VALUE_TYPE).  The handle must have been created with that precision. */
 B200SPMV_API int b200spmv_multiply_f32(b200spmv_matrix *m, const float *x_d, float *y_d, void *stream);
 B200SPMV_API int b200spmv_multiply_host_f32(b200spmv_matrix *m, const float *x_h, float *y_h);
+/* Y[:, 0..k) := A * X[:, 0..k) for k = 1..8 fp32 vectors: b200spmv_multiply_multi for CRS handles created with precision
+ * = 1 or 2 (X[c*ldx + j], Y[r*ldy + j]; ldx, ldy >= k, in floats; the same rules for columns >= k, beta = 0 and streams).
+ * The matrix (4 B values) is streamed once, and one row of X -- up to 8 columns in one 32-byte sector -- is gathered once
+ * per entry; for one contiguous vector b200spmv_multiply_f32 is faster.  The kernel (scalar multi_kernel_f32: 1 row-chunk
+ * stream, 2 / 3 entry stream TMA- / load-fed, 0 on precision-0 handles and on matrices without entries):
+ *   - row-chunk stream handles: column j of Y has the bits of b200spmv_multiply_f32 on column j of X (one thread per row,
+ *     ascending column order, unfused mul / add in fp32 (precision 1) or fp64 (precision 2), rounded to fp32 once);
+ *   - every other handle (b200spmv_multiply_f32 runs the tile-stream there) runs the entry stream, whose metadata the first
+ *     call builds (it synchronises).  Sums are re-associated: precision 1 within (n+1) 2^-24 sum|a x| of the exact row sum,
+ *     precision 2 (fp64 products and sums, carried in fp64 across tiles, rounded to fp32 once) within 2^-24 |s| +
+ *     n 2^-53 sum|a x|.
+ * The first call on an entry-stream handle allocates per-handle buffers: made inside a stream capture it is refused with
+ * B200SPMV_ERR_STATE; later calls can be captured.  Errors, decided before any CUDA call and in this order:
+ * B200SPMV_ERR_INVALID (NULL handle, k outside 1..8, ldx or ldy < k), B200SPMV_ERR_UNSUPPORTED (formats other than CRS),
+ * B200SPMV_ERR_STATE (precision = 0, value_f32 handles included: use b200spmv_multiply_multi; before convert),
+ * B200SPMV_ERR_INVALID (NULL X or Y with nCol or nRow > 0). */
+B200SPMV_API int b200spmv_multiply_multi_f32(b200spmv_matrix *m, int k, const float *X_d, long long ldx,
+                                             float *Y_d, long long ldy, void *stream);
 /* Rows [rowBegin,rowEnd) only (CRS, SS, CSS, ELL, DIA; others return B200SPMV_ERR_UNSUPPORTED): used by
  * the row-partitioned multi-GPU path to overlap the interior block with the halo exchange, and by
  * b200spmv_multiply_host to overlap the D2H copy of finished rows with the rest of the multiply. */

@@ -54,6 +54,7 @@ def _load():
     lib.b200spmv_multiply.argtypes = [vp, vp, vp, vp]
     lib.b200spmv_multiply_host.argtypes = [vp, vp, vp]
     lib.b200spmv_multiply_multi.argtypes = [vp, ip, vp, ll, vp, ll, vp]
+    lib.b200spmv_multiply_multi_f32.argtypes = [vp, ip, vp, ll, vp, ll, vp]
     lib.b200spmv_multiply_f32.argtypes = [vp, vp, vp, vp]
     lib.b200spmv_multiply_host_f32.argtypes = [vp, vp, vp]
     lib.b200spmv_multiply_rows.argtypes = [vp, ip, ip, vp, vp, vp]

@@ -235,6 +235,24 @@ int b200spmv_multiply_multi(b200spmv_matrix *m, int k, const double *X_d, long l
     return m->impl->multiply_multi(k, X_d, ldx, Y_d, ldy, (cudaStream_t)stream);
 }
 
+int b200spmv_multiply_multi_f32(b200spmv_matrix *m, int k, const float *X_d, long long ldx, float *Y_d, long long ldy,
+                                void *stream)
+{
+    clear_error();
+    if (!m) { set_error("multiply_multi_f32: NULL handle"); return B200SPMV_ERR_INVALID; }
+    if (k < 1 || k > 8 || ldx < k || ldy < k) {
+        set_error("multiply_multi_f32: k=%d (1..8), ldx=%lld, ldy=%lld (>= k)", k, ldx, ldy);
+        return B200SPMV_ERR_INVALID;
+    }
+    if (m->format != B200SPMV_CRS) { set_error("multiply_multi_f32: CRS handles only (format %d)", m->format); return B200SPMV_ERR_UNSUPPORTED; }
+    if (!m->opt.precision) {
+        set_error("multiply_multi_f32: the handle was created with precision = 0 (fp64 vectors), use b200spmv_multiply_multi");
+        return B200SPMV_ERR_STATE;
+    }
+    B2_TRY(check_ready(m, X_d, Y_d));
+    return m->impl->multiply_multi_f32(k, X_d, ldx, Y_d, ldy, (cudaStream_t)stream);
+}
+
 int b200spmv_multiply_f32(b200spmv_matrix *m, const float *x_d, float *y_d, void *stream)
 {
     B2_TRY(check_ready(m, x_d, y_d));

@@ -108,6 +108,11 @@ struct RowBlocked : Format {
         for (size_t g = 0; g < blk.size(); g++) B2_TRY(blk[g]->multiply_multi(k, X, ldx, Y + (long long)rb[g] * ldy, ldy, s));
         return B200SPMV_OK;
     }
+    int multiply_multi_f32(int k, const float *X, long long ldx, float *Y, long long ldy, cudaStream_t s) override
+    {
+        for (size_t g = 0; g < blk.size(); g++) B2_TRY(blk[g]->multiply_multi_f32(k, X, ldx, Y + (long long)rb[g] * ldy, ldy, s));
+        return B200SPMV_OK;
+    }
     bool has_rows() const override
     {
         for (auto &b : blk) if (!b->has_rows()) return false;

@@ -130,13 +130,14 @@ chunk_stream_kernel(const int *__restrict__ ptr, const int *__restrict__ idx, co
     }
 }
 
-// The multi-vector form (fp64 values, overwrite): chunks arrive exactly as in chunk_stream_kernel, and the thread of row r
-// sums KP vectors (columns j < k of X; KP = k rounded up to 1, 2, 4, 8) over the row's entries in ascending column order,
-// each with the unfused mul / add of the single multiply.  W2: X rows gathered in 16-byte pairs (ld_xrow).
-template <int MAXL, int TH, bool DICT, int KP, bool W2>
+// The multi-vector form (overwrite; VT, XT, AT as in chunk_stream_kernel): chunks arrive exactly as in chunk_stream_kernel,
+// and the thread of row r sums KP vectors (columns j < k of X; KP = k rounded up to 1, 2, 4, 8) over the row's entries in
+// ascending column order, each with the unfused mul / add of the single multiply.  VEC: X rows gathered in 8- or 16-byte
+// pieces (ld_xrow).
+template <typename VT, typename XT, typename AT, int MAXL, int TH, bool DICT, int KP, bool VEC>
 __global__ void __launch_bounds__(TH, 1)
 chunk_stream_multi_kernel(const int *__restrict__ ptr, const int *__restrict__ idx, const int *__restrict__ meta,
-                          const double *__restrict__ val, const double *__restrict__ X, long long ldx, double *__restrict__ Y,
+                          const VT *__restrict__ val, const XT *__restrict__ X, long long ldx, XT *__restrict__ Y,
                           long long ldy, int kv, int rowBegin, int rowEnd, int chunk0, int nChunks, int capI, int capV, int S)
 {
     constexpr int MI = CS_META_INTS(TH);
@@ -144,18 +145,18 @@ chunk_stream_multi_kernel(const int *__restrict__ ptr, const int *__restrict__ i
     __shared__ __align__(8) uint64_t bar[CS_MAXSTAGES];
     __shared__ int sbaseI[CS_MAXSTAGES], sbaseV[CS_MAXSTAGES];
     int *sidx = reinterpret_cast<int *>(cs_smem);
-    double *sval = reinterpret_cast<double *>(cs_smem + (size_t)S * capI * sizeof(int));
+    VT *sval = reinterpret_cast<VT *>(cs_smem + (size_t)S * capI * sizeof(int));
     const int tid = threadIdx.x;
     const uint64_t pol_stream = policy_evict_first(), pol_x = policy_evict_last();
 
     auto issue = [&](int s, long long g, int b, int e) {
         const int *srcI = idx + b;
-        const double *srcV = val + b;
+        const VT *srcV = val + b;
         const int misI = (int)((reinterpret_cast<uintptr_t>(srcI) & 15) / sizeof(int));
-        const int misV = (int)((reinterpret_cast<uintptr_t>(srcV) & 15) / sizeof(double));
+        const int misV = (int)((reinterpret_cast<uintptr_t>(srcV) & 15) / sizeof(VT));
         const int n = e - b;
         const uint32_t bytesI = DICT ? (uint32_t)(MI * sizeof(int)) : n ? (uint32_t)(((n + misI) * (int)sizeof(int) + 15) & ~15) : 0u;
-        const uint32_t bytesV = n ? (uint32_t)(((n + misV) * (int)sizeof(double) + 15) & ~15) : 0u;
+        const uint32_t bytesV = n ? (uint32_t)(((n + misV) * (int)sizeof(VT) + 15) & ~15) : 0u;
         sbaseI[s] = b - misI;
         sbaseV[s] = b - misV;
         mbar_expect_tx(&bar[s], bytesI + bytesV);
@@ -221,9 +222,9 @@ chunk_stream_multi_kernel(const int *__restrict__ ptr, const int *__restrict__ i
             vo = s * capV + (p - sbaseV[s]);
             len = q - p;
         }
-        double acc[KP];
+        AT acc[KP];
 #pragma unroll
-        for (int v = 0; v < KP; v++) acc[v] = 0.0;
+        for (int v = 0; v < KP; v++) acc[v] = (AT)0;
 #pragma unroll
         for (int j = 0; j < MAXL; j++)
             if (j < len) {
@@ -234,17 +235,17 @@ chunk_stream_multi_kernel(const int *__restrict__ ptr, const int *__restrict__ i
                 } else {
                     col = sidx[io + j];
                 }
-                double xv[KP];
-                ld_xrow<KP, W2>(xv, X + (long long)col * ldx, kv, pol_x);
-                const double a = sval[vo + j];
+                XT xv[KP];
+                ld_xrow<KP, VEC>(xv, X + (long long)col * ldx, kv, pol_x);
+                const AT a = (AT)sval[vo + j];
 #pragma unroll
-                for (int v = 0; v < KP; v++) acc[v] = __dadd_rn(acc[v], __dmul_rn(a, xv[v]));
+                for (int v = 0; v < KP; v++) acc[v] = Arith<AT>::add(acc[v], Arith<AT>::mul(a, (AT)xv[v]));
             }
         if (valid) {
-            double *yr = Y + (long long)r * ldy;
+            XT *yr = Y + (long long)r * ldy;
 #pragma unroll
             for (int v = 0; v < KP; v++)
-                if (v < kv) yr[v] = acc[v];
+                if (v < kv) yr[v] = (XT)acc[v];
         }
         __syncthreads();
         if (tid == 0 && cIssue < nChunks) issue(s, chunk0 + cIssue, nb, ne);
@@ -439,13 +440,13 @@ int ChunkStream::run_f32(const float *x, float *y, int rb, int re, int acc, bool
 }
 
 // the multi-vector launch: stages, grid and occupancy as in cs_launch
-template <int MAXL, int TH, bool DICT, int KP, bool W2>
-static int cs_multi_launch(const ChunkStream &c, int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s)
+template <typename VT, typename XT, typename AT, int MAXL, int TH, bool DICT, int KP, bool VEC>
+static int cs_multi_launch(const ChunkStream &c, int k, const XT *X, long long ldx, XT *Y, long long ldy, cudaStream_t s)
 {
-    constexpr int S = 2;
-    const int capI = DICT ? CS_META_INTS(TH) : (c.cap + 8) & ~3, capV = (c.cap + 4) & ~1;
-    const size_t smem = (size_t)S * ((size_t)capI * 4 + (size_t)capV * sizeof(double));
-    auto kern = chunk_stream_multi_kernel<MAXL, TH, DICT, KP, W2>;
+    constexpr int S = 2, VA = 16 / (int)sizeof(VT);
+    const int capI = DICT ? CS_META_INTS(TH) : (c.cap + 8) & ~3, capV = (c.cap + 2 * VA) & ~(VA - 1);
+    const size_t smem = (size_t)S * ((size_t)capI * 4 + (size_t)capV * sizeof(VT));
+    auto kern = chunk_stream_multi_kernel<VT, XT, AT, MAXL, TH, DICT, KP, VEC>;
     static int sms = 0;
     static std::map<std::pair<int, size_t>, int> per_sm;
     int dev = 0;
@@ -462,39 +463,53 @@ static int cs_multi_launch(const ChunkStream &c, int k, const double *X, long lo
     }
     const int nChunks = ceil_div(c.nRow, TH);
     const int grid = std::min(nChunks, sms * it->second);
-    kern<<<grid, TH, smem, s>>>(c.ptr, c.idx, c.meta.p, static_cast<const double *>(c.val), X, ldx, Y, ldy, k, 0, c.nRow, 0,
+    kern<<<grid, TH, smem, s>>>(c.ptr, c.idx, c.meta.p, static_cast<const VT *>(c.val), X, ldx, Y, ldy, k, 0, c.nRow, 0,
                                 nChunks, capI, capV, S);
     B2_KERNEL_CHECK();
     return B200SPMV_OK;
 }
 
-template <int MAXL, int TH, bool DICT>
-static int cs_multi_k(const ChunkStream &c, int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s)
+template <typename VT, typename XT, typename AT, int MAXL, int TH, bool DICT>
+static int cs_multi_k(const ChunkStream &c, int k, const XT *X, long long ldx, XT *Y, long long ldy, cudaStream_t s)
 {
-    const bool w2 = (ldx & 1) == 0 && (reinterpret_cast<uintptr_t>(X) & 15) == 0;
 #define CS_MK(KP)                                                                                              \
-    return w2 ? cs_multi_launch<MAXL, TH, DICT, KP, true>(c, k, X, ldx, Y, ldy, s)                             \
-              : cs_multi_launch<MAXL, TH, DICT, KP, false>(c, k, X, ldx, Y, ldy, s)
-    if (k == 1) return cs_multi_launch<MAXL, TH, DICT, 1, false>(c, k, X, ldx, Y, ldy, s);
+    return ld_xrow_vec(X, ldx, KP) ? cs_multi_launch<VT, XT, AT, MAXL, TH, DICT, KP, true>(c, k, X, ldx, Y, ldy, s) \
+                                   : cs_multi_launch<VT, XT, AT, MAXL, TH, DICT, KP, false>(c, k, X, ldx, Y, ldy, s)
+    if (k == 1) return cs_multi_launch<VT, XT, AT, MAXL, TH, DICT, 1, false>(c, k, X, ldx, Y, ldy, s);
     if (k == 2) CS_MK(2);
     if (k <= 4) CS_MK(4);
     CS_MK(8);
 #undef CS_MK
 }
 
-template <int MAXL, int TH>
-static int cs_multi_feed(const ChunkStream &c, int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s)
+template <typename VT, typename XT, typename AT>
+static int cs_multi_dispatch(const ChunkStream &c, int k, const XT *X, long long ldx, XT *Y, long long ldy, cudaStream_t s)
 {
-    if (c.feed == CS_FEED_DICT) return cs_multi_k<MAXL, TH, true>(c, k, X, ldx, Y, ldy, s);
-    return cs_multi_k<MAXL, TH, false>(c, k, X, ldx, Y, ldy, s);
+#define CS_MF(MAXL, TH)                                                                                         \
+    return c.feed == CS_FEED_DICT ? cs_multi_k<VT, XT, AT, MAXL, TH, true>(c, k, X, ldx, Y, ldy, s)              \
+                                  : cs_multi_k<VT, XT, AT, MAXL, TH, false>(c, k, X, ldx, Y, ldy, s)
+    if (c.th == 512) {
+        if (c.maxLen <= 8) CS_MF(8, 512);
+        CS_MF(16, 512);
+    }
+    if (c.maxLen <= 8) CS_MF(8, 256);
+    CS_MF(16, 256);
+#undef CS_MF
 }
 
 int ChunkStream::run_multi(int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s) const
 {
     if (f32) { set_error("multiply_multi: the row-chunk stream holds fp32 values"); return B200SPMV_ERR_UNSUPPORTED; }
     if (nRow == 0) return B200SPMV_OK;
-    if (th == 512) return maxLen <= 8 ? cs_multi_feed<8, 512>(*this, k, X, ldx, Y, ldy, s) : cs_multi_feed<16, 512>(*this, k, X, ldx, Y, ldy, s);
-    return maxLen <= 8 ? cs_multi_feed<8, 256>(*this, k, X, ldx, Y, ldy, s) : cs_multi_feed<16, 256>(*this, k, X, ldx, Y, ldy, s);
+    return cs_multi_dispatch<double, double, double>(*this, k, X, ldx, Y, ldy, s);
+}
+
+int ChunkStream::run_multi_f32(int k, const float *X, long long ldx, float *Y, long long ldy, bool acc64, cudaStream_t s) const
+{
+    if (!f32) { set_error("row-chunk stream: fp32 vectors need fp32 value storage"); return B200SPMV_ERR_STATE; }
+    if (nRow == 0) return B200SPMV_OK;
+    if (acc64) return cs_multi_dispatch<float, float, double>(*this, k, X, ldx, Y, ldy, s);
+    return cs_multi_dispatch<float, float, float>(*this, k, X, ldx, Y, ldy, s);
 }
 
 }  // namespace b2

@@ -49,6 +49,8 @@ struct ChunkStream {
     // Y[:, 0..k) := A X[:, 0..k) (k <= 8, row-major with leading dimensions ldx, ldy; fp64 values): the same chunks, one
     // thread per row summing every vector in the order of run(), so each column of Y has the bits of run() on that column
     int run_multi(int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s) const;
+    // the same with fp32 values and vectors, sums in fp32 or (acc64) fp64: each column has the bits of run_f32
+    int run_multi_f32(int k, const float *X, long long ldx, float *Y, long long ldy, bool acc64, cudaStream_t s) const;
 };
 
 }  // namespace b2

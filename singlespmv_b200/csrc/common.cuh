@@ -100,6 +100,12 @@ struct Format {
         set_error("multiply_multi: this format has no multi-vector multiply (CRS has)");
         return B200SPMV_ERR_UNSUPPORTED;
     }
+    // the same with fp32 vectors (b200spmv_multiply_multi_f32, options.precision = 1 / 2)
+    virtual int multiply_multi_f32(int, const float *, long long, float *, long long, cudaStream_t)
+    {
+        set_error("multiply_multi_f32: this format has no multi-vector multiply (CRS has)");
+        return B200SPMV_ERR_UNSUPPORTED;
+    }
     virtual int multiply_rows(int, int, const double *, double *, cudaStream_t)
     {
         set_error("multiply_rows: this format does not support row ranges (CRS, SS, CSS, ELL, DIA do)");
@@ -210,6 +216,13 @@ __device__ __forceinline__ double ld_stream_d1(const double *p, uint64_t pol)
                  : "=d"(r) : "l"(p), "l"(pol));
     return r;
 }
+__device__ __forceinline__ float4 ld_stream_f4(const float *p, uint64_t pol)
+{
+    float4 r;
+    asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.f32 {%0,%1,%2,%3}, [%4], %5;"
+                 : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p), "l"(pol));
+    return r;
+}
 // x gathers: cached in L1 (stencil reuse) and kept in L2 with evict-last priority.
 __device__ __forceinline__ double ld_x(const double *p, uint64_t pol)
 {
@@ -299,6 +312,55 @@ __device__ __forceinline__ void ld_xrow(double (&xv)[KP], const double *p, int n
         }
     }
 }
+// fp32 X: with VEC (ldx a multiple of W = min(KP, 4), X aligned to W floats, j0 a multiple of W) groups of W columns come
+// in one 8- or 16-byte load; one row of X holds up to 8 columns in a single 32-byte sector.
+__device__ __forceinline__ float ld_xm(const float *p, uint64_t pol)
+{
+    float r;
+    asm("ld.global.nc.L2::cache_hint.f32 %0, [%1], %2;" : "=f"(r) : "l"(p), "l"(pol));
+    return r;
+}
+__device__ __forceinline__ float2 ld_xm2(const float *p, uint64_t pol)
+{
+    float2 r;
+    asm("ld.global.nc.L2::cache_hint.v2.f32 {%0,%1}, [%2], %3;" : "=f"(r.x), "=f"(r.y) : "l"(p), "l"(pol));
+    return r;
+}
+__device__ __forceinline__ float4 ld_xm4(const float *p, uint64_t pol)
+{
+    float4 r;
+    asm("ld.global.nc.L2::cache_hint.v4.f32 {%0,%1,%2,%3}, [%4], %5;"
+        : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p), "l"(pol));
+    return r;
+}
+template <int KP, bool VEC>
+__device__ __forceinline__ void ld_xrow(float (&xv)[KP], const float *p, int n, uint64_t pol)
+{
+    constexpr int W = VEC ? (KP < 4 ? KP : 4) : 1;
+#pragma unroll
+    for (int v = 0; v < KP; v += W) {
+        if (W == 4 && v + W - 1 < n) {
+            const float4 t = ld_xm4(p + v, pol);
+            xv[v] = t.x; xv[v + 1] = t.y; xv[v + 2] = t.z; xv[v + 3] = t.w;
+        } else if (W == 2 && v + W - 1 < n) {
+            const float2 t = ld_xm2(p + v, pol);
+            xv[v] = t.x; xv[v + 1] = t.y;
+        } else {
+#pragma unroll
+            for (int i = 0; i < W; i++) xv[v + i] = v + i < n ? ld_xm(p + v + i, pol) : 0.0f;
+        }
+    }
+}
+#endif
+// The vector gathers ld_xrow may use for k columns of X (KP = k rounded up): pairs of fp64 columns, W = min(KP, 4) fp32
+// columns; ldx and X must be aligned to that width
+template <typename XT>
+static inline bool ld_xrow_vec(const XT *X, long long ldx, int KP)
+{
+    const int w = sizeof(XT) == 8 ? 2 : (KP < 4 ? KP : 4);
+    return ldx % w == 0 && reinterpret_cast<uintptr_t>(X) % (w * sizeof(XT)) == 0;
+}
+#ifdef __CUDACC__
 
 __device__ __forceinline__ double warp_sum(double v)
 {

@@ -73,7 +73,7 @@ struct CrsFormat : Format {
         // entry stream, crs_path = 1 the tile-stream.
         use_es = false;
         if (!short_rows && !f32 && !prec && (path_opt == 4 || (path_opt == 0 && gathers_need_l2(band)))) {
-            B2_TRY(es.build(ptr.p, idx.p, val.p, nRow, nnz, gathers_need_l2(band), s));
+            B2_TRY(es.build(ptr.p, idx.p, val.p, false, nRow, nnz, gathers_need_l2(band), s));
             use_es = es.ok;
         }
         B2_CUDA(cudaStreamSynchronize(s));
@@ -111,9 +111,27 @@ struct CrsFormat : Format {
                 return B200SPMV_ERR_STATE;
             }
             B2_TRY(ensure_band(s));
-            B2_TRY(es.build(ptr.p, idx.p, val.p, nRow, nnz, gathers_need_l2(band), s));
+            B2_TRY(es.build(ptr.p, idx.p, val.p, false, nRow, nnz, gathers_need_l2(band), s));
         }
         return es.run_multi(k, X, ldx, Y, ldy, s);
+    }
+    // The fp32-vector form (precision 1 / 2): row-chunk stream handles run its K-vector form, every other handle (the
+    // single multiply runs the tile-stream there) the entry stream on val32, whose metadata the first call builds.
+    int multiply_multi_f32(int k, const float *X, long long ldx, float *Y, long long ldy, cudaStream_t s) override
+    {
+        if (!prec) { set_error("multiply_multi_f32: the handle was created with precision = 0 (fp64 vectors), use b200spmv_multiply_multi"); return B200SPMV_ERR_STATE; }
+        if (short_rows) return cs.run_multi_f32(k, X, ldx, Y, ldy, prec == 2, s);
+        if (nnz == 0) return zero_rows_multi(nRow, k, Y, ldy, s);
+        if (!es.ok) {
+            cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+            if (cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone) {
+                set_error("multiply_multi_f32: first call on this handle inside a stream capture; call it once outside the capture first");
+                return B200SPMV_ERR_STATE;
+            }
+            B2_TRY(ensure_band(s));
+            B2_TRY(es.build(ptr.p, idx.p, val32.p, true, nRow, nnz, gathers_need_l2(band), s));
+        }
+        return es.run_multi_f32(k, X, ldx, Y, ldy, prec == 2, s);
     }
     int ensure_band(cudaStream_t s)
     {
@@ -145,6 +163,15 @@ struct CrsFormat : Format {
             if (f32) *out = 0;
             else if (short_rows) *out = 1;
             else if (use_es) *out = es.tma ? 2 : 3;
+            else {
+                if (ensure_band(nullptr) != B200SPMV_OK) return false;
+                *out = gathers_need_l2(band) ? 3 : 2;
+            }
+            return true;
+        }
+        if (n == "multi_kernel_f32") {   // b200spmv_multiply_multi_f32: the same numbering, 0 on precision-0 handles and
+            if (!prec || nnz == 0) *out = 0;                     // without entries (Y is only zero-filled)
+            else if (short_rows) *out = 1;
             else {
                 if (ensure_band(nullptr) != B200SPMV_OK) return false;
                 *out = gathers_need_l2(band) ? 3 : 2;

@@ -267,44 +267,69 @@ __global__ void entry_stream_fixup_kernel(const unsigned *__restrict__ bits, con
     if (r >= rowLo && r < rowHi) y[r] = __dadd_rn(y[r], sum);
 }
 
+// the values of a lane's 4 entries of a full group: from the stage (TMA) or by streaming loads
+template <bool TMA>
+__device__ __forceinline__ void es_vals4(double (&a)[4], const double *V, uint64_t pol)
+{
+    double2 v0, v1;
+    if (TMA) {
+        v0 = *reinterpret_cast<const double2 *>(V);
+        v1 = *reinterpret_cast<const double2 *>(V + 2);
+    } else {
+        v0 = ld_stream_d2(V, pol);
+        v1 = ld_stream_d2(V + 2, pol);
+    }
+    a[0] = v0.x; a[1] = v0.y; a[2] = v1.x; a[3] = v1.y;
+}
+template <bool TMA>
+__device__ __forceinline__ void es_vals4(float (&a)[4], const float *V, uint64_t pol)
+{
+    const float4 v = TMA ? *reinterpret_cast<const float4 *>(V) : ld_stream_f4(V, pol);
+    a[0] = v.x; a[1] = v.y; a[2] = v.z; a[3] = v.w;
+}
+
 // ---------------------------------------------------------------- multiply of k <= ES_KMAX vectors (X, Y row-major)
 // The kernel above with every sum carried for KP vectors at once: the entry stream, start bits, ballots and scans are
 // shared, the lane gathers the KP values of a column in one row of X (ld_xrow).  k > KP: the tile is reduced once per
 // group of KP vectors (TMA-fed from the same stage, load-fed from L2).  Carries: carry[t * k + j].
-template <bool TMA, int KP, bool W2>
+// VT = stored value type, XT = type of X and Y, AT = type of products and sums (fp32 vectors: fp32 or fp64).  With fp32 Y
+// (TAIL) the row still open at the end of a tile is not stored: its partial goes to the tile's tail slot carry[(nT + t) * k
+// + j] in AT, and the fix-up writes that row once -- so a precision-2 row is rounded to fp32 once, after every carry.
+template <typename VT, typename XT, typename AT, bool TMA, int KP, bool VEC>
 __global__ void __launch_bounds__(ES_THREADS)
-entry_stream_multi_kernel(const int *__restrict__ idx, const double *__restrict__ val, const unsigned *__restrict__ bits,
-                          const int *__restrict__ grpRun, const int *__restrict__ nzrow, const double *__restrict__ X,
-                          long long ldx, double *__restrict__ Y, long long ldy, int kv, double *__restrict__ carry, int nnz,
+entry_stream_multi_kernel(const int *__restrict__ idx, const VT *__restrict__ val, const unsigned *__restrict__ bits,
+                          const int *__restrict__ grpRun, const int *__restrict__ nzrow, const XT *__restrict__ X,
+                          long long ldx, XT *__restrict__ Y, long long ldy, int kv, AT *__restrict__ carry, int nnz,
                           int tileLo, int tileHi, int rowLo, int rowHi)
 {
+    constexpr bool TAIL = sizeof(XT) == 4;
     constexpr int E = ES_E;
     constexpr int CHUNK = E / ES_WARPS;
     constexpr int GROUPS = CHUNK / 128;
     extern __shared__ __align__(128) unsigned char es_smem[];
     __shared__ __align__(8) uint64_t full[2];
-    __shared__ double rPiece[ES_WARPS][ES_KMAX], rTail[ES_WARPS][ES_KMAX];
+    __shared__ AT rPiece[ES_WARPS][ES_KMAX], rTail[ES_WARPS][ES_KMAX];
     __shared__ int rRun[ES_WARPS];
     int *scol = reinterpret_cast<int *>(es_smem);
-    double *sval = reinterpret_cast<double *>(es_smem + 2 * E * sizeof(int));
+    VT *sval = reinterpret_cast<VT *>(es_smem + 2 * E * sizeof(int));
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const uint64_t pol_stream = policy_evict_first(), pol_x = policy_evict_last();
     const unsigned lt = (1u << lane) - 1u;
 
     auto row_of = [&](int run) { return nzrow ? nzrow[run] : run; };
-    auto store = [&](int run, int j0, const double (&a)[KP]) {
+    auto store = [&](int run, int j0, const AT (&a)[KP]) {
         const int r = row_of(run);
         if (r >= rowLo && r < rowHi) {
-            double *yr = Y + (long long)r * ldy + j0;
+            XT *yr = Y + (long long)r * ldy + j0;
 #pragma unroll
             for (int v = 0; v < KP; v++)
-                if (j0 + v < kv) yr[v] = a[v];
+                if (j0 + v < kv) yr[v] = (XT)a[v];
         }
     };
     auto issue = [&](int s, int t) {
         const long long t0 = (long long)t * E;
         const int n = (int)min((long long)E, (long long)nnz - t0);
-        const uint32_t b4 = (uint32_t)((n * 4 + 15) & ~15), b8 = (uint32_t)(n * 8 + 15) & ~15u;
+        const uint32_t b4 = (uint32_t)((n * 4 + 15) & ~15), b8 = (uint32_t)(n * (int)sizeof(VT) + 15) & ~15u;
         mbar_expect_tx(&full[s], b4 + b8);
         tma_load_1d(scol + s * E, idx + t0, b4, &full[s], pol_stream);
         tma_load_1d(sval + s * E, val + t0, b8, &full[s], pol_stream);
@@ -328,12 +353,12 @@ entry_stream_multi_kernel(const int *__restrict__ idx, const double *__restrict_
         const int nw = min(ES_WARPS, (n + CHUNK - 1) / CHUNK);
         if (TMA) mbar_wait(&full[s], (uint32_t)(k >> 1) & 1u);
         const int *Cc = TMA ? scol + s * E : idx + t0;
-        const double *V = TMA ? sval + s * E : val + t0;
+        const VT *V = TMA ? sval + s * E : val + t0;
         for (int j0 = 0; j0 < kv && nGroups > 0; j0 += KP) {
             bool started = false;
-            double cin[KP], piece[KP];
+            AT cin[KP], piece[KP];
 #pragma unroll
-            for (int v = 0; v < KP; v++) cin[v] = piece[v] = 0.0;
+            for (int v = 0; v < KP; v++) cin[v] = piece[v] = (AT)0;
             int lastRun = -1;
 #pragma unroll
             for (int g = 0; g < GROUPS; g++) {
@@ -341,49 +366,44 @@ entry_stream_multi_kernel(const int *__restrict__ idx, const double *__restrict_
                 const int e = c0 + g * 128 + 4 * lane;
                 const long long ge = t0 + e;
                 int4 c;
-                double2 v0, v1;
+                VT a[4];
                 if (c0 + g * 128 + 128 <= n) {
-                    if (TMA) {
-                        c = *reinterpret_cast<const int4 *>(Cc + e);
-                        v0 = *reinterpret_cast<const double2 *>(V + e);
-                        v1 = *reinterpret_cast<const double2 *>(V + e + 2);
-                    } else {
-                        c = ld_stream_i4(Cc + e, pol_stream);
-                        v0 = ld_stream_d2(V + e, pol_stream);
-                        v1 = ld_stream_d2(V + e + 2, pol_stream);
-                    }
+                    if (TMA) c = *reinterpret_cast<const int4 *>(Cc + e);
+                    else c = ld_stream_i4(Cc + e, pol_stream);
+                    es_vals4<TMA>(a, V + e, pol_stream);
                 } else {
                     c.x = e < n ? Cc[e] : 0; c.y = e + 1 < n ? Cc[e + 1] : 0; c.z = e + 2 < n ? Cc[e + 2] : 0; c.w = e + 3 < n ? Cc[e + 3] : 0;
-                    v0.x = e < n ? V[e] : 0.0; v0.y = e + 1 < n ? V[e + 1] : 0.0; v1.x = e + 2 < n ? V[e + 2] : 0.0; v1.y = e + 3 < n ? V[e + 3] : 0.0;
+                    a[0] = e < n ? V[e] : (VT)0; a[1] = e + 1 < n ? V[e + 1] : (VT)0; a[2] = e + 2 < n ? V[e + 2] : (VT)0; a[3] = e + 3 < n ? V[e + 3] : (VT)0;
                 }
                 const unsigned word = __ldg(bits + (ge >> 5));
                 const unsigned b = (word >> (unsigned)(ge & 31)) & 0xFu;
                 const int base = __ldg(grpRun + (ge >> 7));
-                double p0[KP], p1[KP], p2[KP], p3[KP];
-                ld_xrow<KP, W2>(p0, X + (long long)c.x * ldx + j0, kv - j0, pol_x);
-                ld_xrow<KP, W2>(p1, X + (long long)c.y * ldx + j0, kv - j0, pol_x);
-                ld_xrow<KP, W2>(p2, X + (long long)c.z * ldx + j0, kv - j0, pol_x);
-                ld_xrow<KP, W2>(p3, X + (long long)c.w * ldx + j0, kv - j0, pol_x);
+                XT x0[KP], x1[KP], x2[KP], x3[KP];
+                ld_xrow<KP, VEC>(x0, X + (long long)c.x * ldx + j0, kv - j0, pol_x);
+                ld_xrow<KP, VEC>(x1, X + (long long)c.y * ldx + j0, kv - j0, pol_x);
+                ld_xrow<KP, VEC>(x2, X + (long long)c.z * ldx + j0, kv - j0, pol_x);
+                ld_xrow<KP, VEC>(x3, X + (long long)c.w * ldx + j0, kv - j0, pol_x);
+                AT p0[KP], p1[KP], p2[KP], p3[KP];
 #pragma unroll
                 for (int v = 0; v < KP; v++) {
-                    p0[v] = __dmul_rn(v0.x, p0[v]); p1[v] = __dmul_rn(v0.y, p1[v]);
-                    p2[v] = __dmul_rn(v1.x, p2[v]); p3[v] = __dmul_rn(v1.y, p3[v]);
+                    p0[v] = Arith<AT>::mul((AT)a[0], (AT)x0[v]); p1[v] = Arith<AT>::mul((AT)a[1], (AT)x1[v]);
+                    p2[v] = Arith<AT>::mul((AT)a[2], (AT)x2[v]); p3[v] = Arith<AT>::mul((AT)a[3], (AT)x3[v]);
                 }
                 const bool b0 = b & 1u, b1 = b & 2u, b2 = b & 4u, b3 = b & 8u;
                 const bool has = b != 0u;
                 const int nStarts = __popc(b);
                 const unsigned m = __ballot_sync(0xffffffffu, has);
                 int runOpen = base - 1 + __popc(m & lt);
-                double head[KP], acc[KP];
+                AT head[KP], acc[KP];
                 if (__any_sync(0xffffffffu, nStarts > 1)) {
                     const unsigned m0 = __ballot_sync(0xffffffffu, b0), m1 = __ballot_sync(0xffffffffu, b1),
                                    m2 = __ballot_sync(0xffffffffu, b2), m3 = __ballot_sync(0xffffffffu, b3);
                     runOpen = base - 1 + __popc(m0 & lt) + __popc(m1 & lt) + __popc(m2 & lt) + __popc(m3 & lt);
 #pragma unroll
-                    for (int v = 0; v < KP; v++) head[v] = acc[v] = 0.0;
+                    for (int v = 0; v < KP; v++) head[v] = acc[v] = (AT)0;
                     bool seen = false;
                     int run = runOpen;
-                    auto step = [&](bool st, const double (&p)[KP]) {
+                    auto step = [&](bool st, const AT (&p)[KP]) {
                         if (st) {
                             if (!seen) {
 #pragma unroll
@@ -397,7 +417,7 @@ entry_stream_multi_kernel(const int *__restrict__ idx, const double *__restrict_
                             for (int v = 0; v < KP; v++) acc[v] = p[v];
                         } else {
 #pragma unroll
-                            for (int v = 0; v < KP; v++) acc[v] = __dadd_rn(acc[v], p[v]);
+                            for (int v = 0; v < KP; v++) acc[v] = Arith<AT>::add(acc[v], p[v]);
                         }
                     };
                     step(b0, p0); step(b1, p1); step(b2, p2); step(b3, p3);
@@ -405,8 +425,8 @@ entry_stream_multi_kernel(const int *__restrict__ idx, const double *__restrict_
                     const bool f0 = b0, f1 = f0 | b1, f2 = f1 | b2;
 #pragma unroll
                     for (int v = 0; v < KP; v++) {
-                        head[v] = __dadd_rn(__dadd_rn((has && !f0) ? p0[v] : 0.0, (has && !f1) ? p1[v] : 0.0), (has && !f2) ? p2[v] : 0.0);
-                        acc[v] = __dadd_rn(__dadd_rn(__dadd_rn((!has || f0) ? p0[v] : 0.0, (!has || f1) ? p1[v] : 0.0), (!has || f2) ? p2[v] : 0.0), p3[v]);
+                        head[v] = Arith<AT>::add(Arith<AT>::add((has && !f0) ? p0[v] : (AT)0, (has && !f1) ? p1[v] : (AT)0), (has && !f2) ? p2[v] : (AT)0);
+                        acc[v] = Arith<AT>::add(Arith<AT>::add(Arith<AT>::add((!has || f0) ? p0[v] : (AT)0, (!has || f1) ? p1[v] : (AT)0), (!has || f2) ? p2[v] : (AT)0), p3[v]);
                     }
                 }
                 const unsigned below = m & (0xffffffffu >> (31 - lane));
@@ -421,7 +441,7 @@ entry_stream_multi_kernel(const int *__restrict__ idx, const double *__restrict_
                         if (cov != 0xffffffffu) { cov |= cov << 8; steps = cov != 0xffffffffu ? 5 : 4; }
                     }
                 }
-                double sc[KP];                                  // the segmented scan, per vector
+                AT sc[KP];                                      // the segmented scan, per vector
 #pragma unroll
                 for (int v = 0; v < KP; v++) sc[v] = acc[v];
 #pragma unroll
@@ -430,19 +450,19 @@ entry_stream_multi_kernel(const int *__restrict__ idx, const double *__restrict_
                         const int d = 1 << i;
 #pragma unroll
                         for (int v = 0; v < KP; v++) {
-                            const double u = __shfl_up_sync(0xffffffffu, sc[v], d);
-                            if (lane - d >= seg) sc[v] = __dadd_rn(sc[v], u);
+                            const AT u = __shfl_up_sync(0xffffffffu, sc[v], d);
+                            if (lane - d >= seg) sc[v] = Arith<AT>::add(sc[v], u);
                         }
                     }
                 }
                 const bool firstInChunk = !started && !(m & lt);
-                double tot[KP];
+                AT tot[KP];
 #pragma unroll
                 for (int v = 0; v < KP; v++) {
-                    if (!below) sc[v] = __dadd_rn(sc[v], cin[v]);
-                    double excl = __shfl_up_sync(0xffffffffu, sc[v], 1);
+                    if (!below) sc[v] = Arith<AT>::add(sc[v], cin[v]);
+                    AT excl = __shfl_up_sync(0xffffffffu, sc[v], 1);
                     if (lane == 0) excl = cin[v];
-                    tot[v] = __dadd_rn(excl, head[v]);
+                    tot[v] = Arith<AT>::add(excl, head[v]);
                     if (has && firstInChunk) piece[v] = tot[v];
                 }
                 if (has && !firstInChunk) store(runOpen, j0, tot);
@@ -467,24 +487,26 @@ entry_stream_multi_kernel(const int *__restrict__ idx, const double *__restrict_
         __syncthreads();                                    // every warp is done with stage s, the chunk records are in place
         if (tid >= 32 && tid < 32 + kv) {                   // one thread per vector stitches the chunks of the tile
             const int j = tid - 32;
-            double tilePiece = 0.0, a2 = 0.0;
+            AT tilePiece = (AT)0, a2 = (AT)0;
             int accRun = -1;
-            auto put = [&](int run, double v) {
+            auto put = [&](int run, AT v) {
                 const int r = row_of(run);
-                if (r >= rowLo && r < rowHi) Y[(long long)r * ldy + j] = v;
+                if (r >= rowLo && r < rowHi) Y[(long long)r * ldy + j] = (XT)v;
             };
             for (int w = 0; w < nw; w++) {
-                const double oPiece = rPiece[w][j], oTail = rTail[w][j];
+                const AT oPiece = rPiece[w][j], oTail = rTail[w][j];
                 const int oRun = rRun[w];
-                if (accRun >= 0) a2 = __dadd_rn(a2, oPiece);
-                else tilePiece = __dadd_rn(tilePiece, oPiece);
+                if (accRun >= 0) a2 = Arith<AT>::add(a2, oPiece);
+                else tilePiece = Arith<AT>::add(tilePiece, oPiece);
                 if (oRun >= 0) {
                     if (accRun >= 0) put(accRun, a2);
                     accRun = oRun;
                     a2 = oTail;
                 }
             }
-            if (accRun >= 0) put(accRun, a2);
+            if (TAIL && accRun >= 0 && t + 1 < tileHi && !((bits[((long long)(t + 1) * E) >> 5] >> (unsigned)(((long long)(t + 1) * E) & 31)) & 1u))
+                carry[((long long)tileHi + t) * kv + j] = a2;       // the row goes on in tile t + 1: the fix-up stores it
+            else if (accRun >= 0) put(accRun, a2);
             carry[(long long)t * kv + j] = tilePiece;
         }
         __syncthreads();                                    // the records are read before the next tile's warps rewrite them
@@ -492,11 +514,14 @@ entry_stream_multi_kernel(const int *__restrict__ idx, const double *__restrict_
     }
 }
 
-// one thread per (tile, vector): entry_stream_fixup_kernel on column j of Y
+// one thread per (tile, vector): entry_stream_fixup_kernel on column j of Y.  TAIL (fp32 Y): the row's partial from the
+// tile in front comes from that tile's tail slot, and Y is written once.
+template <typename XT, typename AT>
 __global__ void entry_stream_multi_fixup_kernel(const unsigned *__restrict__ bits, const int *__restrict__ grpRun,
-                                                const int *__restrict__ nzrow, double *__restrict__ Y, long long ldy, int kv,
-                                                const double *__restrict__ carry, int E, int tileLo, int tileHi)
+                                                const int *__restrict__ nzrow, XT *__restrict__ Y, long long ldy, int kv,
+                                                const AT *__restrict__ carry, int E, int tileLo, int tileHi)
 {
+    constexpr bool TAIL = sizeof(XT) == 4;
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const int t = tileLo + 1 + (int)(i / kv), j = (int)(i % kv);
     if (t >= tileHi) return;
@@ -505,33 +530,38 @@ __global__ void entry_stream_multi_fixup_kernel(const unsigned *__restrict__ bit
     if (first_bit(t)) return;
     const int run = run_at(t);
     if (!first_bit(t - 1) && run_at(t - 1) == run) return;
-    double sum = 0.0;
-    for (int u = t; u < tileHi && !first_bit(u) && run_at(u) == run; u++) sum = __dadd_rn(sum, carry[(long long)u * kv + j]);
-    double *yr = Y + (long long)(nzrow ? nzrow[run] : run) * ldy + j;
-    *yr = __dadd_rn(*yr, sum);
+    AT sum = (AT)0;
+    for (int u = t; u < tileHi && !first_bit(u) && run_at(u) == run; u++) sum = Arith<AT>::add(sum, carry[(long long)u * kv + j]);
+    XT *yr = Y + (long long)(nzrow ? nzrow[run] : run) * ldy + j;
+    if (TAIL) *yr = (XT)Arith<AT>::add(carry[((long long)tileHi + t - 1) * kv + j], sum);
+    else *yr = Arith<AT>::add(*yr, sum);
 }
 
 // Y[r, j] = 0 for the listed rows (all rows [0, n) when rows == NULL) and j < k
-__global__ void es_zero_rows_multi_kernel(const int *__restrict__ rows, int n, int kv, double *__restrict__ Y, long long ldy)
+template <typename XT>
+__global__ void es_zero_rows_multi_kernel(const int *__restrict__ rows, int n, int kv, XT *__restrict__ Y, long long ldy)
 {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (long long)n * kv) return;
     const int q = (int)(i / kv);
-    Y[(long long)(rows ? rows[q] : q) * ldy + (int)(i % kv)] = 0.0;
+    Y[(long long)(rows ? rows[q] : q) * ldy + (int)(i % kv)] = (XT)0;
 }
 
-int zero_rows_multi(int nRow, int k, double *Y, long long ldy, cudaStream_t s)
+template <typename XT>
+static int zero_rows_multi_t(int nRow, int k, XT *Y, long long ldy, cudaStream_t s)
 {
     if (nRow <= 0) return B200SPMV_OK;
     es_zero_rows_multi_kernel<<<ceil_div((long long)nRow * k, 256), 256, 0, s>>>(nullptr, nRow, k, Y, ldy);
     B2_KERNEL_CHECK();
     return B200SPMV_OK;
 }
+int zero_rows_multi(int nRow, int k, double *Y, long long ldy, cudaStream_t s) { return zero_rows_multi_t(nRow, k, Y, ldy, s); }
+int zero_rows_multi(int nRow, int k, float *Y, long long ldy, cudaStream_t s) { return zero_rows_multi_t(nRow, k, Y, ldy, s); }
 
-int EntryStream::build(const int *ptr_d, const int *idx_d, const double *val_d, int nRow_, int nnz_, bool gather_bound,
-                       cudaStream_t s)
+int EntryStream::build(const int *ptr_d, const int *idx_d, const void *val_d, bool val_is_f32, int nRow_, int nnz_,
+                       bool gather_bound, cudaStream_t s)
 {
-    ptr = ptr_d; idx = idx_d; val = val_d; nRow = nRow_; nnz = nnz_;
+    ptr = ptr_d; idx = idx_d; val = val_d; f32 = val_is_f32; nRow = nRow_; nnz = nnz_;
     ok = false;
     range_cache.clear();
     carryK.release();
@@ -541,7 +571,8 @@ int EntryStream::build(const int *ptr_d, const int *idx_d, const double *val_d, 
     const int nGroups = ceil_div((long long)nTiles * ES_E, 128);
     B2_TRY(bits.alloc((size_t)nGroups * 4 + 4));
     B2_TRY(grpRun.alloc((size_t)nGroups + 1));
-    B2_TRY(carry.alloc((size_t)nTiles));
+    if (f32) carry.release();                              // run_rows (fp64 only) owns these; run_multi* use carryK
+    else B2_TRY(carry.alloc((size_t)nTiles));
     B2_CUDA(cudaMemsetAsync(bits.p, 0, bits.bytes(), s));
     DevBuf<int> cnt;
     B2_TRY(cnt.alloc(1));
@@ -603,7 +634,7 @@ static int es_launch(EntryStream &T, const double *x, double *y, int tileLo, int
     const int nT = tileHi - tileLo;
     const int perSm = std::min(it->second, 6);
     const int grid = TMA ? std::min(nT, sms * perSm) : nT;
-    kern<<<grid, ES_THREADS, smem, s>>>(T.idx, T.val, T.bits.p, T.grpRun.p, T.nEmpty ? T.nzrow.p : nullptr, x, y, T.carry.p, T.nnz, tileLo,
+    kern<<<grid, ES_THREADS, smem, s>>>(T.idx, static_cast<const double *>(T.val), T.bits.p, T.grpRun.p, T.nEmpty ? T.nzrow.p : nullptr, x, y, T.carry.p, T.nnz, tileLo,
                                         tileHi, rb, re);
     B2_KERNEL_CHECK();
     if (nT > 1) {
@@ -642,11 +673,11 @@ int EntryStream::run_rows(const double *x, double *y, int rb, int re, cudaStream
     return es_launch<false>(*this, x, y, lo, hi, rb, re, s);
 }
 
-template <bool TMA, int KP, bool W2>
-static int es_multi_launch(EntryStream &T, int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s)
+template <typename VT, typename XT, typename AT, bool TMA, int KP, bool VEC>
+static int es_multi_launch(EntryStream &T, int k, const XT *X, long long ldx, XT *Y, long long ldy, cudaStream_t s)
 {
-    constexpr size_t smem = TMA ? 24 * (size_t)ES_E : 0;
-    auto kern = entry_stream_multi_kernel<TMA, KP, W2>;
+    constexpr size_t smem = TMA ? (4 + sizeof(VT)) * 2 * (size_t)ES_E : 0;
+    auto kern = entry_stream_multi_kernel<VT, XT, AT, TMA, KP, VEC>;
     static std::map<int, int> per_sm;
     static int sms = 0;
     int dev = 0;
@@ -662,44 +693,72 @@ static int es_multi_launch(EntryStream &T, int k, const double *X, long long ldx
     }
     const int nT = T.nTiles;
     const int grid = TMA ? std::min(nT, sms * std::min(it->second, 6)) : nT;
-    kern<<<grid, ES_THREADS, smem, s>>>(T.idx, T.val, T.bits.p, T.grpRun.p, T.nEmpty ? T.nzrow.p : nullptr, X, ldx, Y, ldy, k,
-                                        T.carryK.p, T.nnz, 0, nT, 0, T.nRow);
+    AT *carry = reinterpret_cast<AT *>(T.carryK.p);
+    kern<<<grid, ES_THREADS, smem, s>>>(T.idx, static_cast<const VT *>(T.val), T.bits.p, T.grpRun.p, T.nEmpty ? T.nzrow.p : nullptr,
+                                        X, ldx, Y, ldy, k, carry, T.nnz, 0, nT, 0, T.nRow);
     B2_KERNEL_CHECK();
     if (nT > 1) {
         entry_stream_multi_fixup_kernel<<<ceil_div((long long)(nT - 1) * k, 256), 256, 0, s>>>(
-            T.bits.p, T.grpRun.p, T.nEmpty ? T.nzrow.p : nullptr, Y, ldy, k, T.carryK.p, ES_E, 0, nT);
+            T.bits.p, T.grpRun.p, T.nEmpty ? T.nzrow.p : nullptr, Y, ldy, k, carry, ES_E, 0, nT);
         B2_KERNEL_CHECK();
     }
     return B200SPMV_OK;
 }
 
-template <bool TMA>
-static int es_multi_k(EntryStream &T, int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s)
+template <typename VT, typename XT, typename AT, bool TMA>
+static int es_multi_k(EntryStream &T, int k, const XT *X, long long ldx, XT *Y, long long ldy, cudaStream_t s)
 {
-    const bool w2 = (ldx & 1) == 0 && (reinterpret_cast<uintptr_t>(X) & 15) == 0;
-    if (k == 1) return es_multi_launch<TMA, 1, false>(T, k, X, ldx, Y, ldy, s);
-    if (k == 2) return w2 ? es_multi_launch<TMA, 2, true>(T, k, X, ldx, Y, ldy, s) : es_multi_launch<TMA, 2, false>(T, k, X, ldx, Y, ldy, s);
-    return w2 ? es_multi_launch<TMA, 4, true>(T, k, X, ldx, Y, ldy, s) : es_multi_launch<TMA, 4, false>(T, k, X, ldx, Y, ldy, s);
+    if (k == 1) return es_multi_launch<VT, XT, AT, TMA, 1, false>(T, k, X, ldx, Y, ldy, s);
+    if (k == 2) {
+        return ld_xrow_vec(X, ldx, 2) ? es_multi_launch<VT, XT, AT, TMA, 2, true>(T, k, X, ldx, Y, ldy, s)
+                                      : es_multi_launch<VT, XT, AT, TMA, 2, false>(T, k, X, ldx, Y, ldy, s);
+    }
+    return ld_xrow_vec(X, ldx, 4) ? es_multi_launch<VT, XT, AT, TMA, 4, true>(T, k, X, ldx, Y, ldy, s)
+                                  : es_multi_launch<VT, XT, AT, TMA, 4, false>(T, k, X, ldx, Y, ldy, s);
+}
+
+// the part shared by both precisions: zero the empty rows, allocate the carries on the first call
+template <typename XT>
+static int es_multi_prologue(EntryStream &T, int k, XT *Y, long long ldy, const char *entry, cudaStream_t s)
+{
+    if (!T.carryK.p) {
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        if (cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone) {
+            set_error("%s: first call on this handle inside a stream capture; call it once outside the capture first", entry);
+            return B200SPMV_ERR_STATE;
+        }
+        // fp32 vectors: the head carries, then the tail slots of entry_stream_multi_kernel (fp64 or fp32, in fp64 room)
+        B2_TRY(T.carryK.alloc((size_t)T.nTiles * ES_KMAX * (T.f32 ? 2 : 1)));
+    }
+    if (T.nEmpty) {
+        es_zero_rows_multi_kernel<<<ceil_div((long long)T.nEmpty * k, 256), 256, 0, s>>>(T.empty.p, T.nEmpty, k, Y, ldy);
+        B2_KERNEL_CHECK();
+    }
+    return B200SPMV_OK;
 }
 
 int EntryStream::run_multi(int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s)
 {
     if (k < 1 || k > ES_KMAX) { set_error("multiply_multi: k=%d outside 1..%d", k, ES_KMAX); return B200SPMV_ERR_INVALID; }
+    if (f32) { set_error("multiply_multi: the entry stream holds fp32 values"); return B200SPMV_ERR_UNSUPPORTED; }
     if (!ok) return zero_rows_multi(nRow, k, Y, ldy, s);      // no entries
-    if (!carryK.p) {
-        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        if (cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone) {
-            set_error("multiply_multi: first call on this handle inside a stream capture; call it once outside the capture first");
-            return B200SPMV_ERR_STATE;
-        }
-        B2_TRY(carryK.alloc((size_t)nTiles * ES_KMAX));
+    B2_TRY(es_multi_prologue(*this, k, Y, ldy, "multiply_multi", s));
+    if (tma) return es_multi_k<double, double, double, true>(*this, k, X, ldx, Y, ldy, s);
+    return es_multi_k<double, double, double, false>(*this, k, X, ldx, Y, ldy, s);
+}
+
+int EntryStream::run_multi_f32(int k, const float *X, long long ldx, float *Y, long long ldy, bool acc64, cudaStream_t s)
+{
+    if (k < 1 || k > ES_KMAX) { set_error("multiply_multi_f32: k=%d outside 1..%d", k, ES_KMAX); return B200SPMV_ERR_INVALID; }
+    if (!f32) { set_error("multiply_multi_f32: the entry stream holds fp64 values"); return B200SPMV_ERR_STATE; }
+    if (!ok) return zero_rows_multi(nRow, k, Y, ldy, s);
+    B2_TRY(es_multi_prologue(*this, k, Y, ldy, "multiply_multi_f32", s));
+    if (acc64) {
+        if (tma) return es_multi_k<float, float, double, true>(*this, k, X, ldx, Y, ldy, s);
+        return es_multi_k<float, float, double, false>(*this, k, X, ldx, Y, ldy, s);
     }
-    if (nEmpty) {
-        es_zero_rows_multi_kernel<<<ceil_div((long long)nEmpty * k, 256), 256, 0, s>>>(empty.p, nEmpty, k, Y, ldy);
-        B2_KERNEL_CHECK();
-    }
-    if (tma) return es_multi_k<true>(*this, k, X, ldx, Y, ldy, s);
-    return es_multi_k<false>(*this, k, X, ldx, Y, ldy, s);
+    if (tma) return es_multi_k<float, float, float, true>(*this, k, X, ldx, Y, ldy, s);
+    return es_multi_k<float, float, float, false>(*this, k, X, ldx, Y, ldy, s);
 }
 
 }  // namespace b2

@@ -26,11 +26,13 @@ constexpr int ES_KMAX = 8;         // vectors of one multi-vector multiply
 
 // Y[r, j] = 0 for r < nRow, j < k (row-major Y): the multi-vector multiply of a matrix without entries
 int zero_rows_multi(int nRow, int k, double *Y, long long ldy, cudaStream_t s);
+int zero_rows_multi(int nRow, int k, float *Y, long long ldy, cudaStream_t s);
 
 struct EntryStream {
     // borrowed
     const int *ptr = nullptr, *idx = nullptr;
-    const double *val = nullptr;
+    const void *val = nullptr;         // fp64, or fp32 when f32 (the multi-vector multiply with fp32 vectors only)
+    bool f32 = false;
     int nRow = 0, nnz = 0;
     // owned
     bool ok = false, tma = false;
@@ -38,16 +40,21 @@ struct EntryStream {
     DevBuf<unsigned> bits;
     DevBuf<int> grpRun, nzrow, empty;
     DevBuf<double> carry;
-    DevBuf<double> carryK;             // nTiles x ES_KMAX carries of run_multi, allocated by its first call
+    DevBuf<double> carryK;             // nTiles x ES_KMAX carries of run_multi (f32: twice that), allocated by its first call
     std::map<std::pair<int, int>, std::pair<int, int>> range_cache;
 
     // gather_bound: the x gathers need L2 residency (primitives.cu gathers_need_l2) -> load-fed, else TMA-fed
-    int build(const int *ptr_d, const int *idx_d, const double *val_d, int nRow_, int nnz_, bool gather_bound, cudaStream_t s);
+    // val_is_f32: fp32 values, for run_multi_f32 only (the metadata does not depend on the value type)
+    int build(const int *ptr_d, const int *idx_d, const void *val_d, bool val_is_f32, int nRow_, int nnz_, bool gather_bound,
+              cudaStream_t s);
     int prepare(int rb, int re);
     int run_rows(const double *x, double *y, int rb, int re, cudaStream_t s);
     // Y[:, 0..k) := A X[:, 0..k) over all rows (k <= ES_KMAX, row-major); each column is summed as run_rows sums it.
     // The first call allocates the carries: refused with B200SPMV_ERR_STATE inside a stream capture.
     int run_multi(int k, const double *X, long long ldx, double *Y, long long ldy, cudaStream_t s);
+    // the same with fp32 values and vectors, products and sums in fp32 or (acc64) fp64.  A row that runs past a tile has its
+    // partial kept in AT until the fix-up adds the later tiles' carries: Y is rounded to fp32 once per row.
+    int run_multi_f32(int k, const float *X, long long ldx, float *Y, long long ldy, bool acc64, cudaStream_t s);
 };
 
 }  // namespace b2

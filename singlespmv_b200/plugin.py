@@ -180,6 +180,11 @@ class SpMatOpt:
         """fp32 vectors (handle created with precision=1 or 2); raw device addresses of float arrays."""
         check(lib.b200spmv_multiply_f32(self.h, C.c_void_p(x_ptr), C.c_void_p(y_ptr), stream))
 
+    def multiply_multi_f32(self, k, X_ptr, ldx, Y_ptr, ldy, stream=None):
+        """Y[:, :k] := A X[:, :k] for k = 1..8 device-resident row-major fp32 vectors (X[c*ldx + j], Y[r*ldy + j]): the
+        matrix is streamed once for all k.  CRS handles created with precision=1 or 2 (b200spmv_multiply_multi_f32)."""
+        check(lib.b200spmv_multiply_multi_f32(self.h, k, C.c_void_p(X_ptr), ldx, C.c_void_p(Y_ptr), ldy, stream))
+
     def multiply_host_f32(self, x, y):
         assert x.dtype == np.float32 and y.dtype == np.float32
         check(lib.b200spmv_multiply_host_f32(self.h, _ptr(x), _ptr(y)))
