@@ -97,7 +97,16 @@ typedef struct {
                             by the lanes' own loads, whichever suits the matrix; 1 = the order-preserving tile kernel (rows <= 64
                             entries bit-identical to the CRS result); 2 / 3 = force the load-fed / the TMA-fed entry stream;
                             other values are rejected */
-    int reserved[5];
+    int transpose;       /* 1 = also build A^T at conversion, for b200spmv_multiply_transpose{,_f32}: A's COO transposed on the
+                            device (a stable, deterministic sort on the column: the host's lexsort of (col, row)), then
+                            converted like A -- the same format and options, row blocks above 2^31-1 entries -- into a
+                            second matrix the handle holds.  Conversion time and device memory grow by about A's; the
+                            transposed COO and its sort scratch are freed before the conversion returns.  A JDS permutation
+                            (b200spmv_jds_set_perm_host) applies to A only: A^T orders ties by ascending row.  If A^T cannot
+                            be built (e.g. B200SPMV_ERR_NOMEM: an ELL of A^T pads to A's longest column), the conversion
+                            fails and the handle stays unconverted.  0 = no A^T (default); other values are rejected.
+                            Not accepted by b200spmv_mg_create */
+    int reserved[4];
 } b200spmv_options;
 
 /* ---- library ---- */
@@ -141,6 +150,18 @@ B200SPMV_API int b200spmv_multiply(b200spmv_matrix *m, const double *x_d, double
  * (before convert, precision 1 / 2, first call inside a capture). */
 B200SPMV_API int b200spmv_multiply_multi(b200spmv_matrix *m, int k, const double *X_d, long long ldx,
                                          double *Y_d, long long ldy, void *stream);
+/* y[0..nCol) := A^T x[0..nRow) for handles created with options.transpose = 1; every y entry is overwritten (beta = 0).
+ * A^T is a matrix of the handle's own format converted from A's transposed COO, so these calls run that format's kernels
+ * on it and have the bits of b200spmv_multiply / b200spmv_multiply_f32 on a handle of the same format and options
+ * converted from the transposed triplets (nCol x nRow, sorted by (col, row)).  The scalars and arrays of A^T are read
+ * with the prefix "t." (t.nRow, t.crs_kernel, t.alg_bytes, t.ptr, ...; B200SPMV_ERR_STATE without A^T); the scalar
+ * "transpose" is 1 when A^T was built.  A^T has carry buffers of its own, but the one-stream-at-a-time rule covers the
+ * handle in both directions: do not overlap b200spmv_multiply and b200spmv_multiply_transpose on different streams.
+ * Errors, decided before any CUDA call and in this order: B200SPMV_ERR_INVALID (NULL handle), B200SPMV_ERR_STATE (before
+ * convert; handle created with transpose = 0), B200SPMV_ERR_INVALID (NULL x with nRow > 0, NULL y with nCol > 0), then
+ * the precision checks of b200spmv_multiply / _f32 (B200SPMV_ERR_STATE). */
+B200SPMV_API int b200spmv_multiply_transpose(b200spmv_matrix *m, const double *x_d, double *y_d, void *stream);
+B200SPMV_API int b200spmv_multiply_transpose_f32(b200spmv_matrix *m, const float *x_d, float *y_d, void *stream);
 /* Host semantics (what SpMV(A_opt, x_opt, y) means to the reference's driver): copies x H2D,
  * multiplies, copies y D2H, synchronises -- like src/opt_cusparse.cpp:72-82. */
 B200SPMV_API int b200spmv_multiply_host(b200spmv_matrix *m, const double *x_h, double *y_h);

@@ -21,7 +21,8 @@ class B200SpmvError(RuntimeError):
 
 class Options(C.Structure):
     _fields_ = [("segment_width", C.c_int), ("n_block", C.c_int), ("csr5_sigma", C.c_int),
-                ("ss_faithful", C.c_int), ("value_f32", C.c_int), ("crs_path", C.c_int), ("profile", C.c_int), ("col_blocks", C.c_int), ("precision", C.c_int), ("hyb_k", C.c_int), ("coo_path", C.c_int), ("reserved", C.c_int * 5)]
+                ("ss_faithful", C.c_int), ("value_f32", C.c_int), ("crs_path", C.c_int), ("profile", C.c_int), ("col_blocks", C.c_int), ("precision", C.c_int), ("hyb_k", C.c_int), ("coo_path", C.c_int),
+                ("transpose", C.c_int), ("reserved", C.c_int * 4)]
 
 
 class Stats(C.Structure):
@@ -56,6 +57,8 @@ def _load():
     lib.b200spmv_multiply_multi.argtypes = [vp, ip, vp, ll, vp, ll, vp]
     lib.b200spmv_multiply_multi_f32.argtypes = [vp, ip, vp, ll, vp, ll, vp]
     lib.b200spmv_multiply_f32.argtypes = [vp, vp, vp, vp]
+    lib.b200spmv_multiply_transpose.argtypes = [vp, vp, vp, vp]
+    lib.b200spmv_multiply_transpose_f32.argtypes = [vp, vp, vp, vp]
     lib.b200spmv_multiply_host_f32.argtypes = [vp, vp, vp]
     lib.b200spmv_multiply_rows.argtypes = [vp, ip, ip, vp, vp, vp]
     lib.b200spmv_prepare_rows.argtypes = [vp, ip, ip]

@@ -11,6 +11,9 @@ const char *last_error_cstr();
 int convert_row_blocked(int format, const b200spmv_options &opt, int nRow, int nCol, long long nnz, const int *row_d,
                         const int *col_d, const double *val_d, cudaStream_t s, std::unique_ptr<Format> &out);
 long long row_block_limit();
+// transpose.cu: A^T's sorted COO (nnz entries) from A's
+int transpose_coo(int nCol, long long nnz, const int *row_d, const int *col_d, const double *val_d, cudaStream_t s,
+                  DevBuf<int> &rowT, DevBuf<int> &colT, DevBuf<double> &valT);
 }
 using namespace b2;
 
@@ -22,6 +25,9 @@ struct b200spmv_matrix {
     b200spmv_options opt{};
     std::unique_ptr<Format> impl;
     bool converted = false, blocked = false;
+    // options.transpose = 1: A^T, converted from A's transposed COO with the same format and options (row-blocked on its own)
+    std::unique_ptr<Format> timpl;
+    bool tblocked = false;
     // plan of the host-semantics pipeline (built on first use)
     int plan_chunks = 0, plan_pieces = 0;
     int chunk_rb[MAX_HOST_CHUNKS + 1] = {}, chunk_need[MAX_HOST_CHUNKS] = {};
@@ -123,6 +129,7 @@ int b200spmv_create(int format, const b200spmv_options *opts, b200spmv_matrix **
         return B200SPMV_ERR_UNSUPPORTED;
     }
     if (o.precision < 0 || o.precision > 2) { set_error("create: precision=%d (0 fp64, 1 fp32, 2 fp32 with fp64 sums)", o.precision); return B200SPMV_ERR_INVALID; }
+    if (o.transpose != 0 && o.transpose != 1) { set_error("create: transpose=%d (0 or 1)", o.transpose); return B200SPMV_ERR_INVALID; }
     if (o.precision && format != B200SPMV_CRS && format != B200SPMV_ELL && format != B200SPMV_DIA && format != B200SPMV_CSR5) {
         set_error("create: the fp32 variant exists for the CRS, ELL, DIA and CSR5 formats");
         return B200SPMV_ERR_UNSUPPORTED;
@@ -146,6 +153,44 @@ int b200spmv_destroy(b200spmv_matrix *m)
     return B200SPMV_OK;
 }
 
+// Converts a sorted COO into impl: row blocks beyond row_block_limit(), else impl's own convert (a row-blocked impl is
+// replaced by a plain one first)
+static int convert_impl(int format, const b200spmv_options &opt, int nRow, int nCol, long long nnz, const int *row_d,
+                        const int *col_d, const double *val_d, cudaStream_t s, std::unique_ptr<Format> &impl,
+                        bool &blocked)
+{
+    if (nnz > row_block_limit()) {
+        // beyond the reference's int32 entry count (src/util.h:8): row blocks with 32-bit offsets each (blocked.cu)
+        std::unique_ptr<Format> f;
+        B2_TRY(convert_row_blocked(format, opt, nRow, nCol, nnz, row_d, col_d, val_d, s, f));
+        impl = std::move(f);
+        blocked = true;
+        return B200SPMV_OK;
+    }
+    if (blocked) {
+        impl.reset(make_format(format, opt));
+        blocked = false;
+    }
+    CooView A{nRow, nCol, (int)nnz, row_d, col_d, val_d};
+    return impl->convert(A, s);
+}
+
+// A^T: its COO (transpose.cu), then a fresh matrix of the handle's format and options converted from it like A
+static int convert_transpose(b200spmv_matrix *m, int nRow, int nCol, long long nnz, const int *row_d, const int *col_d,
+                             const double *val_d, cudaStream_t s)
+{
+    DevBuf<int> rowT, colT;
+    DevBuf<double> valT;
+    B2_TRY(transpose_coo(nCol, nnz, row_d, col_d, val_d, s, rowT, colT, valT));
+    b200spmv_options o = m->opt;
+    o.transpose = 0;
+    m->timpl.reset(make_format(m->format, o));
+    m->tblocked = false;
+    B2_TRY(convert_impl(m->format, o, nCol, nRow, nnz, rowT.p, colT.p, valT.p, s, m->timpl, m->tblocked));
+    B2_CUDA(cudaStreamSynchronize(s));                           // A^T's COO is freed on return
+    return B200SPMV_OK;
+}
+
 int b200spmv_convert_coo_device(b200spmv_matrix *m, int nRow, int nCol, long long nnz, const int *row_d,
                                 const int *col_d, const double *val_d, void *stream)
 {
@@ -156,22 +201,19 @@ int b200spmv_convert_coo_device(b200spmv_matrix *m, int nRow, int nCol, long lon
     B2_TRY(require_device());
     m->converted = false;
     m->plan_chunks = m->plan_pieces = 0;
-    if (nnz > row_block_limit()) {
-        // beyond the reference's int32 entry count (src/util.h:8): row blocks with 32-bit offsets each (blocked.cu)
-        std::unique_ptr<Format> f;
-        B2_TRY(convert_row_blocked(m->format, m->opt, nRow, nCol, nnz, row_d, col_d, val_d, (cudaStream_t)stream, f));
-        m->impl = std::move(f);
-        m->blocked = m->converted = true;
-        return B200SPMV_OK;
+    m->timpl.reset();                                           // the old A^T's memory is free while the new one is built
+    B2_TRY(convert_impl(m->format, m->opt, nRow, nCol, nnz, row_d, col_d, val_d, (cudaStream_t)stream, m->impl, m->blocked));
+    if (m->opt.transpose) {
+        const int st = convert_transpose(m, nRow, nCol, nnz, row_d, col_d, val_d, (cudaStream_t)stream);
+        if (st != B200SPMV_OK) {
+            m->timpl.reset();
+            const std::string why = last_error_cstr();
+            set_error("convert: the transposed conversion (A^T, %d x %d) failed: %s", nCol, nRow, why.c_str());
+            return st;
+        }
     }
-    if (m->blocked) {
-        m->impl.reset(make_format(m->format, m->opt));
-        m->blocked = false;
-    }
-    CooView A{nRow, nCol, (int)nnz, row_d, col_d, val_d};
-    int st = m->impl->convert(A, (cudaStream_t)stream);
-    if (st == B200SPMV_OK) m->converted = true;
-    return st;
+    m->converted = true;
+    return B200SPMV_OK;
 }
 
 int b200spmv_convert_coo_host(b200spmv_matrix *m, int nRow, int nCol, long long nnz, const int *row_h,
@@ -214,6 +256,29 @@ int b200spmv_multiply(b200spmv_matrix *m, const double *x_d, double *y_d, void *
 {
     B2_TRY(check_ready(m, x_d, y_d));
     return m->impl->multiply(x_d, y_d, (cudaStream_t)stream);
+}
+
+// y[0..nCol) := A^T x[0..nRow): A^T's matrix multiplies like any other (x and y swap their lengths)
+static int check_transpose_ready(b200spmv_matrix *m, const void *x, const void *y, const char *who)
+{
+    clear_error();
+    if (!m) { set_error("%s: NULL handle", who); return B200SPMV_ERR_INVALID; }
+    if (!m->converted) { set_error("%s: matrix not converted yet", who); return B200SPMV_ERR_STATE; }
+    if (!m->timpl) { set_error("%s: the handle was created with transpose = 0 (no A^T)", who); return B200SPMV_ERR_STATE; }
+    if ((!x && m->timpl->nCol > 0) || (!y && m->timpl->nRow > 0)) { set_error("%s: NULL vector", who); return B200SPMV_ERR_INVALID; }
+    return B200SPMV_OK;
+}
+
+int b200spmv_multiply_transpose(b200spmv_matrix *m, const double *x_d, double *y_d, void *stream)
+{
+    B2_TRY(check_transpose_ready(m, x_d, y_d, "multiply_transpose"));
+    return m->timpl->multiply(x_d, y_d, (cudaStream_t)stream);
+}
+
+int b200spmv_multiply_transpose_f32(b200spmv_matrix *m, const float *x_d, float *y_d, void *stream)
+{
+    B2_TRY(check_transpose_ready(m, x_d, y_d, "multiply_transpose_f32"));
+    return m->timpl->multiply_f32(x_d, y_d, (cudaStream_t)stream);
 }
 
 int b200spmv_multiply_multi(b200spmv_matrix *m, int k, const double *X_d, long long ldx, double *Y_d, long long ldy,
@@ -426,6 +491,12 @@ int b200spmv_get_scalar(b200spmv_matrix *m, const char *name, long long *out)
     if (!m->converted) { set_error("get_scalar: matrix not converted yet"); return B200SPMV_ERR_STATE; }
     std::string n(name);
     Format *f = m->impl.get();
+    if (n == "transpose") { *out = m->timpl ? 1 : 0; return B200SPMV_OK; }
+    if (n.compare(0, 2, "t.") == 0) {                           // t.<name>: the same scalar of A^T
+        if (!m->timpl) { set_error("get_scalar: '%s' names A^T, and the handle was created with transpose = 0", name); return B200SPMV_ERR_STATE; }
+        f = m->timpl.get();
+        n.erase(0, 2);
+    }
     if (n == "nRow") { *out = f->nRow; return B200SPMV_OK; }
     if (n == "nCol") { *out = f->nCol; return B200SPMV_OK; }
     if (n == "nNnz") { if (!f->scalar(n, out)) *out = f->nnz; return B200SPMV_OK; }
@@ -440,7 +511,14 @@ long long b200spmv_get_array(b200spmv_matrix *m, const char *name, void *dst_h, 
 {
     if (!m || !name) { set_error("get_array: NULL argument"); return B200SPMV_ERR_INVALID; }
     if (!m->converted) { set_error("get_array: matrix not converted yet"); return B200SPMV_ERR_STATE; }
-    long long r = m->impl->array(std::string(name), dst_h, dst_bytes);
+    std::string n(name);
+    Format *f = m->impl.get();
+    if (n.compare(0, 2, "t.") == 0) {                           // t.<name>: the same array of A^T
+        if (!m->timpl) { set_error("get_array: '%s' names A^T, and the handle was created with transpose = 0", name); return B200SPMV_ERR_STATE; }
+        f = m->timpl.get();
+        n.erase(0, 2);
+    }
+    long long r = f->array(n, dst_h, dst_bytes);
     if (r == -1000) {
         set_error("get_array: format %d has no array '%s'", m->format, name);
         return B200SPMV_ERR_INVALID;

@@ -259,6 +259,10 @@ int b200spmv_mg_create(int nGPU, int format, const b200spmv_options *opts, b200s
     clear_error();
     if (!out || nGPU < 1) { set_error("mg_create: bad argument"); return B200SPMV_ERR_INVALID; }
     *out = nullptr;
+    if (opts && opts->transpose) {                              // a block's local A^T is not a block of the global A^T
+        set_error("mg_create: options.transpose is not supported by the multi-GPU handle");
+        return B200SPMV_ERR_UNSUPPORTED;
+    }
     int have = 0;
     if (cudaGetDeviceCount(&have) != cudaSuccess || have < nGPU) {
         cudaGetLastError();

@@ -109,12 +109,13 @@ class SpMatOpt:
     ``scalar(name)`` / ``array(name, dtype)`` read the fields back under the reference's names, in the
     reference's logical layout, for parity checks."""
 
-    def __init__(self, fmt, segment_width=0, n_block=0, csr5_sigma=0, ss_faithful=0, value_f32=0, crs_path=0, profile=0, col_blocks=0, hyb_k=0, precision=0, coo_path=0):
+    def __init__(self, fmt, segment_width=0, n_block=0, csr5_sigma=0, ss_faithful=0, value_f32=0, crs_path=0, profile=0, col_blocks=0, hyb_k=0, precision=0, coo_path=0,
+                 transpose=0):
         self.fmt = fmt
         o = Options()
         o.segment_width, o.n_block, o.csr5_sigma, o.ss_faithful = segment_width, n_block, csr5_sigma, ss_faithful
         o.value_f32, o.crs_path, o.profile, o.col_blocks = value_f32, crs_path, profile, col_blocks
-        o.hyb_k, o.precision, o.coo_path = hyb_k, precision, coo_path
+        o.hyb_k, o.precision, o.coo_path, o.transpose = hyb_k, precision, coo_path, transpose
         self.h = C.c_void_p()
         check(lib.b200spmv_create(FORMATS[fmt], C.byref(o), C.byref(self.h)))
         self.nRow = self.nCol = self.nNnz = 0
@@ -161,6 +162,17 @@ class SpMatOpt:
         """Y[:, :k] := A X[:, :k] for k = 1..8 device-resident row-major vectors (X[c*ldx + j], Y[r*ldy + j]): the matrix is
         streamed once for all k.  CRS handles with fp64 values and vectors (b200spmv_multiply_multi)."""
         check(lib.b200spmv_multiply_multi(self.h, k, C.c_void_p(X_ptr), ldx, C.c_void_p(Y_ptr), ldy, stream))
+
+    def multiply_transpose(self, x_ptr, y_ptr, stream=None):
+        """y := A^T x for device-resident vectors, x of nRow and y of nCol entries (b200spmv_multiply_transpose).  Handles
+        created with transpose=1, which convert A^T as a second matrix of the same format; its scalars and arrays are read
+        with the prefix "t." (scalar("t.nRow"), array("t.ptr", ...))."""
+        check(lib.b200spmv_multiply_transpose(self.h, C.c_void_p(x_ptr), C.c_void_p(y_ptr), stream))
+
+    def multiply_transpose_f32(self, x_ptr, y_ptr, stream=None):
+        """y := A^T x with fp32 vectors: multiply_transpose for handles created with transpose=1 and precision=1 or 2
+        (b200spmv_multiply_transpose_f32)."""
+        check(lib.b200spmv_multiply_transpose_f32(self.h, C.c_void_p(x_ptr), C.c_void_p(y_ptr), stream))
 
     def multiply_rows(self, row_begin, row_end, x_ptr, y_ptr, stream=None):
         check(lib.b200spmv_multiply_rows(self.h, row_begin, row_end, C.c_void_p(x_ptr), C.c_void_p(y_ptr), stream))
