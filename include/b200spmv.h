@@ -92,7 +92,10 @@ typedef struct {
                             x and y are float arrays, products and sums in fp32; 2 = the same storage and vectors with
                             fp64 products and sums.  Multiply with b200spmv_multiply_f32 / _host_f32; tolerance 1e-5
                             against the reference's (fp64) CRS result.  Halves the bytes of every array but the indices */
-    int hyb_k;           /* HYB: width of the ELL part; 0 = the largest width that max(4096, nRow/3) rows still fill */
+    int hyb_k;           /* HYB: width K of the ELL part (the first K entries of every row; the rest form the COO tail).
+                            0 = the largest width k <= 4096 that at least min(nRow, max(4096, nRow/3)) rows fill (rows
+                            longer than 4096 count as 4096 long, so K never exceeds 4096); K = 1 when no width qualifies,
+                            0 for a matrix without entries.  n > 0 = min(n, longest row).  Negative values are rejected */
     int coo_path;        /* COO: 0 = entry stream (segmented warp scans; sums re-associated within 1e-12), fed by TMA bulk copies or
                             by the lanes' own loads, whichever suits the matrix; 1 = the order-preserving tile kernel (rows <= 64
                             entries bit-identical to the CRS result); 2 / 3 = force the load-fed / the TMA-fed entry stream;

@@ -124,6 +124,10 @@ int b200spmv_create(int format, const b200spmv_options *opts, b200spmv_matrix **
         set_error("create: bad option (crs_path=%d, 0..4 without 2; coo_path=%d, 0..3)", o.crs_path, o.coo_path);
         return B200SPMV_ERR_INVALID;
     }
+    if (o.hyb_k < 0) {
+        set_error("create: hyb_k=%d (0 = the width rule, > 0 = that width)", o.hyb_k);
+        return B200SPMV_ERR_INVALID;
+    }
     if (o.value_f32 && format != B200SPMV_CRS) {
         set_error("create: value_f32 is implemented for the CRS format only");
         return B200SPMV_ERR_UNSUPPORTED;

@@ -128,7 +128,7 @@ def test_multiply_rows(sp, oracle, fmt, opt):
     torch.cuda.synchronize()
     y = yd.cpu().numpy()
     assert np.all(y[:1000] == -3.0) and np.all(y[2000:] == -3.0) and np.array_equal(y[1000:2000], y_ref[1000:2000]) or fmt == "css"
-    for bad in ("coo", "jds", "csr5"):
+    for bad in ("coo", "jds", "csr5", "hyb"):
         B_opt, _ = run_host(sp, bad, 3, 3, [0, 1], [0, 1], [1.0, 2.0], np.ones(3))
         with pytest.raises(sp.B200SpmvError) as e:
             B_opt.multiply_rows(0, 1, xd.data_ptr(), yd.data_ptr())
@@ -846,7 +846,7 @@ def test_row_blocked_matches_unblocked(sp, oracle, fmt, monkeypatch):
             ys.append(y.cpu().numpy())
         y_ref = oracle.crs_result(nr, row, col, val, x)
         assert_y(ys[1], y_ref, row, col, val, x, nr)
-        if fmt in ("crs", "ell", "jds", "dia", "ss"):          # one thread per row of at most 64 entries either way
+        if fmt in ("crs", "ell", "jds", "dia", "ss", "hyb"):   # one thread per row of at most 64 entries either way
             short = np.bincount(row, minlength=nr) <= 64
             assert np.array_equal(ys[0][short], ys[1][short]), fmt
         if cut.scalar("has_rows"):
