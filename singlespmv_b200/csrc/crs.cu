@@ -42,6 +42,9 @@ struct CrsFormat : Format {
     {
         nRow = A.nRow; nCol = A.nCol; nnz = A.nnz;
         rowOffset = A.rowOffset;
+        // the entry stream borrows ptr / idx / val, which are reallocated below; the multi-vector multiplies build it
+        // lazily on tile-stream handles and must find nothing of an earlier matrix
+        es.reset();
         B2_TRY(validate_sorted_coo(A, s));
         B2_TRY(ptr.alloc((size_t)nRow + 1));
         B2_TRY(idx.alloc((size_t)nnz + CS_SLACK));

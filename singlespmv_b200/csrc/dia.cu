@@ -13,6 +13,7 @@
 // windows from L2 instead of 27.  Per row the diagonals are accumulated in ascending order with
 // unfused mul/add = the reference's order (and, padding zeros aside, opt_crs.cpp's) -> bit-identical y.
 #include <algorithm>
+#include <set>
 
 #include "common.cuh"
 
@@ -23,7 +24,7 @@ constexpr int DIA_RPT = 2;
 constexpr int DIA_R = DIA_THREADS * DIA_RPT;
 constexpr int DIA_MAX_DIAG = 64;     // TMA variant: per-diagonal window bases live in shared memory
 constexpr int DIA_MAX_RUNS = 16;
-
+constexpr int DIA_MAX_SMEM = 200 * 1024;   // TMA variant: largest x-window staging a handle may ask for
 
 struct DiaRuns {
     int n;
@@ -255,6 +256,21 @@ dia_spmv_f32_kernel(const float *__restrict__ diag, size_t ld, int nDiag, const 
     y[r] = (float)acc;
 }
 
+// Windows beyond the default 48 KB of dynamic shared memory need the kernels' opt-in limit raised.  That limit belongs
+// to the kernel on a device, not to a handle, so it is raised once per device to the largest size any handle may ask
+// for: a handle converted later can never lower it below what a live handle launches with.
+static int dia_tma_allow_max_smem()
+{
+    static std::set<int> raised;
+    int dev = 0;
+    B2_CUDA(cudaGetDevice(&dev));
+    if (raised.count(dev)) return B200SPMV_OK;
+    for (auto kern : {dia_spmv_tma_kernel<5, 6>, dia_spmv_tma_kernel<7, 5>, dia_spmv_tma_kernel<3, 8>})
+        B2_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, DIA_MAX_SMEM));
+    raised.insert(dev);
+    return B200SPMV_OK;
+}
+
 struct DiaFormat : Format {
     int nDiag = 0;
     size_t ld = 0;
@@ -336,12 +352,8 @@ struct DiaFormat : Format {
                 soff += (DIA_R + runs.cnt[g] + 1 + 1) & ~1;       // window + alignment slack, kept even
             }
             smem_bytes = (size_t)soff * sizeof(double);
-            if (smem_bytes > 200 * 1024) tma_ok = false;
-            else if (smem_bytes > 48 * 1024) {
-                B2_CUDA(cudaFuncSetAttribute(dia_spmv_tma_kernel<5, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
-                B2_CUDA(cudaFuncSetAttribute(dia_spmv_tma_kernel<7, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
-                B2_CUDA(cudaFuncSetAttribute(dia_spmv_tma_kernel<3, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
-            }
+            if (smem_bytes > DIA_MAX_SMEM) tma_ok = false;
+            else if (smem_bytes > 48 * 1024) B2_TRY(dia_tma_allow_max_smem());
         }
         return B200SPMV_OK;
     }

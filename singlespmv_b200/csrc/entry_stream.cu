@@ -558,21 +558,35 @@ static int zero_rows_multi_t(int nRow, int k, XT *Y, long long ldy, cudaStream_t
 int zero_rows_multi(int nRow, int k, double *Y, long long ldy, cudaStream_t s) { return zero_rows_multi_t(nRow, k, Y, ldy, s); }
 int zero_rows_multi(int nRow, int k, float *Y, long long ldy, cudaStream_t s) { return zero_rows_multi_t(nRow, k, Y, ldy, s); }
 
+void EntryStream::reset()
+{
+    ptr = idx = nullptr;
+    val = nullptr;
+    f32 = false;
+    nRow = nnz = 0;
+    ok = tma = false;
+    nTiles = nEmpty = 0;
+    bits.release();
+    grpRun.release();
+    nzrow.release();
+    empty.release();
+    carry.release();
+    carryK.release();
+    range_cache.clear();
+}
+
 int EntryStream::build(const int *ptr_d, const int *idx_d, const void *val_d, bool val_is_f32, int nRow_, int nnz_,
                        bool gather_bound, cudaStream_t s)
 {
+    reset();
     ptr = ptr_d; idx = idx_d; val = val_d; f32 = val_is_f32; nRow = nRow_; nnz = nnz_;
-    ok = false;
-    range_cache.clear();
-    carryK.release();
     if (nnz <= 0 || nRow <= 0) return B200SPMV_OK;
     tma = !gather_bound;
     nTiles = ceil_div(nnz, ES_E);
     const int nGroups = ceil_div((long long)nTiles * ES_E, 128);
     B2_TRY(bits.alloc((size_t)nGroups * 4 + 4));
     B2_TRY(grpRun.alloc((size_t)nGroups + 1));
-    if (f32) carry.release();                              // run_rows (fp64 only) owns these; run_multi* use carryK
-    else B2_TRY(carry.alloc((size_t)nTiles));
+    if (!f32) B2_TRY(carry.alloc((size_t)nTiles));         // run_rows (fp64 only) owns these; run_multi* use carryK
     B2_CUDA(cudaMemsetAsync(bits.p, 0, bits.bytes(), s));
     DevBuf<int> cnt;
     B2_TRY(cnt.alloc(1));
@@ -592,8 +606,6 @@ int EntryStream::build(const int *ptr_d, const int *idx_d, const void *val_d, bo
         B2_TRY(nzrow.alloc((size_t)(nRow - nEmpty)));
         es_nzrow_kernel<<<ceil_div(nRow, 256), 256, 0, s>>>(ptr, nRow, bits.p, grpRun.p, nzrow.p);
         B2_KERNEL_CHECK();
-    } else {
-        nzrow.release();
     }
     B2_CUDA(cudaStreamSynchronize(s));
     ok = true;

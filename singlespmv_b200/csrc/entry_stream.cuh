@@ -47,6 +47,10 @@ struct EntryStream {
     // val_is_f32: fp32 values, for run_multi_f32 only (the metadata does not depend on the value type)
     int build(const int *ptr_d, const int *idx_d, const void *val_d, bool val_is_f32, int nRow_, int nnz_, bool gather_bound,
               cudaStream_t s);
+    // back to the state of a new EntryStream: ok = false, borrowed pointers and shape cleared, metadata, carries and
+    // cached row ranges released.  build() starts with it; a conversion that does not build the entry stream calls it,
+    // so nothing of an earlier matrix survives.
+    void reset();
     int prepare(int rb, int re);
     int run_rows(const double *x, double *y, int rb, int re, cudaStream_t s);
     // Y[:, 0..k) := A X[:, 0..k) over all rows (k <= ES_KMAX, row-major); each column is summed as run_rows sums it.
