@@ -365,6 +365,20 @@ int ChunkStream::build(const int *ptr_d, const int *idx_d, const void *val_d, bo
     return B200SPMV_OK;
 }
 
+// CTAs per SM of the single multiply, from the occupancy limit: shed CTAs while their stages take more than
+// CS_SMEM_PER_SM of the SM's 256 KB of L1 and shared memory, but never below CS_MIN_THREADS_PER_SM threads.  The stages
+// hold the values only, so the L1 the gathers of x hit in is what the stages leave.  Measured on c5 (B200, fp64,
+// dictionary feed, profiles/chunk_ctas_ab.md): 6 CTAs of 29.9 KB (180 KB) lost to 5 (150 KB) in every session; 4 CTAs
+// (1024 threads) lost to both; fp32 at 8 CTAs of 15.6 KB (125 KB) lost 4 % at 6 and 9 % at 5.
+constexpr size_t CS_SMEM_PER_SM = 160 * 1024;
+constexpr int CS_MIN_THREADS_PER_SM = 1280;
+static int cs_ctas_per_sm(int occupancy, int th, size_t smem)
+{
+    int n = occupancy;
+    while ((n - 1) * th >= CS_MIN_THREADS_PER_SM && (size_t)n * smem > CS_SMEM_PER_SM) n--;
+    return n;
+}
+
 // the launch of one feed
 template <typename VT, typename XT, typename AT, int MAXL, int TH, bool ACC, bool DICT>
 static int cs_launch(const ChunkStream &c, const XT *x, XT *y, int rb, int re, int acc, cudaStream_t s)
@@ -391,7 +405,7 @@ static int cs_launch(const ChunkStream &c, const XT *x, XT *y, int rb, int re, i
         if (n < 1) { set_error("row-chunk stream: %zu bytes of shared memory do not fit", smem); return B200SPMV_ERR_UNSUPPORTED; }
         it = per_sm.emplace(key, n).first;
     }
-    const int perSm = env_b > 0 ? std::min(it->second, env_b) : it->second;
+    const int perSm = env_b > 0 ? std::min(it->second, env_b) : cs_ctas_per_sm(it->second, TH, smem);
     const int chunk0 = rb / TH, nChunks = ceil_div(re, TH) - chunk0;
     const int grid = std::min(nChunks, sms * perSm);
     kern<<<grid, TH, smem, s>>>(c.ptr, c.idx, c.meta.p, static_cast<const VT *>(c.val), x, y, rb, re, chunk0, nChunks, capI, capV, S, acc);
