@@ -24,6 +24,15 @@
  *     overlap it with b200spmv_multiply on the same handle)
  *   - there is NO CPU fallback: without a CUDA device every compute entry fails with
  *     B200SPMV_ERR_CUDA.
+ *   - signed zeros, infinities and NaN (stored-entry semantics; every format and path but DIA and ss_faithful SS / CSS):
+ *     y[i] depends only on the stored entries of row i and on x at their columns.  With p = a * x[c] the exact products
+ *     of those entries, y[i] is NaN if any p is NaN (a NaN in x or A, a stored 0 times +-Inf) or if the row has both
+ *     +Inf and -Inf products; else +-Inf if it has infinite products of one sign; else finite.  This holds whatever
+ *     order a kernel sums in, as long as the finite part of the row cannot overflow.  A row whose products are all +-0
+ *     (an empty row too) is +0.0.  No kernel reads x for a slot that holds no entry (padding, ragged tile ends).
+ *   - DIA and SS / CSS with ss_faithful = 1 have the reference's padding semantics instead: they run the reference's own
+ *     operations, 0 * x over its padding included (DIA cannot tell padding from stored zeros), and give its bits.
+ *   - results claimed bit-identical to the reference are so on the bits, NaN aside: a NaN's payload is unspecified.
  */
 #ifndef B200SPMV_H
 #define B200SPMV_H

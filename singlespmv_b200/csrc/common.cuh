@@ -153,7 +153,7 @@ int max_row_length(const int *ptr_d, int nRow, int *out_h, cudaStream_t s);
 int exclusive_scan_i32(const int *in_d, int *out_d, int n, cudaStream_t s);
 int exclusive_scan_i64(const long long *in_d, long long *out_d, int n, cudaStream_t s);
 int sum_i32_as_i64(const int *in_d, int n, long long *out_h, cudaStream_t s);
-// min and max of in_d[b..e) (e > b); synchronous
+// min and max of the non-negative values of in_d[b..e) (negative ones are ELL padding); synchronous
 int minmax_i32(const int *in_d, long long b, long long e, int *mn_h, int *mx_h);
 // largest |col - row| (synchronises); gathers_need_l2: the x entries a stretch of rows touches span more than 32 MB
 int max_band(const int *row_d, const int *col_d, int nnz, int rowOffset, int *band_h, cudaStream_t s);

@@ -290,7 +290,10 @@ coo_stream_kernel(const int *__restrict__ row, const int *__restrict__ col, cons
                     v0.x = e < n ? V[e] : 0.0; v0.y = e + 1 < n ? V[e + 1] : 0.0; v1.x = e + 2 < n ? V[e + 2] : 0.0; v1.y = e + 3 < n ? V[e + 3] : 0.0;
                 }
                 const double x0 = ld_x(x + c.x, pol_x), x1 = ld_x(x + c.y, pol_x), x2 = ld_x(x + c.z, pol_x), x3 = ld_x(x + c.w, pol_x);
-                const double p0 = __dmul_rn(v0.x, x0), p1 = __dmul_rn(v0.y, x1), p2 = __dmul_rn(v1.x, x2), p3 = __dmul_rn(v1.y, x3);
+                double p0 = __dmul_rn(v0.x, x0), p1 = __dmul_rn(v0.y, x1), p2 = __dmul_rn(v1.x, x2), p3 = __dmul_rn(v1.y, x3);
+                if (!fullGroup) {                             // a missing entry adds +0.0, not 0 * x[0] (NaN if x[0] is)
+                    p0 = e < n ? p0 : 0.0; p1 = e + 1 < n ? p1 : 0.0; p2 = e + 2 < n ? p2 : 0.0; p3 = e + 3 < n ? p3 : 0.0;
+                }
                 int rprev = __shfl_up_sync(0xffffffffu, r.w, 1);
                 if (lane == 0) rprev = lastRow;
                 const bool b0 = r.x != rprev, b1 = r.y != r.x, b2 = r.z != r.y, b3 = r.w != r.z;
@@ -306,7 +309,7 @@ coo_stream_kernel(const int *__restrict__ row, const int *__restrict__ col, cons
                     auto step = [&](bool b, int rp, int rc, double p) {
                         if (b) {
                             if (!seen) head = acc;
-                            else y[rp] = acc;                 // a run that started and ended in this lane
+                            else y[rp] = __dadd_rn(acc, 0.0); // a run that started and ended in this lane (+ 0.0: see below)
 #pragma unroll 1
                             for (int z = rp + 1; z < rc; z++) y[z] = 0.0;  // empty rows in front of the new run (beta = 0)
                             seen = true;
@@ -352,7 +355,7 @@ coo_stream_kernel(const int *__restrict__ row, const int *__restrict__ col, cons
                     // this lane's first start closes the run that was open in front of it
                     const double total = __dadd_rn(excl, head);
                     const bool firstInChunk = !started && !(m & ((1u << lane) - 1u));
-                    if (!firstInChunk) y[rprev] = total;
+                    if (!firstInChunk) y[rprev] = __dadd_rn(total, 0.0);   // + 0.0: a run of -0.0 products (acc = p) gives +0.0
                     else piece = total;                       // continues a run of an earlier chunk (0 if the chunk begins with a start)
                 }
                 if (!started && m) piece = __shfl_sync(0xffffffffu, piece, __ffs(m) - 1);
@@ -385,12 +388,12 @@ coo_stream_kernel(const int *__restrict__ row, const int *__restrict__ col, cons
                 if (accRow >= 0) a2 = __dadd_rn(a2, oPiece);
                 else tilePiece = __dadd_rn(tilePiece, oPiece);
                 if (oRow >= 0) {
-                    if (accRow >= 0) y[accRow] = a2;
+                    if (accRow >= 0) y[accRow] = __dadd_rn(a2, 0.0);
                     accRow = oRow;
                     a2 = oTail;
                 }
             }
-            if (accRow >= 0) y[accRow] = a2;
+            if (accRow >= 0) y[accRow] = __dadd_rn(a2, 0.0);
             carry[t] = tilePiece;
         }
         if (TMA && tid == 0 && t + 2 * (int)gridDim.x < nTiles) issue(s, t + 2 * gridDim.x);

@@ -2,7 +2,9 @@
 // K = longest row :28-31, slot k >= len padded with col = k, val = 0 :46-52, multiply over all K
 // slots :75-89).  Device layout = sliced ELL: slices of 32 rows (one warp), slice-local width
 // rounded to V slots, stored [slice][k/V][lane][V] so that a lane reads V column ids and V
-// values with 128-bit loads and a warp request is one contiguous 512 B / 1 KB run.
+// values with 128-bit loads and a warp request is one contiguous 512 B / 1 KB run.  Padding
+// slots hold ELL_PAD and take +0.0 for x (a NaN or Inf in x reaches only the rows that store
+// it); the exported arrays show them as the reference's col = k, val = 0.
 #include "colblocks.cuh"
 #include "common.cuh"
 
@@ -25,11 +27,16 @@ __global__ void ell_slice_groups_kernel(const int *__restrict__ beg, const int *
     if (lane == 0) groups[s] = (len + V - 1) / V;
 }
 
-// padCol: column of the slots beyond K (0 for the format's own layout; the first column of the block for a column block)
+// Padding slots (the reference's K slots beyond a row's length, the slots that round a slice up to V, a column block's
+// padding) hold the column ELL_PAD and value 0: the kernel takes +0.0 for their x (ell_x), so a NaN or Inf in x reaches
+// only the rows that store its column.  The logical export (ell_logical_kernel) shows them as the reference's col = k,
+// val = 0.
+constexpr int ELL_PAD = -1;
+
 template <int V, typename VT>
 __global__ void ell_fill_kernel(const int *__restrict__ beg, const int *__restrict__ end, const int *__restrict__ col,
                                 const double *__restrict__ val, int nRow, int nSlices,
-                                const long long *__restrict__ slice_off, int K, int padCol, int *__restrict__ ecol,
+                                const long long *__restrict__ slice_off, int *__restrict__ ecol,
                                 VT *__restrict__ eval)
 {
     const int s = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -44,11 +51,18 @@ __global__ void ell_fill_kernel(const int *__restrict__ beg, const int *__restri
             const int k = (int)(g - g0) * V + j;
             const size_t at = ((size_t)g * 32 + lane) * V + j;
             const bool real = k < len;
-            // padding: col = slot index (opt_ell.cpp:48) for the reference's K slots; the extra slots that round a
-            // slice up to V (k >= K, never exported) point at column 0 so that no gather leaves x when K is close to nCol
-            ecol[at] = real ? col[b + k] : ((r < nRow && k < K) ? k : padCol);
+            ecol[at] = real ? col[b + k] : ELL_PAD;
             eval[at] = real ? (VT)val[b + k] : (VT)0;      // fp32 storage: rounded to nearest once, here
         }
+}
+
+// x at a slot's column; +0.0 at a padding slot.  The gather itself always runs (x[0] for padding): loads predicated on
+// the column made c4 ELL 1.5-2 % slower on a B200.
+template <typename XT>
+__device__ __forceinline__ XT ell_x(const XT *x, int c, uint64_t pol)
+{
+    const XT v = ld_x(x + max(c, 0), pol);
+    return c == ELL_PAD ? (XT)0 : v;
 }
 
 template <int V, typename VT> struct EllGroup {
@@ -95,7 +109,8 @@ __device__ __forceinline__ void ell_load(EllGroup<V, float> &g, const int *ecol,
 
 
 // One lane per row; the K-loop runs in ascending slot order with unfused mul/add, i.e. the
-// reference's own order -> y is bit-identical to opt_ell.cpp / opt_crs.cpp (fp64).
+// reference's own order -> y is bit-identical to opt_ell.cpp / opt_crs.cpp (fp64).  A padding slot adds 0 * 0 = +0.0,
+// which leaves the sum (seeded with +0.0 or a y that was) as it is.
 // VT = stored value type, XT = type of x and y, AT = type of the products and the row sum.
 // ACC = CS_CONTINUE: the row sums continue what y holds (acc = y[r]; ...; y[r] = acc): the next column block of the same
 // running sum.  ACC = CS_ADD: y[r] = y[r] + sum (CSS adds its block sums, src/opt_css.cpp:298).
@@ -121,9 +136,9 @@ ell_spmv_kernel(const long long *__restrict__ slice_off, const int *__restrict__
         ell_load<V>(b, ecol, eval, ((size_t)(g + 1) * 32 + lane) * V, pol_stream);
         XT xa[V], xb[V];
 #pragma unroll
-        for (int j = 0; j < V; j++) xa[j] = ld_x(x + a.c[j], pol_x);
+        for (int j = 0; j < V; j++) xa[j] = ell_x(x, a.c[j], pol_x);
 #pragma unroll
-        for (int j = 0; j < V; j++) xb[j] = ld_x(x + b.c[j], pol_x);
+        for (int j = 0; j < V; j++) xb[j] = ell_x(x, b.c[j], pol_x);
 #pragma unroll
         for (int j = 0; j < V; j++) acc = Arith<AT>::add(acc, Arith<AT>::mul((AT)xa[j], (AT)a.v[j]));
 #pragma unroll
@@ -134,7 +149,7 @@ ell_spmv_kernel(const long long *__restrict__ slice_off, const int *__restrict__
         ell_load<V>(a, ecol, eval, ((size_t)g * 32 + lane) * V, pol_stream);
         XT xa[V];
 #pragma unroll
-        for (int j = 0; j < V; j++) xa[j] = ld_x(x + a.c[j], pol_x);
+        for (int j = 0; j < V; j++) xa[j] = ell_x(x, a.c[j], pol_x);
 #pragma unroll
         for (int j = 0; j < V; j++) acc = Arith<AT>::add(acc, Arith<AT>::mul((AT)xa[j], (AT)a.v[j]));
     }
@@ -154,7 +169,7 @@ __global__ void ell_logical_kernel(const long long *__restrict__ slice_off, cons
     const long long g0 = slice_off[s], g1 = slice_off[s + 1];
     if (k < (int)(g1 - g0) * V) {
         const size_t at = ((size_t)(g0 + k / V) * 32 + lane) * V + k % V;
-        lcol[i] = ecol[at];
+        lcol[i] = ecol[at] == ELL_PAD ? k : ecol[at];
         lval[i] = (double)eval[at];
     } else {
         lcol[i] = k;
@@ -190,8 +205,8 @@ struct EllFormat : Format {
         else B2_TRY(eval.alloc((size_t)slots));
         if (nSlices) {
             const int grid = ceil_div((long long)nSlices * 32, 256);
-            if (prec) ell_fill_kernel<VV, float><<<grid, 256, 0, s>>>(ptr, ptr + 1, A.col, A.val, nRow, nSlices, slice_off.p, K, 0, ecol.p, eval32.p);
-            else ell_fill_kernel<VV, double><<<grid, 256, 0, s>>>(ptr, ptr + 1, A.col, A.val, nRow, nSlices, slice_off.p, K, 0, ecol.p, eval.p);
+            if (prec) ell_fill_kernel<VV, float><<<grid, 256, 0, s>>>(ptr, ptr + 1, A.col, A.val, nRow, nSlices, slice_off.p, ecol.p, eval32.p);
+            else ell_fill_kernel<VV, double><<<grid, 256, 0, s>>>(ptr, ptr + 1, A.col, A.val, nRow, nSlices, slice_off.p, ecol.p, eval.p);
             B2_KERNEL_CHECK();
         }
         return B200SPMV_OK;
@@ -239,7 +254,7 @@ struct EllFormat : Format {
         if (rb < 0 || re > nRow || rb > re) { set_error("col_extent: bad row range [%d,%d)", rb, re); return B200SPMV_ERR_INVALID; }
         if (rb == re) { *cmin = 0; *cmax = -1; return B200SPMV_OK; }
         if ((cb != nullptr)) return Format::col_extent(rb, re, cmin, cmax);
-        long long g[2] = {0, 0};                        // whole slices: padding columns (slot numbers) included
+        long long g[2] = {0, 0};                        // whole slices (minmax_i32 passes over the padding)
         B2_CUDA(cudaMemcpy(&g[0], slice_off.p + rb / 32, sizeof(long long), cudaMemcpyDeviceToHost));
         B2_CUDA(cudaMemcpy(&g[1], slice_off.p + ceil_div(re, 32), sizeof(long long), cudaMemcpyDeviceToHost));
         if (g[1] <= g[0]) { *cmin = 0; *cmax = -1; return B200SPMV_OK; }
@@ -362,8 +377,8 @@ struct EllColBlocks : ColBlockEngine {
             B2_TRY(k->ecol.alloc((size_t)k->slots));
             B2_TRY(k->eval.alloc((size_t)k->slots));
             if (nSlices) {
-                ell_fill_kernel<2, double><<<ceil_div((long long)nSlices * 32, 256), 256, 0, s>>>(beg, end, A.col, A.val, nRow, nSlices, k->slice_off.p, 0,
-                                                                                                 (int)std::min<long long>((long long)b * B, A.nCol - 1), k->ecol.p, k->eval.p);
+                ell_fill_kernel<2, double><<<ceil_div((long long)nSlices * 32, 256), 256, 0, s>>>(beg, end, A.col, A.val, nRow, nSlices, k->slice_off.p,
+                                                                                                 k->ecol.p, k->eval.p);
                 B2_KERNEL_CHECK();
             }
             blk.push_back(std::move(k));

@@ -87,9 +87,11 @@ entry_stream_kernel(const int *__restrict__ idx, const double *__restrict__ val,
     const uint64_t pol_stream = policy_evict_first(), pol_x = policy_evict_last();
     const unsigned lt = (1u << lane) - 1u;
 
-    auto store = [&](int run, double v) {                   // y of the run-th non-empty row, if the caller asked for that row
+    // y of the run-th non-empty row, if the caller asked for that row.  + 0.0 turns a sum of -0.0 products (a run that
+    // starts with acc = p) into +0.0, as the reference's sum from +0.0 gives; it changes no other value
+    auto store = [&](int run, double v) {
         const int r = nzrow ? nzrow[run] : run;
-        if (r >= rowLo && r < rowHi) y[r] = v;
+        if (r >= rowLo && r < rowHi) y[r] = __dadd_rn(v, 0.0);
     };
     auto issue = [&](int s, int t) {                        // thread 0 only
         const long long t0 = (long long)t * E;
@@ -130,7 +132,8 @@ entry_stream_kernel(const int *__restrict__ idx, const double *__restrict__ val,
                 const long long ge = t0 + e;                // global entry index of the lane's first entry
                 int4 c;
                 double2 v0, v1;
-                if (c0 + g * 128 + 128 <= n) {
+                const bool full = c0 + g * 128 + 128 <= n;
+                if (full) {
                     if (TMA) {
                         c = *reinterpret_cast<const int4 *>(Cc + e);
                         v0 = *reinterpret_cast<const double2 *>(V + e);
@@ -148,7 +151,10 @@ entry_stream_kernel(const int *__restrict__ idx, const double *__restrict__ val,
                 const unsigned b = (word >> (unsigned)(ge & 31)) & 0xFu;
                 const int base = __ldg(grpRun + (ge >> 7));                     // row starts in front of the group
                 const double x0 = ld_x(x + c.x, pol_x), x1 = ld_x(x + c.y, pol_x), x2 = ld_x(x + c.z, pol_x), x3 = ld_x(x + c.w, pol_x);
-                const double p0 = __dmul_rn(v0.x, x0), p1 = __dmul_rn(v0.y, x1), p2 = __dmul_rn(v1.x, x2), p3 = __dmul_rn(v1.y, x3);
+                double p0 = __dmul_rn(v0.x, x0), p1 = __dmul_rn(v0.y, x1), p2 = __dmul_rn(v1.x, x2), p3 = __dmul_rn(v1.y, x3);
+                if (!full) {                                // a missing entry adds +0.0, not 0 * x[0] (NaN if x[0] is)
+                    p0 = e < n ? p0 : 0.0; p1 = e + 1 < n ? p1 : 0.0; p2 = e + 2 < n ? p2 : 0.0; p3 = e + 3 < n ? p3 : 0.0;
+                }
                 const bool b0 = b & 1u, b1 = b & 2u, b2 = b & 4u, b3 = b & 8u;
                 const bool has = b != 0u;
                 const int nStarts = __popc(b);
@@ -323,7 +329,7 @@ entry_stream_multi_kernel(const int *__restrict__ idx, const VT *__restrict__ va
             XT *yr = Y + (long long)r * ldy + j0;
 #pragma unroll
             for (int v = 0; v < KP; v++)
-                if (j0 + v < kv) yr[v] = (XT)a[v];
+                if (j0 + v < kv) yr[v] = (XT)Arith<AT>::add(a[v], (AT)0);   // + 0: a sum of -0.0 products is +0.0 (store above)
         }
     };
     auto issue = [&](int s, int t) {
@@ -367,7 +373,8 @@ entry_stream_multi_kernel(const int *__restrict__ idx, const VT *__restrict__ va
                 const long long ge = t0 + e;
                 int4 c;
                 VT a[4];
-                if (c0 + g * 128 + 128 <= n) {
+                const bool full = c0 + g * 128 + 128 <= n;
+                if (full) {
                     if (TMA) c = *reinterpret_cast<const int4 *>(Cc + e);
                     else c = ld_stream_i4(Cc + e, pol_stream);
                     es_vals4<TMA>(a, V + e, pol_stream);
@@ -388,6 +395,13 @@ entry_stream_multi_kernel(const int *__restrict__ idx, const VT *__restrict__ va
                 for (int v = 0; v < KP; v++) {
                     p0[v] = Arith<AT>::mul((AT)a[0], (AT)x0[v]); p1[v] = Arith<AT>::mul((AT)a[1], (AT)x1[v]);
                     p2[v] = Arith<AT>::mul((AT)a[2], (AT)x2[v]); p3[v] = Arith<AT>::mul((AT)a[3], (AT)x3[v]);
+                }
+                if (!full) {                                    // a missing entry adds +0.0, not 0 * X[0, j]
+#pragma unroll
+                    for (int v = 0; v < KP; v++) {
+                        p0[v] = e < n ? p0[v] : (AT)0; p1[v] = e + 1 < n ? p1[v] : (AT)0;
+                        p2[v] = e + 2 < n ? p2[v] : (AT)0; p3[v] = e + 3 < n ? p3[v] : (AT)0;
+                    }
                 }
                 const bool b0 = b & 1u, b1 = b & 2u, b2 = b & 4u, b3 = b & 8u;
                 const bool has = b != 0u;
@@ -491,7 +505,7 @@ entry_stream_multi_kernel(const int *__restrict__ idx, const VT *__restrict__ va
             int accRun = -1;
             auto put = [&](int run, AT v) {
                 const int r = row_of(run);
-                if (r >= rowLo && r < rowHi) Y[(long long)r * ldy + j] = (XT)v;
+                if (r >= rowLo && r < rowHi) Y[(long long)r * ldy + j] = (XT)Arith<AT>::add(v, (AT)0);
             };
             for (int w = 0; w < nw; w++) {
                 const AT oPiece = rPiece[w][j], oTail = rTail[w][j];

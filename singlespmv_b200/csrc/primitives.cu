@@ -133,6 +133,7 @@ __global__ void minmax_kernel(const int *__restrict__ in, long long b, long long
     int mn = 0x7fffffff, mx = -0x7fffffff - 1;
     for (long long i = b + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < e; i += (long long)gridDim.x * blockDim.x) {
         const int v = in[i];
+        if (v < 0) continue;                                   // ELL padding (ELL_PAD): references no column
         mn = min(mn, v);
         mx = max(mx, v);
     }
